@@ -24,6 +24,7 @@ counters cross NVLink (NCCL all-reduce).
            with an oracle check on a query slice x the whole gallery (reference arithmetic on the host).
 `dim8064`: the Market shape at the real concat width D = 8 064 = 63 x 128 (SURVEY 8d).
 `checks`:  at N > 1 the headline result is checked against the oracle on a 64-query slice of the GLOBAL gallery.
+`--dump-outputs DIR`: the per-query results of the last timed step as DIR/<name>.npy, to compare two builds.
 The process exits non-zero (after printing the line) if any oracle check is outside north_star's tolerances.
 """
 from __future__ import annotations
@@ -476,13 +477,15 @@ def run_ours(args):
         engine.kernel_events = []          # events around the distance GEMM launches
     ev0.record()
     for _ in range(args.steps):
-        step_device()
+        last = step_device()
         if c_path:
             for k, v in engine.last_phase_ms().items():
                 phase_sum[k] = phase_sum.get(k, 0.0) + v
     ev1.record()
     barrier()
     launches = _lib.launch_count() - n0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)     # here: the e2e passes below reuse the engine's top-k arrays
     ms_total = ev0.elapsed_time(ev1)
     if c_path:
         engine.set_phase_timing(False)
@@ -654,6 +657,22 @@ def run_ours(args):
     return rc
 
 
+def dump_outputs(out_dir, res):
+    """What one step of the headline path returns to its caller (RankEngine.run's RankResult, plus the mAP / CMC the caller
+    reads from it) as DIR/<name>.npy in float32 / float64: the workload is seeded, so two builds of the project can be
+    compared output for output.  nq = 3 368 and topk <= 128 keep the files under 6 MB in all."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"ap": res.ap, "is_valid": res.is_valid, "first_rank": res.first_rank, "topk_index": res.topk_index,
+              "topk_dist": res.topk_dist, "mAP": np.float64(res.mean_ap()), "cmc": res.cmc(10, True)}
+    for name, a in arrays.items():
+        if a is None:
+            continue
+        a = np.asarray(a)
+        if a.dtype not in (np.float32, np.float64):
+            a = a.astype(np.float64)                  # integer outputs (ranks, indices, flags) are exact in float64
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def bench_pooling(torch, pps_b200, _lib, peaks, dev, args):
     """pps_pool_fwd on Market-shaped conv5 maps: [1024, 2048, 24, 8] fp32 (1.6 GB in, 0.5 GB out per launch;
     far larger than L2), n = 6 parts, 63 combos, mode max_ave.  Algorithmic bytes = 4*C*H*W + 4*63*C per image."""
@@ -703,7 +722,11 @@ def main():
     ap.add_argument("--no-dim8064", action="store_true")
     ap.add_argument("--no-checks", action="store_true")
     ap.add_argument("--no-numa-bind", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         return run_reference(args)
