@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define PPS_ABI_VERSION 5
+#define PPS_ABI_VERSION 6
 
 /* ---- error codes (the Python mirror turns every non-zero code into RuntimeError,
  * like CAFFE_ENFORCE does: detectron/tests/test_zero_even_op.py:50-53) ---- */
@@ -527,6 +527,53 @@ int pps_evaluate_host(const float* q_feats, long long nq,
                       double* out_map, double* out_cmc,
                       double* out_ap, uint8_t* out_valid, int32_t* out_first_rank,
                       int32_t* out_topk_index, float* out_topk_dist);
+
+/* ------------------------------------------------------------------------------------
+ * Part 2h — resident gallery index: the k nearest gallery rows of unlabelled queries (person retrieval).
+ *
+ * No ids, no cameras, no junk filter: the plain Euclidean top-k of pps_dist_tc's distances, smallest first, ties by
+ * gallery index (what rank_eval's top-k gives when no gallery item shares a query's id).
+ *
+ * pps_search_topk_tc   top-k admission with the roles of pps_dist_topk_tc swapped: the gallery rows [ng] are the
+ *                      256-row M operand and the queries [nq] the N operand (N = 32, 64, 128 or 256, the smallest that
+ *                      holds the batch; larger batches take query tiles of 256), so that a small batch streams the
+ *                      gallery once instead of occupying a few rows of every MMA.  Same operands and arithmetic as
+ *                      pps_dist_tc (its distances, bit for bit).  Every distance whose bits are <= tk_bound[q] is
+ *                      appended as (bits << 32 | col0 + row) to tk_cand[q][tk_cap] through tk_cnt[q] (which counts
+ *                      past tk_cap; pps_topk_merge detects it) - the layout pps_topk_merge consumes.  Nothing else is
+ *                      written.  flags: 0, PPS_DIST_SQUARED, PPS_DIST_SQRT_RN.
+ * pps_index_*          a gallery kept on one device as split operand planes [planes][capacity][kpad] plus the norm
+ *                      array (PPS_PREC_F16X3: capacity norms, then capacity inverse scales - the pps_split_rows_slab
+ *                      layout).  pps_index_add appends n rows (device pointer, row stride ld elements) of the index's
+ *                      dtype; the capacity doubles when exceeded.  dtype PPS_DTYPE_F16 uses PPS_PREC_F16X1; dtype
+ *                      PPS_DTYPE_F32 takes PPS_PREC_F16X3 or PPS_PREC_BF16X1/3/6 (PPS_PREC_FP32: PPS_ERR_UNSUPPORTED).
+ * pps_index_search     d_keys[nq][k] = the k nearest rows of the queries d_q [nq, dim] (the index's dtype, row stride
+ *                      ldq) as top-k keys whose gallery index is index_offset + row (a shard passes its first global
+ *                      row); pps_topk_unpack turns them into distances / int32 indices (-1 / inf past the index's
+ *                      size).  index_offset + size must stay below 2^31 (PPS_ERR_UNSUPPORTED otherwise).  The first
+ *                      min(size, 32768) rows are a materialised block swept by pps_topk_update; the rest is covered by
+ *                      pps_search_topk_tc + pps_topk_merge in chunks that grow with the rows already seen.  The call
+ *                      reads back one 4-byte overflow flag (its only synchronisation); when a candidate buffer ran over
+ *                      the search is repeated with materialised blocks only.  Scratch is owned by the index and only
+ *                      grows.  flags: 0, or test hooks PPS_INDEX_TKCAP(n) (candidate entries per query, <= 2048) and
+ *                      PPS_INDEX_PREFIX(n) (n * 256 rows in the materialised prefix, n <= 127).
+ * Calls on one index are ordered by the caller (one stream, or events between streams); every call sets the index's
+ * device for its duration.  A sharded gallery: one index per rank, index_offset = the rows of the ranks before, an
+ * all-gather of the [nq][k] keys and the k smallest per query (every rank's list is sorted, keys are unique).
+ * ---------------------------------------------------------------------------------- */
+#define PPS_INDEX_TKCAP(n)  (((n) & 0xffff) << 8)
+#define PPS_INDEX_PREFIX(n) (((n) & 0x7f) << 24)
+int pps_search_topk_tc(const void* g_planes, const float* g_sqnorm, long long ng, int g_planes_n, long long g_plane_rows,
+                       const void* q_planes, const float* q_sqnorm, long long nq, int q_planes_n, long long q_plane_rows,
+                       int dim, int precision, int flags, long long col0, const uint32_t* tk_bound, uint32_t* tk_cnt,
+                       uint64_t* tk_cand, int tk_cap, void* stream);
+typedef struct pps_index pps_index;
+int       pps_index_create(int device, int dim, int dtype, int precision, pps_index** out);
+int       pps_index_destroy(pps_index* idx);
+int       pps_index_add(pps_index* idx, const void* d_rows, long long n, long long ld, void* stream);
+long long pps_index_size(const pps_index* idx);
+int       pps_index_search(pps_index* idx, const void* d_q, long long nq, long long ldq, int k,
+                           long long index_offset, int flags, void* stream, uint64_t* d_keys);
 
 /* ------------------------------------------------------------------------------------
  * Next row (SURVEY §8f.4) — the reference's training-side triplet mining ops.

@@ -7,13 +7,14 @@ from .pooling import (ReIDPoolCfg, add_pps_part_head, add_pps_part_head_, blob_n
                       pps_pool, pps_pool_autograd, pps_pool_backward, pyramid_combs, uniform_partition_split)
 from .evaluator import (PairLists, RankEngine, RankResult, cmc, compute_dist, evaluate, evaluate_arrays, evaluate_host, mean_ap,
                         rank_distmat, rank_eval, reid_results)
+from .index import GalleryIndex
 from .embedding import ReidEmbedHead, add_reid_outputs, embed_maps, fold_bn, l2_normalize_rows
 from .rerank import re_ranking, re_ranking_from_features
 
 __all__ = [
     "ReIDPoolCfg", "add_pps_part_head", "add_pps_part_head_", "blob_names", "comb_to_mask", "mask_to_comb",
     "pps_pool", "pps_pool_autograd", "pps_pool_backward", "pyramid_combs", "uniform_partition_split",
-    "PairLists", "RankEngine", "RankResult", "cmc", "compute_dist", "evaluate", "evaluate_arrays", "evaluate_host", "mean_ap",
+    "GalleryIndex", "PairLists", "RankEngine", "RankResult", "cmc", "compute_dist", "evaluate", "evaluate_arrays", "evaluate_host", "mean_ap",
     "rank_distmat", "rank_eval", "reid_results",
     "ReidEmbedHead", "add_reid_outputs", "embed_maps", "fold_bn", "l2_normalize_rows",
     "re_ranking", "re_ranking_from_features",

@@ -13,7 +13,7 @@ import threading
 from . import build as _build
 
 # ---- constants (keep in sync with include/pps_b200.h) ----
-ABI_VERSION = 5
+ABI_VERSION = 6
 PPS_OK = 0
 PPS_ERR_INVALID_ARG = -1
 PPS_ERR_SHAPE = -2
@@ -27,6 +27,16 @@ PPS_ERR_PASS_RESIZE = -9
 PASS_NO_EPILOGUE_TOPK = 1
 PASS_SIZING = 2
 PASS_NO_FUSED_COUNT = 4
+
+
+def index_tkcap(n: int) -> int:
+    """PPS_INDEX_TKCAP(n): pps_index_search test hook, candidate entries per query and chunk."""
+    return (n & 0xffff) << 8
+
+
+def index_prefix(n: int) -> int:
+    """PPS_INDEX_PREFIX(n): pps_index_search test hook, n * 256 rows in the materialised prefix."""
+    return (n & 0x7f) << 24
 
 POOL_AVG_MAX = 0
 POOL_MAX_AVE = 1
@@ -135,6 +145,12 @@ SIGNATURES = {
     "pps_ctx_phase_ms": (_i, [_vp, _vp]),
     "pps_evaluate_host": (_i, [_vp, _ll, _vp, _ll, _i, _vp, _vp, _vp, _vp, _i, _i, _i, _i,
                                _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "pps_search_topk_tc": (_i, [_vp, _vp, _ll, _i, _ll, _vp, _vp, _ll, _i, _ll, _i, _i, _i, _ll, _vp, _vp, _vp, _i, _vp]),
+    "pps_index_create": (_i, [_i, _i, _i, _i, C.POINTER(_vp)]),
+    "pps_index_destroy": (_i, [_vp]),
+    "pps_index_add": (_i, [_vp, _vp, _ll, _ll, _vp]),
+    "pps_index_size": (_ll, [_vp]),
+    "pps_index_search": (_i, [_vp, _vp, _ll, _ll, _i, _ll, _i, _vp, _vp]),
     "pps_pairwise_distance_fwd": (_i, [_vp, _i, _i, _vp, _vp]),
     "pps_pairwise_distance_bwd": (_i, [_vp, _vp, _i, _i, _vp, _vp]),
     "pps_batch_hard_fwd": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _vp]),

@@ -13,7 +13,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT_DIR = os.path.join(HERE, "_C")
 LIB_PATH = os.path.join(OUT_DIR, "libpps_b200.so")
-SOURCES = ["pps_pool.cu", "split_prep.cu", "dist_gemm.cu", "pairs.cu", "rank.cu", "triplet.cu", "rerank.cu", "c_api.cu", "pass.cu"]
+SOURCES = ["pps_pool.cu", "split_prep.cu", "dist_gemm.cu", "pairs.cu", "rank.cu", "triplet.cu", "rerank.cu", "c_api.cu", "pass.cu", "index.cu"]
 HEADERS = [os.path.join(CSRC, "common.cuh"), os.path.join(CSRC, "ctx.cuh"), os.path.join(CSRC, "dist_tiles.cuh"), os.path.join(os.path.dirname(HERE), "include", "pps_b200.h")]
 
 NVCC_FLAGS = [

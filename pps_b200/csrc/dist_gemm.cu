@@ -248,7 +248,7 @@ __device__ __forceinline__ void dist_tc2_body(const CUtensorMap& tmA, const CUte
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&tmA);
     tma_prefetch_desc(&tmB);
-    if (EPI != EPI_RANK) tma_prefetch_desc(&tmO);
+    if (EPI != EPI_RANK && EPI != EPI_SEARCH) tma_prefetch_desc(&tmO);
     for (int s = 0; s < kMaxStages2; ++s) {
       mbar_init(&full[s], 1);
       mbar_init(&empty[s], CL4 ? 2 : 1);   // CL4: a slot also receives the other pair's B half, so both pairs' MMAs free it
@@ -419,6 +419,11 @@ __device__ __forceinline__ void dist_tc2_body(const CUtensorMap& tmA, const CUte
           bn_s[256 + etid] = gj < g.m2 ? __ldg(g.b_scale + gj) : 0.f;
           if (BN > 128) bn_s[256 + etid + 128] = gj + 128 < g.m2 ? __ldg(g.b_scale + gj + 128) : 0.f;
         }
+        if (EPI == EPI_SEARCH) {               // the admission bound of every query column, double-buffered like |b|^2
+          uint32_t* bd = reinterpret_cast<uint32_t*>(stage_out) + as * 256;
+          bd[etid] = gj < g.m2 ? __ldg(rf.tk_bound + gj) : 0u;
+          if (BN > 128) bd[etid + 128] = gj + 128 < g.m2 ? __ldg(rf.tk_bound + gj + 128) : 0u;
+        }
       }
       asm volatile("bar.sync 1, %0;" ::"n"(kEpiThreads) : "memory");
       const float an = (EPI != EPI_AFFINE_RELU && gi < g.m1 && !want_dot) ? __ldg(g.a_sqnorm + gi) : 0.f;
@@ -428,12 +433,64 @@ __device__ __forceinline__ void dist_tc2_body(const CUtensorMap& tmA, const CUte
       mbar_wait(&tfull[as], aph);
       tc_fence_after();
       const uint32_t tbase = tmem_base + as * BN + ((uint32_t)(lane_grp * 32) << 16);
-      const int c_first = EPI == EPI_RANK ? col_half * 128 : 0, c_stop = EPI == EPI_RANK ? c_first + 128 : BN;
+      // EPI_SEARCH: chunks of 32 query columns up to the last query of the tile
+      const int c_first = EPI == EPI_RANK ? col_half * 128 : 0;
+      const int c_stop = EPI == EPI_RANK ? c_first + 128 : EPI == EPI_SEARCH ? (int)min((long long)BN, (g.m2 - n0 + 31) & ~31LL) : BN;
 #pragma unroll 1
       for (int c = c_first; c < c_stop; c += 32, ++chunk_it) {
         uint32_t r[32];
         tmem_ld_32x32(tbase + c, r);
-        if (EPI == EPI_RANK) {
+        if (EPI == EPI_SEARCH) {
+          // thread = gallery row, columns = queries.  pps_dist_tc's arithmetic with the roles swapped:
+          // (-2ab + |q|^2) + |g|^2 with -2ab = (-2 / (s_g s_q)) dot exact, so every distance has pps_dist_tc's bits.
+          tmem_ld_wait();
+          const uint32_t* bd = reinterpret_cast<const uint32_t*>(stage_out) + as * 256 + c;
+          const float4* qn4 = reinterpret_cast<const float4*>(bn + c);
+          const bool row_ok = gi < g.m1;
+          const long long valid_cols = g.m2 - n0 - c;          // query columns of this chunk that exist
+          uint32_t v[32];
+          bool hit = false;
+#pragma unroll
+          for (int j = 0; j < 8; ++j) {
+            const float4 q4 = qn4[j];
+            const float qq[4] = {q4.x, q4.y, q4.z, q4.w};
+            float sc[4] = {cs, cs, cs, cs};
+            if (scaled) {
+              const float4 s4 = reinterpret_cast<const float4*>(sc_s + c)[j];
+              sc[0] = cs * s4.x; sc[1] = cs * s4.y; sc[2] = cs * s4.z; sc[3] = cs * s4.w;
+            }
+            const uint4 b4 = reinterpret_cast<const uint4*>(bd)[j];
+            const uint32_t bb[4] = {b4.x, b4.y, b4.z, b4.w};
+#pragma unroll
+            for (int e = 0; e < 4; ++e) {
+              const float dot = __uint_as_float(r[4 * j + e]);
+              float d2 = __fadd_rn(__fmaf_rn(sc[e], dot, qq[e]), an);
+              d2 = fmaxf(d2, 0.f);
+              v[4 * j + e] = __float_as_uint(want_sq ? d2 : (sqrt_rn ? __fsqrt_rn(d2) : sqrt_approx(d2)));
+              hit |= (v[4 * j + e] <= bb[e]) & (4 * j + e < valid_cols);   // distances are >= 0: bits order like values
+            }
+          }
+          // admission, aggregated per (warp, query): one atomic reserves the slots of every lane that passes
+          if (__any_sync(0xffffffffu, hit && row_ok)) {
+            const uint32_t lanes_below = (1u << lane) - 1u;
+            const unsigned long long gkey = (unsigned long long)(uint32_t)(rf.col0 + gi);
+#pragma unroll
+            for (int e = 0; e < 32; ++e) {                     // (unrolled: v[] must stay in registers)
+              const bool pass = row_ok && e < valid_cols && v[e] <= bd[e];
+              const uint32_t m = __ballot_sync(0xffffffffu, pass);
+              if (m) {
+                const long long col = (long long)n0 + c + e;
+                const int leader = __ffs(m) - 1;
+                uint32_t base = 0;
+                if (lane == leader) base = atomicAdd(rf.tk_cnt + col, (uint32_t)__popc(m));
+                base = __shfl_sync(0xffffffffu, base, leader);
+                const uint32_t slot = base + (uint32_t)__popc(m & lanes_below);
+                if (pass && slot < (uint32_t)rf.tk_cap)
+                  rf.tk_cand[col * rf.tk_cap + slot] = ((unsigned long long)v[e] << 32) | gkey;
+              }
+            }
+          }
+        } else if (EPI == EPI_RANK) {
           tmem_ld_wait();
           const int valid_cols = n_end - n0 - c;             // columns of this chunk inside the gallery block
           const long long colg = rf.col0 + n0 + c;           // global gallery index of the chunk's first column
@@ -603,7 +660,7 @@ __device__ __forceinline__ void dist_tc2_body(const CUtensorMap& tmA, const CUte
         if (gi < g.m1 && tie_corr) atomicAdd(rf.cnt_first + gi, tie_corr);
       }
     }
-    if (EPI != EPI_RANK) bulk_wait_group_read<0>();
+    if (EPI != EPI_RANK && EPI != EPI_SEARCH) bulk_wait_group_read<0>();
   }
 
   tc_fence_before();
@@ -936,6 +993,92 @@ extern "C" int pps_dist_topk_tc(const void* a_planes, const float* a_sqnorm, lon
   rf.tk_bound = tk_bound; rf.tk_cnt = tk_cnt; rf.tk_cand = reinterpret_cast<unsigned long long*>(tk_cand); rf.tk_cap = tk_cap;
   return dist_tc_impl(a_planes, a_sqnorm, m1, a_planes_n, a_plane_rows, b_planes, b_sqnorm, m2, b_planes_n, b_plane_rows, dim,
                       precision, flags, dist, ldd, stream, &rf);
+}
+
+// Top-k admission for a batch of queries against a block of gallery rows, with the roles of pps_dist_topk_tc swapped: the
+// gallery is the 256-row M operand and the queries are N = BN in {32, 64, 128, 256} (the smallest that holds the batch;
+// larger batches take several query tiles of 256).  A small batch then streams the gallery through the SMs once instead
+// of filling a few rows of every 256-row MMA.  Nothing is written but the candidates.
+template <int BN>
+static int launch_search(const CUtensorMap& tmA, const CUtensorMap& tmB, const Gemm2Args& ga, const RankFuse& rf, int dev,
+                         long long pairs, cudaStream_t st) {
+  static thread_local int configured_dev = -1;
+  if (configured_dev != dev) {
+    PPS_CUDA_TRY(cudaFuncSetAttribute(dist_tc2_kernel<BN, EPI_SEARCH>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                      (int)kGemm2Smem));
+    configured_dev = dev;
+  }
+  dist_tc2_kernel<BN, EPI_SEARCH><<<(unsigned)(2 * pairs), kGemmThreads, kGemm2Smem, st>>>(tmA, tmB, tmA /*no output map*/,
+                                                                                           ga, rf);
+  PPS_LAUNCH_CHECK("dist_tc2_kernel<search>");
+  return PPS_OK;
+}
+
+extern "C" int pps_search_topk_tc(const void* g_planes, const float* g_sqnorm, long long ng, int g_planes_n,
+                                  long long g_plane_rows, const void* q_planes, const float* q_sqnorm, long long nq,
+                                  int q_planes_n, long long q_plane_rows, int dim, int precision, int flags, long long col0,
+                                  const uint32_t* tk_bound, uint32_t* tk_cnt, uint64_t* tk_cand, int tk_cap, void* stream) {
+  if (ng < 0 || nq < 0 || dim <= 0 || col0 < 0 || tk_cap < 1) return PPS_ERR_INVALID_ARG;
+  if (flags & ~(PPS_DIST_SQUARED | PPS_DIST_SQRT_RN)) return PPS_ERR_INVALID_ARG;   // keys order by the bits of a distance
+  if (g_plane_rows == 0) g_plane_rows = ng;
+  if (q_plane_rows == 0) q_plane_rows = nq;
+  if (g_plane_rows < ng || q_plane_rows < nq || col0 + ng > 0xffffffffLL) return PPS_ERR_INVALID_ARG;
+  if (ng == 0 || nq == 0) return PPS_OK;
+  if (!g_planes || !g_sqnorm || !q_planes || !q_sqnorm || !tk_bound || !tk_cnt || !tk_cand) return PPS_ERR_INVALID_ARG;
+  if ((reinterpret_cast<uintptr_t>(g_planes) & 15u) || (reinterpret_cast<uintptr_t>(q_planes) & 15u)) return PPS_ERR_ALIGN;
+  if (ng > 0x7fffff00LL || nq > 0x7fffff00LL) return PPS_ERR_UNSUPPORTED;   // TMA coordinates are int32
+  GemmArgs terms;
+  bool f16 = false;
+  const int need = setup_terms(precision, terms, &f16);
+  if (need == 0 || g_planes_n < need || q_planes_n < need) return PPS_ERR_INVALID_ARG;
+  const int sms = sm_count();
+  if (sms < 2) return PPS_ERR_UNSUPPORTED;
+  const bool scaled = precision == PPS_PREC_F16X3;
+  const int bn = nq <= 32 ? 32 : nq <= 64 ? 64 : nq <= 128 ? 128 : 256;
+  const int kpad = pps_kpad(dim);
+  const uint32_t fmt = f16 ? 0u : 1u;
+  Gemm2Args ga;
+  GemmArgs& g = ga.g;
+  g.nterms = terms.nterms;
+  for (int t = 0; t < terms.nterms; ++t) {     // the same (query plane, gallery plane) products in the same order
+    g.term_a[t] = terms.term_b[t];
+    g.term_b[t] = terms.term_a[t];
+  }
+  g.m1 = ng; g.m2 = nq;
+  g.kblocks = kpad / kBK;
+  g.idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | ((uint32_t)(bn >> 3) << 17) | ((uint32_t)(256 >> 4) << 24);
+  g.a_sqnorm = g_sqnorm; g.b_sqnorm = q_sqnorm;
+  g.a_scale = scaled ? g_sqnorm + g_plane_rows : nullptr;
+  g.b_scale = scaled ? q_sqnorm + q_plane_rows : nullptr;
+  g.out = nullptr; g.ldo = 0; g.flags = flags;
+  static const int env_sqrt = [] { const char* e = getenv("PPS_SQRT_RN"); return e ? atoi(e) : -1; }();   // as pps_dist_tc
+  if (env_sqrt >= 0) g.flags = env_sqrt ? (g.flags | PPS_DIST_SQRT_RN) : (g.flags & ~PPS_DIST_SQRT_RN);
+  g.m_tiles = (int)((ng + 255) / 256);
+  g.n_tiles = (int)((nq + bn - 1) / bn);
+  ga.planes = need;
+  ga.sep_small = 0;
+  ga.stages = kRing2Bytes / (need * (kTile2Bytes + (bn / 2) * kBK * 2));
+  if (ga.stages > kMaxStages2) ga.stages = kMaxStages2;
+  ga.groups = 1; ga.a_group_rows = 0; ga.b_group_rows = 0; ga.out_group_cols = 0;
+  CUtensorMap tmA, tmB;
+  int rc = make_operand_map(&tmA, g_planes, ng, g_plane_rows, kpad, g_planes_n, kT2Rows, f16);
+  if (rc) return rc;
+  rc = make_operand_map(&tmB, q_planes, nq, q_plane_rows, kpad, q_planes_n, bn / 2, f16);
+  if (rc) return rc;
+  RankFuse rf{};
+  rf.col0 = col0;
+  rf.tk_bound = tk_bound; rf.tk_cnt = tk_cnt; rf.tk_cand = reinterpret_cast<unsigned long long*>(tk_cand); rf.tk_cap = tk_cap;
+  int dev = 0;
+  PPS_CUDA_TRY(cudaGetDevice(&dev));
+  const long long tiles = (long long)g.m_tiles * g.n_tiles;
+  const long long pairs = tiles < sms / 2 ? tiles : sms / 2;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  switch (bn) {
+    case 32: return launch_search<32>(tmA, tmB, ga, rf, dev, pairs, st);
+    case 64: return launch_search<64>(tmA, tmB, ga, rf, dev, pairs, st);
+    case 128: return launch_search<128>(tmA, tmB, ga, rf, dev, pairs, st);
+    default: return launch_search<256>(tmA, tmB, ga, rf, dev, pairs, st);
+  }
 }
 
 extern "C" int pps_dist_fp32(const float* a, long long lda, const float* a_sqnorm, long long m1, const float* b,

@@ -65,9 +65,11 @@ constexpr int EPI_DIST = 0;          // |a|^2 + |b|^2 - 2ab, clamp, sqrt (or squ
 constexpr int EPI_AFFINE_RELU = 1;   // max(0, dot * alpha[col] + beta[col])   (a_sqnorm = alpha, b_sqnorm = beta)
 constexpr int EPI_RANK = 2;          // distance as EPI_DIST, consumed by the counting epilogue; no matrix
 constexpr int EPI_DIST_TOPK = 3;     // EPI_DIST + one compare per element against the row's top-k admission bound
+constexpr int EPI_SEARCH = 4;        // A = gallery, B = queries: distance -> top-k admission per COLUMN; no matrix
 
 // Tile order.  EPI_DIST / EPI_AFFINE_RELU: tile t = pair, pair + npairs, ... with the m index fastest, so that the
-// CTA pairs running concurrently share B tiles in L2.  EPI_RANK: a CTA pair keeps ONE m tile per run (its rows'
+// CTA pairs running concurrently share B tiles in L2.  EPI_SEARCH: the same tiles with the n index fastest, so that a
+// gallery (m) tile is read from HBM once and its other query tiles find it in L2.  EPI_RANK: a CTA pair keeps ONE m tile per run (its rows'
 // thresholds and counters stay in shared memory) and walks a contiguous range of n tiles.
 //   npairs >= m_tiles: k = npairs / m_tiles pairs per m tile walk n tiles [0, Na) in k aligned parts - the pairs that own
 //     the other m tiles walk the same n range at the same pace, which keeps the L2 sharing of B - and the X = npairs % m_tiles
@@ -124,8 +126,13 @@ struct TileWalk {
       if (t >= tiles) return false;
       grp = t / tiles_per_group;
       const long long tt = t % tiles_per_group;
-      m_tile = (int)(tt % m_tiles);
-      n_tile = (int)(tt / m_tiles);
+      if (EPI == EPI_SEARCH) {
+        m_tile = (int)(tt / n_tiles);
+        n_tile = (int)(tt % n_tiles);
+      } else {
+        m_tile = (int)(tt % m_tiles);
+        n_tile = (int)(tt / m_tiles);
+      }
       return true;
     }
     if (balanced) {

@@ -1202,7 +1202,13 @@ def merge_topk_keys(key, topk, group):
     world = dist_mod.get_world_size(group)
     gathered = [torch.empty_like(key) for _ in range(world)]
     dist_mod.all_gather(gathered, key, group=group)
-    allk = torch.cat(gathered, dim=1)
+    return merge_key_lists(gathered, topk)
+
+
+def merge_key_lists(keys, topk):
+    """The k smallest of several [nq, k] top-k key lists per query (the merge step of merge_topk_keys)."""
+    import torch
+    allk = torch.cat(list(keys), dim=1)
     big = torch.iinfo(torch.int64).max
     allk = torch.where(allk == -1, torch.full_like(allk, big), allk)
     merged = torch.sort(allk, dim=1).values[:, :topk]
