@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define PPS_ABI_VERSION 6
+#define PPS_ABI_VERSION 7
 
 /* ---- error codes (the Python mirror turns every non-zero code into RuntimeError,
  * like CAFFE_ENFORCE does: detectron/tests/test_zero_even_op.py:50-53) ---- */
@@ -531,8 +531,12 @@ int pps_evaluate_host(const float* q_feats, long long nq,
 /* ------------------------------------------------------------------------------------
  * Part 2h — resident gallery index: the k nearest gallery rows of unlabelled queries (person retrieval).
  *
- * No ids, no cameras, no junk filter: the plain Euclidean top-k of pps_dist_tc's distances, smallest first, ties by
- * gallery index (what rank_eval's top-k gives when no gallery item shares a query's id).
+ * The Euclidean top-k of pps_dist_tc's distances, smallest first, ties by gallery index (what rank_eval's top-k gives
+ * when no gallery item shares a query's id).  Optional exclusion by tag: one int64 tag per gallery row and one exclude
+ * tag per query; row r is left out of query q's result if and only if tag[r] == exclude_tag[q].  Two encodings:
+ *   cross-camera search         tag = camera of the row, exclude tag = camera of the query
+ *   the evaluation's junk rule  tag = (id << 32) | camera (ids in int32, cameras in [0, 2^32)): the result equals
+ *                               rank_eval's top-k (same id and camera left out) bit for bit
  *
  * pps_search_topk_tc   top-k admission with the roles of pps_dist_topk_tc swapped: the gallery rows [ng] are the
  *                      256-row M operand and the queries [nq] the N operand (N = 32, 64, 128 or 256, the smallest that
@@ -542,11 +546,19 @@ int pps_evaluate_host(const float* q_feats, long long nq,
  *                      appended as (bits << 32 | col0 + row) to tk_cand[q][tk_cap] through tk_cnt[q] (which counts
  *                      past tk_cap; pps_topk_merge detects it) - the layout pps_topk_merge consumes.  Nothing else is
  *                      written.  flags: 0, PPS_DIST_SQUARED, PPS_DIST_SQRT_RN.
+ * pps_search_topk_excl_tc   the same without the pairs whose tags are equal: g_tags[ng] (row r of this block: the tag
+ *                      of row col0 + r is g_tags[r]) and q_tags[nq], both required.  The tags are compared only for
+ *                      elements within the bound; an excluded element takes no slot.
+ * pps_topk_update_excl pps_topk_update without the columns c with g_tags[c] == q_tags[q] (g_tags[ncols]: column c's
+ *                      tag, q_tags[nq]).  n_excluded (may be null): n_excluded[q] = the number of such columns in this
+ *                      call (every column's tag is read then; otherwise only those of admitted columns).
  * pps_index_*          a gallery kept on one device as split operand planes [planes][capacity][kpad] plus the norm
  *                      array (PPS_PREC_F16X3: capacity norms, then capacity inverse scales - the pps_split_rows_slab
  *                      layout).  pps_index_add appends n rows (device pointer, row stride ld elements) of the index's
  *                      dtype; the capacity doubles when exceeded.  dtype PPS_DTYPE_F16 uses PPS_PREC_F16X1; dtype
  *                      PPS_DTYPE_F32 takes PPS_PREC_F16X3 or PPS_PREC_BF16X1/3/6 (PPS_PREC_FP32: PPS_ERR_UNSUPPORTED).
+ *                      pps_index_add_tagged appends rows with their tags d_tags[n] (device).  The first non-empty add
+ *                      decides whether the index is tagged; a later add of the other kind is PPS_ERR_INVALID_ARG.
  * pps_index_search     d_keys[nq][k] = the k nearest rows of the queries d_q [nq, dim] (the index's dtype, row stride
  *                      ldq) as top-k keys whose gallery index is index_offset + row (a shard passes its first global
  *                      row); pps_topk_unpack turns them into distances / int32 indices (-1 / inf past the index's
@@ -556,7 +568,13 @@ int pps_evaluate_host(const float* q_feats, long long nq,
  *                      reads back one 4-byte overflow flag (its only synchronisation); when a candidate buffer ran over
  *                      the search is repeated with materialised blocks only.  Scratch is owned by the index and only
  *                      grows.  flags: 0, or test hooks PPS_INDEX_TKCAP(n) (candidate entries per query, <= 2048) and
- *                      PPS_INDEX_PREFIX(n) (n * 256 rows in the materialised prefix, n <= 127).
+ *                      PPS_INDEX_PREFIX(n) (n * 256 rows in the materialised prefix, n <= 127).  On a tagged index
+ *                      it ignores the tags.
+ * pps_index_search_excluding   pps_index_search without the rows whose tag equals the query's d_q_tags[q] (device,
+ *                      [nq], required); PPS_ERR_INVALID_ARG on a non-empty untagged index.  Fewer than k remaining rows:
+ *                      padded with -1 / inf.  Same schedule with the excluding kernels; when the gallery is larger than
+ *                      the prefix, the prefix sweep counts every query's excluded rows and one more 4-byte read-back
+ *                      (the largest count) shrinks the chunks by the excluded share (at most 0.9).
  * Calls on one index are ordered by the caller (one stream, or events between streams); every call sets the index's
  * device for its duration.  A sharded gallery: one index per rank, index_offset = the rows of the ranks before, an
  * all-gather of the [nq][k] keys and the k smallest per query (every rank's list is sorted, keys are unique).
@@ -567,13 +585,26 @@ int pps_search_topk_tc(const void* g_planes, const float* g_sqnorm, long long ng
                        const void* q_planes, const float* q_sqnorm, long long nq, int q_planes_n, long long q_plane_rows,
                        int dim, int precision, int flags, long long col0, const uint32_t* tk_bound, uint32_t* tk_cnt,
                        uint64_t* tk_cand, int tk_cap, void* stream);
+int pps_search_topk_excl_tc(const void* g_planes, const float* g_sqnorm, long long ng, int g_planes_n,
+                            long long g_plane_rows, const void* q_planes, const float* q_sqnorm, long long nq,
+                            int q_planes_n, long long q_plane_rows, int dim, int precision, int flags, long long col0,
+                            const uint32_t* tk_bound, uint32_t* tk_cnt, uint64_t* tk_cand, int tk_cap, void* stream,
+                            const int64_t* g_tags, const int64_t* q_tags);
+int pps_topk_update_excl(const float* dist, long long ldd, long long nq, long long ncols, long long col0,
+                         const int64_t* g_tags, const int64_t* q_tags, uint64_t* topk_key, int k,
+                         uint32_t* n_excluded, void* stream);
 typedef struct pps_index pps_index;
 int       pps_index_create(int device, int dim, int dtype, int precision, pps_index** out);
 int       pps_index_destroy(pps_index* idx);
 int       pps_index_add(pps_index* idx, const void* d_rows, long long n, long long ld, void* stream);
+int       pps_index_add_tagged(pps_index* idx, const void* d_rows, long long n, long long ld, const int64_t* d_tags,
+                               void* stream);
 long long pps_index_size(const pps_index* idx);
 int       pps_index_search(pps_index* idx, const void* d_q, long long nq, long long ldq, int k,
                            long long index_offset, int flags, void* stream, uint64_t* d_keys);
+int       pps_index_search_excluding(pps_index* idx, const void* d_q, long long nq, long long ldq,
+                                     const int64_t* d_q_tags, int k, long long index_offset, int flags, void* stream,
+                                     uint64_t* d_keys);
 
 /* ------------------------------------------------------------------------------------
  * Next row (SURVEY §8f.4) — the reference's training-side triplet mining ops.

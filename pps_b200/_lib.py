@@ -13,7 +13,7 @@ import threading
 from . import build as _build
 
 # ---- constants (keep in sync with include/pps_b200.h) ----
-ABI_VERSION = 6
+ABI_VERSION = 7
 PPS_OK = 0
 PPS_ERR_INVALID_ARG = -1
 PPS_ERR_SHAPE = -2
@@ -151,6 +151,11 @@ SIGNATURES = {
     "pps_index_add": (_i, [_vp, _vp, _ll, _ll, _vp]),
     "pps_index_size": (_ll, [_vp]),
     "pps_index_search": (_i, [_vp, _vp, _ll, _ll, _i, _ll, _i, _vp, _vp]),
+    "pps_search_topk_excl_tc": (_i, [_vp, _vp, _ll, _i, _ll, _vp, _vp, _ll, _i, _ll, _i, _i, _i, _ll, _vp, _vp, _vp, _i, _vp,
+                                     _vp, _vp]),
+    "pps_topk_update_excl": (_i, [_vp, _ll, _ll, _ll, _ll, _vp, _vp, _vp, _i, _vp, _vp]),
+    "pps_index_add_tagged": (_i, [_vp, _vp, _ll, _ll, _vp, _vp]),
+    "pps_index_search_excluding": (_i, [_vp, _vp, _ll, _ll, _vp, _i, _ll, _i, _vp, _vp]),
     "pps_pairwise_distance_fwd": (_i, [_vp, _i, _i, _vp, _vp]),
     "pps_pairwise_distance_bwd": (_i, [_vp, _vp, _i, _i, _vp, _vp]),
     "pps_batch_hard_fwd": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _vp]),

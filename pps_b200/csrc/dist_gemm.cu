@@ -248,7 +248,7 @@ __device__ __forceinline__ void dist_tc2_body(const CUtensorMap& tmA, const CUte
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&tmA);
     tma_prefetch_desc(&tmB);
-    if (EPI != EPI_RANK && EPI != EPI_SEARCH) tma_prefetch_desc(&tmO);
+    if (EPI != EPI_RANK && !epi_search(EPI)) tma_prefetch_desc(&tmO);
     for (int s = 0; s < kMaxStages2; ++s) {
       mbar_init(&full[s], 1);
       mbar_init(&empty[s], CL4 ? 2 : 1);   // CL4: a slot also receives the other pair's B half, so both pairs' MMAs free it
@@ -373,6 +373,8 @@ __device__ __forceinline__ void dist_tc2_body(const CUtensorMap& tmA, const CUte
     uint32_t rk_bound = 0u;                     // top-k admission bound of this row (EPI_RANK with candidate lists)
     const bool rk_admit = EPI == EPI_RANK && rf.tk_cand != nullptr;
     long long tab_base = 0;                     // element offset of (row group, j = 0, this row) in the global tables
+    long long row_tag = 0;                      // EPI_SEARCH_EXCL: this row's tag, loaded for m tile tag_tile
+    int tag_tile = -1;
     TileWalk<EPI> w(ga, pair, npairs);
     for (; w.next(); ++acc_it) {
       const int m0 = w.m_tile * kClusterRows + pair_row0 + (int)rank * kT2Rows;       // output row (within the group's rows)
@@ -419,7 +421,7 @@ __device__ __forceinline__ void dist_tc2_body(const CUtensorMap& tmA, const CUte
           bn_s[256 + etid] = gj < g.m2 ? __ldg(g.b_scale + gj) : 0.f;
           if (BN > 128) bn_s[256 + etid + 128] = gj + 128 < g.m2 ? __ldg(g.b_scale + gj + 128) : 0.f;
         }
-        if (EPI == EPI_SEARCH) {               // the admission bound of every query column, double-buffered like |b|^2
+        if (epi_search(EPI)) {                 // the admission bound of every query column, double-buffered like |b|^2
           uint32_t* bd = reinterpret_cast<uint32_t*>(stage_out) + as * 256;
           bd[etid] = gj < g.m2 ? __ldg(rf.tk_bound + gj) : 0u;
           if (BN > 128) bd[etid + 128] = gj + 128 < g.m2 ? __ldg(rf.tk_bound + gj + 128) : 0u;
@@ -435,12 +437,12 @@ __device__ __forceinline__ void dist_tc2_body(const CUtensorMap& tmA, const CUte
       const uint32_t tbase = tmem_base + as * BN + ((uint32_t)(lane_grp * 32) << 16);
       // EPI_SEARCH: chunks of 32 query columns up to the last query of the tile
       const int c_first = EPI == EPI_RANK ? col_half * 128 : 0;
-      const int c_stop = EPI == EPI_RANK ? c_first + 128 : EPI == EPI_SEARCH ? (int)min((long long)BN, (g.m2 - n0 + 31) & ~31LL) : BN;
+      const int c_stop = EPI == EPI_RANK ? c_first + 128 : epi_search(EPI) ? (int)min((long long)BN, (g.m2 - n0 + 31) & ~31LL) : BN;
 #pragma unroll 1
       for (int c = c_first; c < c_stop; c += 32, ++chunk_it) {
         uint32_t r[32];
         tmem_ld_32x32(tbase + c, r);
-        if (EPI == EPI_SEARCH) {
+        if (epi_search(EPI)) {
           // thread = gallery row, columns = queries.  pps_dist_tc's arithmetic with the roles swapped:
           // (-2ab + |q|^2) + |g|^2 with -2ab = (-2 / (s_g s_q)) dot exact, so every distance has pps_dist_tc's bits.
           tmem_ld_wait();
@@ -474,9 +476,17 @@ __device__ __forceinline__ void dist_tc2_body(const CUtensorMap& tmA, const CUte
           if (__any_sync(0xffffffffu, hit && row_ok)) {
             const uint32_t lanes_below = (1u << lane) - 1u;
             const unsigned long long gkey = (unsigned long long)(uint32_t)(rf.col0 + gi);
+            // EPI_SEARCH_EXCL: the row's tag is loaded on the row's first hit of the tile (the n tiles of one m tile
+            // share it)
+            if (EPI == EPI_SEARCH_EXCL && hit && row_ok && tag_tile != w.m_tile) {
+              row_tag = __ldg(rf.g_tags + gi);
+              tag_tile = w.m_tile;
+            }
 #pragma unroll
             for (int e = 0; e < 32; ++e) {                     // (unrolled: v[] must stay in registers)
-              const bool pass = row_ok && e < valid_cols && v[e] <= bd[e];
+              bool pass = row_ok && e < valid_cols && v[e] <= bd[e];
+              if (EPI == EPI_SEARCH_EXCL && pass)              // one address per warp: an L1 broadcast
+                pass = row_tag != __ldg(rf.q_tags + ((long long)n0 + c + e));
               const uint32_t m = __ballot_sync(0xffffffffu, pass);
               if (m) {
                 const long long col = (long long)n0 + c + e;
@@ -660,7 +670,7 @@ __device__ __forceinline__ void dist_tc2_body(const CUtensorMap& tmA, const CUte
         if (gi < g.m1 && tie_corr) atomicAdd(rf.cnt_first + gi, tie_corr);
       }
     }
-    if (EPI != EPI_RANK && EPI != EPI_SEARCH) bulk_wait_group_read<0>();
+    if (EPI != EPI_RANK && !epi_search(EPI)) bulk_wait_group_read<0>();
   }
 
   tc_fence_before();
@@ -999,25 +1009,33 @@ extern "C" int pps_dist_topk_tc(const void* a_planes, const float* a_sqnorm, lon
 // gallery is the 256-row M operand and the queries are N = BN in {32, 64, 128, 256} (the smallest that holds the batch;
 // larger batches take several query tiles of 256).  A small batch then streams the gallery through the SMs once instead
 // of filling a few rows of every 256-row MMA.  Nothing is written but the candidates.
-template <int BN>
+// The exclusion is an instance of its own (EPI_SEARCH_EXCL), so that the untagged kernel keeps its code.
+template <int BN, int EPI>
 static int launch_search(const CUtensorMap& tmA, const CUtensorMap& tmB, const Gemm2Args& ga, const RankFuse& rf, int dev,
                          long long pairs, cudaStream_t st) {
   static thread_local int configured_dev = -1;
   if (configured_dev != dev) {
-    PPS_CUDA_TRY(cudaFuncSetAttribute(dist_tc2_kernel<BN, EPI_SEARCH>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    PPS_CUDA_TRY(cudaFuncSetAttribute(dist_tc2_kernel<BN, EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                       (int)kGemm2Smem));
     configured_dev = dev;
   }
-  dist_tc2_kernel<BN, EPI_SEARCH><<<(unsigned)(2 * pairs), kGemmThreads, kGemm2Smem, st>>>(tmA, tmB, tmA /*no output map*/,
-                                                                                           ga, rf);
-  PPS_LAUNCH_CHECK("dist_tc2_kernel<search>");
+  dist_tc2_kernel<BN, EPI><<<(unsigned)(2 * pairs), kGemmThreads, kGemm2Smem, st>>>(tmA, tmB, tmA /*no output map*/, ga, rf);
+  PPS_LAUNCH_CHECK(EPI == EPI_SEARCH ? "dist_tc2_kernel<search>" : "dist_tc2_kernel<search_excl>");
   return PPS_OK;
 }
 
-extern "C" int pps_search_topk_tc(const void* g_planes, const float* g_sqnorm, long long ng, int g_planes_n,
-                                  long long g_plane_rows, const void* q_planes, const float* q_sqnorm, long long nq,
-                                  int q_planes_n, long long q_plane_rows, int dim, int precision, int flags, long long col0,
-                                  const uint32_t* tk_bound, uint32_t* tk_cnt, uint64_t* tk_cand, int tk_cap, void* stream) {
+template <int BN>
+static int launch_search(const CUtensorMap& tmA, const CUtensorMap& tmB, const Gemm2Args& ga, const RankFuse& rf, int dev,
+                         long long pairs, cudaStream_t st) {
+  return rf.q_tags ? launch_search<BN, EPI_SEARCH_EXCL>(tmA, tmB, ga, rf, dev, pairs, st)
+                   : launch_search<BN, EPI_SEARCH>(tmA, tmB, ga, rf, dev, pairs, st);
+}
+
+// g_tags / q_tags: both null (no exclusion) or both set (pps_search_topk_excl_tc)
+static int search_topk_impl(const void* g_planes, const float* g_sqnorm, long long ng, int g_planes_n, long long g_plane_rows,
+                            const void* q_planes, const float* q_sqnorm, long long nq, int q_planes_n, long long q_plane_rows,
+                            int dim, int precision, int flags, long long col0, const uint32_t* tk_bound, uint32_t* tk_cnt,
+                            uint64_t* tk_cand, int tk_cap, const int64_t* g_tags, const int64_t* q_tags, void* stream) {
   if (ng < 0 || nq < 0 || dim <= 0 || col0 < 0 || tk_cap < 1) return PPS_ERR_INVALID_ARG;
   if (flags & ~(PPS_DIST_SQUARED | PPS_DIST_SQRT_RN)) return PPS_ERR_INVALID_ARG;   // keys order by the bits of a distance
   if (g_plane_rows == 0) g_plane_rows = ng;
@@ -1068,6 +1086,7 @@ extern "C" int pps_search_topk_tc(const void* g_planes, const float* g_sqnorm, l
   RankFuse rf{};
   rf.col0 = col0;
   rf.tk_bound = tk_bound; rf.tk_cnt = tk_cnt; rf.tk_cand = reinterpret_cast<unsigned long long*>(tk_cand); rf.tk_cap = tk_cap;
+  rf.g_tags = reinterpret_cast<const long long*>(g_tags); rf.q_tags = reinterpret_cast<const long long*>(q_tags);
   int dev = 0;
   PPS_CUDA_TRY(cudaGetDevice(&dev));
   const long long tiles = (long long)g.m_tiles * g.n_tiles;
@@ -1079,6 +1098,26 @@ extern "C" int pps_search_topk_tc(const void* g_planes, const float* g_sqnorm, l
     case 128: return launch_search<128>(tmA, tmB, ga, rf, dev, pairs, st);
     default: return launch_search<256>(tmA, tmB, ga, rf, dev, pairs, st);
   }
+}
+
+extern "C" int pps_search_topk_tc(const void* g_planes, const float* g_sqnorm, long long ng, int g_planes_n,
+                                  long long g_plane_rows, const void* q_planes, const float* q_sqnorm, long long nq,
+                                  int q_planes_n, long long q_plane_rows, int dim, int precision, int flags, long long col0,
+                                  const uint32_t* tk_bound, uint32_t* tk_cnt, uint64_t* tk_cand, int tk_cap, void* stream) {
+  return search_topk_impl(g_planes, g_sqnorm, ng, g_planes_n, g_plane_rows, q_planes, q_sqnorm, nq, q_planes_n, q_plane_rows,
+                          dim, precision, flags, col0, tk_bound, tk_cnt, tk_cand, tk_cap, nullptr, nullptr, stream);
+}
+
+// pps_search_topk_tc without the pairs whose tags are equal: row r of the block is no candidate of query q when
+// g_tags[r] == q_tags[q].  The tags are compared only for elements that pass the bound.
+extern "C" int pps_search_topk_excl_tc(const void* g_planes, const float* g_sqnorm, long long ng, int g_planes_n,
+                                       long long g_plane_rows, const void* q_planes, const float* q_sqnorm, long long nq,
+                                       int q_planes_n, long long q_plane_rows, int dim, int precision, int flags,
+                                       long long col0, const uint32_t* tk_bound, uint32_t* tk_cnt, uint64_t* tk_cand,
+                                       int tk_cap, void* stream, const int64_t* g_tags, const int64_t* q_tags) {
+  if (ng > 0 && nq > 0 && (!g_tags || !q_tags)) return PPS_ERR_INVALID_ARG;
+  return search_topk_impl(g_planes, g_sqnorm, ng, g_planes_n, g_plane_rows, q_planes, q_sqnorm, nq, q_planes_n, q_plane_rows,
+                          dim, precision, flags, col0, tk_bound, tk_cnt, tk_cand, tk_cap, g_tags, q_tags, stream);
 }
 
 extern "C" int pps_dist_fp32(const float* a, long long lda, const float* a_sqnorm, long long m1, const float* b,
@@ -1246,6 +1285,7 @@ extern "C" int pps_dist_rank_topk_tc(const void* a_planes, const float* a_sqnorm
   rf.tk_bound = tk_cand ? tk_bound : nullptr; rf.tk_cnt = tk_cand ? tk_cnt : nullptr;
   rf.tk_cand = reinterpret_cast<unsigned long long*>(tk_cand); rf.tk_cap = tk_cand ? tk_cap : 0;
   rf.progress = nullptr; rf.window = 0;
+  rf.g_tags = nullptr; rf.q_tags = nullptr;
   static thread_local int configured_dev = -1;
   int dev = 0;
   PPS_CUDA_TRY(cudaGetDevice(&dev));

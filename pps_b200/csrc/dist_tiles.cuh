@@ -59,6 +59,9 @@ struct RankFuse {
   // done); a producer starts tile j only when j <= min over its stream + window.  window = 0: off.
   uint32_t* progress;
   int window;
+  // EPI_SEARCH_EXCL: row r of the block is no candidate of query q when g_tags[r] == q_tags[q]
+  const long long* g_tags;  // [rows of the block]
+  const long long* q_tags;  // [queries]
 };
 
 constexpr int EPI_DIST = 0;          // |a|^2 + |b|^2 - 2ab, clamp, sqrt (or squared / raw dot by flags) -> matrix
@@ -66,9 +69,11 @@ constexpr int EPI_AFFINE_RELU = 1;   // max(0, dot * alpha[col] + beta[col])   (
 constexpr int EPI_RANK = 2;          // distance as EPI_DIST, consumed by the counting epilogue; no matrix
 constexpr int EPI_DIST_TOPK = 3;     // EPI_DIST + one compare per element against the row's top-k admission bound
 constexpr int EPI_SEARCH = 4;        // A = gallery, B = queries: distance -> top-k admission per COLUMN; no matrix
+constexpr int EPI_SEARCH_EXCL = 5;   // EPI_SEARCH without the (row, query) pairs whose tags are equal
+__host__ __device__ constexpr bool epi_search(int epi) { return epi == EPI_SEARCH || epi == EPI_SEARCH_EXCL; }
 
 // Tile order.  EPI_DIST / EPI_AFFINE_RELU: tile t = pair, pair + npairs, ... with the m index fastest, so that the
-// CTA pairs running concurrently share B tiles in L2.  EPI_SEARCH: the same tiles with the n index fastest, so that a
+// CTA pairs running concurrently share B tiles in L2.  EPI_SEARCH(_EXCL): the same tiles with the n index fastest, so that a
 // gallery (m) tile is read from HBM once and its other query tiles find it in L2.  EPI_RANK: a CTA pair keeps ONE m tile per run (its rows'
 // thresholds and counters stay in shared memory) and walks a contiguous range of n tiles.
 //   npairs >= m_tiles: k = npairs / m_tiles pairs per m tile walk n tiles [0, Na) in k aligned parts - the pairs that own
@@ -126,7 +131,7 @@ struct TileWalk {
       if (t >= tiles) return false;
       grp = t / tiles_per_group;
       const long long tt = t % tiles_per_group;
-      if (EPI == EPI_SEARCH) {
+      if (epi_search(EPI)) {
         m_tile = (int)(tt / n_tiles);
         n_tile = (int)(tt % n_tiles);
       } else {

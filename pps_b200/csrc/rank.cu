@@ -485,22 +485,32 @@ __global__ void __launch_bounds__(128) rank_finalize_kernel(long long nq, const 
 // key = (float bits << 32) | global gallery index: unsigned order == (distance, index) order
 // for the non-negative distances this path produces.
 // ------------------------------------------------------------------------------------
+// TAGS (a separate instance, so that the untagged sweep keeps its registers and occupancy): column c is skipped when
+// g_tags[c] == q_tags[q].  The tag is compared at admission only, unless the excluded columns are counted (n_tag_excl
+// set): then every column's tag is read.
+template <bool TAGS>
 __global__ void __launch_bounds__(kTopkThreads) topk_update_kernel(const float* __restrict__ dist, long long ldd,
                                                                     long long ncols, long long col0,
                                                                     const int32_t* __restrict__ excl_off,
                                                                     const int32_t* __restrict__ excl_g,
                                                                     const uint8_t* __restrict__ excl_keep,
+                                                                    const long long* __restrict__ g_tags,
+                                                                    const long long* __restrict__ q_tags,
+                                                                    uint32_t* __restrict__ n_tag_excl,
                                                                     unsigned long long* __restrict__ topk_key, int k) {
   __shared__ unsigned long long cand[kCand];
   __shared__ int s_n;
   __shared__ unsigned long long s_bound;
+  __shared__ uint32_t s_excl;
   const int q = blockIdx.x, tid = threadIdx.x;
   unsigned long long* state = topk_key + (long long)q * k;
   for (int i = tid; i < kCand; i += kTopkThreads) cand[i] = i < k ? state[i] : ~0ull;
-  if (tid == 0) { s_n = k; s_bound = state[k - 1]; }
+  if (tid == 0) { s_n = k; s_bound = state[k - 1]; if (TAGS) s_excl = 0u; }
   __syncthreads();
   const float* drow = dist + (long long)q * ldd;
   const int x0 = excl_off ? excl_off[q] : 0, x1 = excl_off ? excl_off[q + 1] : 0;
+  const long long qtag = TAGS ? q_tags[q] : 0;
+  uint32_t n_tx = 0;
   const long long tile = 4LL * kTopkThreads;
   for (long long c0 = 0; c0 < ncols; c0 += tile) {
     const unsigned long long bound = s_bound;
@@ -510,8 +520,14 @@ __global__ void __launch_bounds__(kTopkThreads) topk_update_kernel(const float* 
       if (c < ncols) {
         const float d = ld_stream_f32(drow + c);
         const unsigned long long key = ((unsigned long long)__float_as_uint(d) << 32) | (unsigned long long)(uint32_t)(col0 + c);
+        bool tag_out = false;
+        if (TAGS && n_tag_excl) {
+          tag_out = __ldg(g_tags + c) == qtag;
+          n_tx += tag_out;
+        }
         if (key < bound) {
-          bool skip = false;
+          if (TAGS && !n_tag_excl) tag_out = __ldg(g_tags + c) == qtag;
+          bool skip = tag_out;
           for (int x = x0; x < x1; ++x)
             skip |= ((long long)excl_g[x] == col0 + c) && !(excl_keep && excl_keep[x]);
           if (!skip) {
@@ -533,6 +549,11 @@ __global__ void __launch_bounds__(kTopkThreads) topk_update_kernel(const float* 
   }
   bitonic_sort_smem(cand, kCand, tid, kTopkThreads);
   for (int i = tid; i < k; i += kTopkThreads) state[i] = cand[i];
+  if (TAGS && n_tag_excl) {
+    if (n_tx) atomicAdd(&s_excl, n_tx);
+    __syncthreads();
+    if (tid == 0) n_tag_excl[q] = s_excl;
+  }
 }
 
 __global__ void topk_fill_kernel(unsigned long long* p, long long n) {
@@ -905,9 +926,28 @@ extern "C" int pps_topk_update(const float* dist, long long ldd, long long nq, l
   if (!dist || !topk_key) return PPS_ERR_INVALID_ARG;
   if (excl_off && !excl_g) return PPS_ERR_INVALID_ARG;
   if (nq > 0x7fffffffLL || col0 + ncols > 0xffffffffLL) return PPS_ERR_UNSUPPORTED;
-  topk_update_kernel<<<(unsigned)nq, kTopkThreads, 0, static_cast<cudaStream_t>(stream)>>>(
-      dist, ldd, ncols, col0, excl_off, excl_g, excl_keep, reinterpret_cast<unsigned long long*>(topk_key), k);
+  topk_update_kernel<false><<<(unsigned)nq, kTopkThreads, 0, static_cast<cudaStream_t>(stream)>>>(
+      dist, ldd, ncols, col0, excl_off, excl_g, excl_keep, nullptr, nullptr, nullptr,
+      reinterpret_cast<unsigned long long*>(topk_key), k);
   PPS_LAUNCH_CHECK("topk_update_kernel");
+  return PPS_OK;
+}
+
+extern "C" int pps_topk_update_excl(const float* dist, long long ldd, long long nq, long long ncols, long long col0,
+                                    const int64_t* g_tags, const int64_t* q_tags, uint64_t* topk_key, int k,
+                                    uint32_t* n_excluded, void* stream) {
+  if (nq < 0 || ncols < 0 || ldd < ncols || k < 1 || k > PPS_TOPK_MAX) return PPS_ERR_INVALID_ARG;
+  if (nq == 0) return PPS_OK;
+  if (!topk_key || !q_tags || (ncols > 0 && (!dist || !g_tags))) return PPS_ERR_INVALID_ARG;
+  if (nq > 0x7fffffffLL || col0 + ncols > 0xffffffffLL) return PPS_ERR_UNSUPPORTED;
+  if (ncols == 0) {
+    if (n_excluded) PPS_CUDA_TRY(cudaMemsetAsync(n_excluded, 0, (size_t)nq * sizeof(uint32_t), static_cast<cudaStream_t>(stream)));
+    return PPS_OK;
+  }
+  topk_update_kernel<true><<<(unsigned)nq, kTopkThreads, 0, static_cast<cudaStream_t>(stream)>>>(
+      dist, ldd, ncols, col0, nullptr, nullptr, nullptr, reinterpret_cast<const long long*>(g_tags),
+      reinterpret_cast<const long long*>(q_tags), n_excluded, reinterpret_cast<unsigned long long*>(topk_key), k);
+  PPS_LAUNCH_CHECK("topk_update_kernel<excl>");
   return PPS_OK;
 }
 

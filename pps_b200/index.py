@@ -3,7 +3,15 @@
 The gallery is split into tensor-core operand planes once, when rows are added (C ABI part 2h, ``pps_index_*``); a search
 splits only the queries and streams the resident planes, the gallery as the 256-row side of every MMA
 (``pps_search_topk_tc``).  Distances and order are those of ``compute_dist`` / ``rank_eval``'s top-k: Euclidean, smallest
-first, ties by gallery index, no id or camera filter.
+first, ties by gallery index.
+
+Rows may carry one int64 tag each (``add(feats, tags)``), and a search may leave out, for every query, the rows whose
+tag equals the query's exclude tag (``search(q, k, exclude_tags)``); the test runs inside the search kernels.  Two
+encodings cover person retrieval:
+
+- cross-camera search: ``tags = gallery cameras``, ``exclude_tags = query cameras``;
+- the evaluation protocol's junk rule (same id and same camera): ``tag = (id << 32) | camera`` for ids in int32 and
+  cameras in [0, 2^32), on both sides.  The result then equals ``rank_eval(..., topk=k)`` bit for bit.
 """
 from __future__ import annotations
 
@@ -27,6 +35,13 @@ class GalleryIndex:
     With ``group`` every rank adds its own rows and ``search`` is collective: one all-gather of the shard sizes (a shard's
     indices start after the rows of the ranks before it) and one of the keys; every rank gets the result of one index
     holding the concatenated shards.
+
+    ``add(feats, tags)`` gives every row an integer tag (numpy or torch, [n], converted to int64 on the index's device);
+    the first non-empty add decides whether the index is tagged, and a later add of the other kind raises.
+    ``search(q, k, exclude_tags)`` ([nq] integers) leaves row r out of query i's result when
+    ``tags[r] == exclude_tags[i]`` and pads with -1 / inf when fewer than k rows remain; it needs a tagged index (an
+    empty one answers with padding).  Without ``exclude_tags`` the tags are ignored.  Sharded: every rank passes the
+    same exclude tags and its own rows' tags.
     """
 
     def __init__(self, dim, dtype=None, precision="f16x3", device=None, group=None):
@@ -75,28 +90,55 @@ class GalleryIndex:
             x = x.contiguous()
         return x, is_np
 
-    def add(self, feats):
-        """Append rows; returns (row0, rows), their range among this index's (local) rows."""
+    def _tags(self, t, n, name):
+        """[n] int64 CUDA tensor on the index's device from integer numpy or torch tags"""
+        import torch
+        if isinstance(t, np.ndarray):
+            if not np.issubdtype(t.dtype, np.integer):
+                raise RuntimeError("%s: expected integer tags, got %s" % (name, t.dtype))
+            t = torch.from_numpy(np.ascontiguousarray(t, dtype=np.int64))
+        elif isinstance(t, torch.Tensor):
+            if t.dtype.is_floating_point or t.dtype.is_complex or t.dtype == torch.bool:
+                raise RuntimeError("%s: expected integer tags, got %s" % (name, t.dtype))
+        else:
+            raise RuntimeError("%s: expected numpy.ndarray or torch.Tensor, got %s" % (name, type(t)))
+        if t.dim() != 1 or int(t.shape[0]) != n:
+            raise RuntimeError("%s: expected shape [%d], got %s" % (name, n, tuple(t.shape)))
+        return t.to(device=self.device, dtype=torch.int64).contiguous()
+
+    def add(self, feats, tags=None):
+        """Append rows (with their tags); returns (row0, rows), their range among this index's (local) rows."""
         import torch
         x, _ = self._rows(feats, "feats")
         row0, n = len(self), int(x.shape[0])
+        ld = int(x.stride(0)) if n else self.dim
         with torch.cuda.device(self.device):
-            _lib.check(self._lib.pps_index_add(self._h, _lib.ptr(x), n, int(x.stride(0)) if n else self.dim,
-                                               _lib.stream_ptr()), "pps_index_add")
+            if tags is None:
+                _lib.check(self._lib.pps_index_add(self._h, _lib.ptr(x), n, ld, _lib.stream_ptr()), "pps_index_add")
+            else:
+                t = self._tags(tags, n, "tags")
+                _lib.check(self._lib.pps_index_add_tagged(self._h, _lib.ptr(x), n, ld, _lib.ptr(t), _lib.stream_ptr()),
+                           "pps_index_add_tagged")
         return row0, n
 
-    def _search_keys(self, q, k, index_offset=0, flags=0):
+    def _search_keys(self, q, k, index_offset=0, flags=0, exclude_tags=None):
         """[nq, k] top-k keys (distance bits << 32 | index_offset + row) of this index alone; flags: PPS_INDEX_* hooks."""
         import torch
         x, is_np = self._rows(q, "q")
         if not isinstance(k, (int, np.integer)) or not 1 <= int(k) <= _lib.TOPK_MAX:
             raise RuntimeError("k must be an integer in [1, %d], got %r" % (_lib.TOPK_MAX, k))
         nq, k = int(x.shape[0]), int(k)
+        ldq = int(x.stride(0)) if nq else self.dim
         keys = torch.empty((nq, k), dtype=torch.int64, device=self.device)
         with torch.cuda.device(self.device):
-            _lib.check(self._lib.pps_index_search(self._h, _lib.ptr(x), nq, int(x.stride(0)) if nq else self.dim, k,
-                                                  int(index_offset), int(flags), _lib.stream_ptr(), _lib.ptr(keys)),
-                       "pps_index_search")
+            if exclude_tags is None:
+                _lib.check(self._lib.pps_index_search(self._h, _lib.ptr(x), nq, ldq, k, int(index_offset), int(flags),
+                                                      _lib.stream_ptr(), _lib.ptr(keys)), "pps_index_search")
+            else:
+                t = self._tags(exclude_tags, nq, "exclude_tags")
+                _lib.check(self._lib.pps_index_search_excluding(self._h, _lib.ptr(x), nq, ldq, _lib.ptr(t), k,
+                                                                int(index_offset), int(flags), _lib.stream_ptr(),
+                                                                _lib.ptr(keys)), "pps_index_search_excluding")
         return keys, is_np
 
     def _unpack(self, keys, is_np):
@@ -112,8 +154,9 @@ class GalleryIndex:
             return dist.cpu().numpy(), index.cpu().numpy()
         return dist, index
 
-    def search(self, q, k):
-        """(dist [nq, k] float32, index [nq, k] int64) of the k nearest gallery rows of every query row."""
+    def search(self, q, k, exclude_tags=None):
+        """(dist [nq, k] float32, index [nq, k] int64) of the k nearest gallery rows of every query row (with
+        exclude_tags: of the rows whose tag is not the query's)."""
         import torch
         offset = 0
         if self.group is not None:
@@ -122,7 +165,7 @@ class GalleryIndex:
             sizes = [torch.empty_like(mine) for _ in range(dist_mod.get_world_size(self.group))]
             dist_mod.all_gather(sizes, mine, group=self.group)
             offset = int(sum(int(s.item()) for s in sizes[:dist_mod.get_rank(self.group)]))
-        keys, is_np = self._search_keys(q, k, offset)
+        keys, is_np = self._search_keys(q, k, offset, exclude_tags=exclude_tags)
         if self.group is not None:
             keys = merge_topk_keys(keys, int(k), self.group)
         return self._unpack(keys, is_np)
