@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define PPS_ABI_VERSION 7
+#define PPS_ABI_VERSION 8
 
 /* ---- error codes (the Python mirror turns every non-zero code into RuntimeError,
  * like CAFFE_ENFORCE does: detectron/tests/test_zero_even_op.py:50-53) ---- */
@@ -575,12 +575,27 @@ int pps_evaluate_host(const float* q_feats, long long nq,
  *                      padded with -1 / inf.  Same schedule with the excluding kernels; when the gallery is larger than
  *                      the prefix, the prefix sweep counts every query's excluded rows and one more 4-byte read-back
  *                      (the largest count) shrinks the chunks by the excluded share (at most 0.9).
+ * pps_index_remove     deletes the local rows d_rows[n] (device int64, any order, duplicates allowed) with np.delete's
+ *                      renumbering: every later row moves down by the number of removed rows before it, and the size
+ *                      shrinks by the number of distinct rows removed (*n_removed, host, may be null).  The index is then
+ *                      the index a fresh pps_index_create + add of the remaining rows in their order (with their tags)
+ *                      gives, so every later search returns that index's answer bit for bit.  A row < 0 or >= size:
+ *                      PPS_ERR_INVALID_ARG and the index is unchanged.  n = 0 does nothing.  The capacity is not reduced;
+ *                      an index emptied by removal decides again at its next non-empty add whether it is tagged.  The
+ *                      rows are compacted on the device: one byte per row marks the removed rows, a scan lists the
+ *                      live rows after the first removed one, and these move down in pieces through an index-owned
+ *                      buffer of at most 256 MiB (about 5 bytes of scratch per row besides it).  d_rows has been read
+ *                      when the call returns: one 24-byte read-back is its only synchronisation, the moves stay queued
+ *                      on `stream`.  flags: 0, or the test hook PPS_INDEX_PIECE(n) (at most n rows per piece).  Sharded:
+ *                      removal is local (a rank removes its own rows); the next search's all-gather of the shard sizes
+ *                      moves the global offsets.
  * Calls on one index are ordered by the caller (one stream, or events between streams); every call sets the index's
  * device for its duration.  A sharded gallery: one index per rank, index_offset = the rows of the ranks before, an
  * all-gather of the [nq][k] keys and the k smallest per query (every rank's list is sorted, keys are unique).
  * ---------------------------------------------------------------------------------- */
 #define PPS_INDEX_TKCAP(n)  (((n) & 0xffff) << 8)
 #define PPS_INDEX_PREFIX(n) (((n) & 0x7f) << 24)
+#define PPS_INDEX_PIECE(n)  (((n) & 0xffff) << 8)   /* pps_index_remove only */
 int pps_search_topk_tc(const void* g_planes, const float* g_sqnorm, long long ng, int g_planes_n, long long g_plane_rows,
                        const void* q_planes, const float* q_sqnorm, long long nq, int q_planes_n, long long q_plane_rows,
                        int dim, int precision, int flags, long long col0, const uint32_t* tk_bound, uint32_t* tk_cnt,
@@ -605,6 +620,8 @@ int       pps_index_search(pps_index* idx, const void* d_q, long long nq, long l
 int       pps_index_search_excluding(pps_index* idx, const void* d_q, long long nq, long long ldq,
                                      const int64_t* d_q_tags, int k, long long index_offset, int flags, void* stream,
                                      uint64_t* d_keys);
+int       pps_index_remove(pps_index* idx, const int64_t* d_rows, long long n, int flags, void* stream,
+                           long long* n_removed);
 
 /* ------------------------------------------------------------------------------------
  * Next row (SURVEY §8f.4) — the reference's training-side triplet mining ops.

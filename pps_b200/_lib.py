@@ -13,7 +13,7 @@ import threading
 from . import build as _build
 
 # ---- constants (keep in sync with include/pps_b200.h) ----
-ABI_VERSION = 7
+ABI_VERSION = 8
 PPS_OK = 0
 PPS_ERR_INVALID_ARG = -1
 PPS_ERR_SHAPE = -2
@@ -37,6 +37,11 @@ def index_tkcap(n: int) -> int:
 def index_prefix(n: int) -> int:
     """PPS_INDEX_PREFIX(n): pps_index_search test hook, n * 256 rows in the materialised prefix."""
     return (n & 0x7f) << 24
+
+
+def index_piece(n: int) -> int:
+    """PPS_INDEX_PIECE(n): pps_index_remove test hook, at most n rows per move piece."""
+    return (n & 0xffff) << 8
 
 POOL_AVG_MAX = 0
 POOL_MAX_AVE = 1
@@ -156,6 +161,7 @@ SIGNATURES = {
     "pps_topk_update_excl": (_i, [_vp, _ll, _ll, _ll, _ll, _vp, _vp, _vp, _i, _vp, _vp]),
     "pps_index_add_tagged": (_i, [_vp, _vp, _ll, _ll, _vp, _vp]),
     "pps_index_search_excluding": (_i, [_vp, _vp, _ll, _ll, _vp, _i, _ll, _i, _vp, _vp]),
+    "pps_index_remove": (_i, [_vp, _vp, _ll, _i, _vp, C.POINTER(_ll)]),
     "pps_pairwise_distance_fwd": (_i, [_vp, _i, _i, _vp, _vp]),
     "pps_pairwise_distance_bwd": (_i, [_vp, _vp, _i, _i, _vp, _vp]),
     "pps_batch_hard_fwd": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _vp]),

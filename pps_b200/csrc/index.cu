@@ -16,6 +16,17 @@
 // candidates.  A query whose excluded rows fill a fraction f of the prefix got its bound from F (1 - f) rows, and a chunk
 // of rows it may all take admits up to k R / (F (1 - f)): the prefix sweep counts each query's excluded rows, one 4-byte
 // read-back gives the largest count, and the chunks shrink by (1 - f^), f^ <= 0.9.
+//
+// Removal (pps_index_remove) compacts the rows in place, with np.delete's renumbering:
+//   1. mark: one byte per row (rm_flag), set for every listed row; out-of-range rows are counted, the first removed row
+//      is an atomicMin.  Block sums of the flags, one block scans them (exclusive offsets + the number removed), and one
+//      12-byte read-back {out of range, removed, first} is the call's only synchronisation.
+//   2. kept list: the live rows of [first, size) in order (int32), from the scanned offsets.
+//   3. move, in pieces [j0, j1) of the kept list: gather rows kept[j0..j1) of every plane, their norms / inverse scales
+//      and tags into the piece buffer, then cudaMemcpyAsync it to rows [first + j0, first + j1).  kept[j] >= first + j,
+//      so a piece's destinations overlap only its own sources (already in the buffer) or earlier pieces' (already read).
+// The moved rows are the bytes a fresh add of the remaining rows would have written (the split is per row), so every
+// later search equals a fresh index's bit for bit.
 #include "ctx.cuh"
 
 namespace {
@@ -51,6 +62,7 @@ struct pps_index {
   int64_t* g_tags = nullptr;    // [capacity] row tags (tagged indexes)
   bool tagged = false;          // decided by the first non-empty add
   GrowBuf qs, qn, dist, tk_bound, tk_cnt, tk_cand, flag, n_excl;
+  GrowBuf rm_flag, rm_bsum, rm_stat, rm_kept, rm_piece;    // scratch of pps_index_remove
   PinBuf flag_h;
   bool scaled() const { return precision == PPS_PREC_F16X3; }
   size_t plane_bytes(long long rows) const { return (size_t)rows * kpad * 2; }
@@ -121,6 +133,142 @@ __global__ void max_u32_kernel(const uint32_t* __restrict__ v, long long n, uint
   if (threadIdx.x == 0) *out = s_max;
 }
 
+// ---- removal (pps_index_remove) ----
+constexpr int kRmThreads = 256;
+constexpr int kRmTile = kRmThreads * 16;            // rows per block of the flag scan: 16 one-byte flags per thread
+constexpr size_t kRmPieceBytes = 256ull << 20;      // the piece buffer of the move
+constexpr unsigned long long kRmNone = ~0ull;
+
+// exclusive prefix of v over the block (blockDim.x a multiple of 32, <= 1024) and the block's total
+__device__ __forceinline__ uint32_t block_excl_scan(uint32_t v, uint32_t* s_warp, uint32_t* total) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
+  uint32_t x = v;
+  for (int o = 1; o < 32; o <<= 1) {
+    const uint32_t y = __shfl_up_sync(~0u, x, o);
+    if (lane >= o) x += y;
+  }
+  if (lane == 31) s_warp[warp] = x;
+  __syncthreads();
+  if (warp == 0) {
+    uint32_t w = lane < nw ? s_warp[lane] : 0u;
+    for (int o = 1; o < 32; o <<= 1) {
+      const uint32_t y = __shfl_up_sync(~0u, w, o);
+      if (lane >= o) w += y;
+    }
+    s_warp[lane] = w;
+  }
+  __syncthreads();
+  *total = s_warp[nw - 1];
+  const uint32_t r = (warp ? s_warp[warp - 1] : 0u) + x - v;
+  __syncthreads();                                   // s_warp is reused by the caller's next scan
+  return r;
+}
+
+// flags of 16 rows (one byte each, 0 or 1) -> how many are set
+__device__ __forceinline__ uint32_t flag_count(uint4 v) { return __popc(v.x) + __popc(v.y) + __popc(v.z) + __popc(v.w); }
+
+// stat: [0] listed rows out of [0, size), [1] distinct rows removed (rm_scan_kernel), [2] first removed row (kRmNone: none)
+__global__ void __launch_bounds__(kRmThreads) rm_mark_kernel(const int64_t* __restrict__ rows, long long n, long long size,
+                                                             uint8_t* __restrict__ flag, unsigned long long* __restrict__ stat) {
+  unsigned long long bad = 0, first = kRmNone;
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+    const long long r = rows[i];
+    if (r < 0 || r >= size) {
+      ++bad;
+    } else {
+      flag[r] = 1;                                   // a duplicate writes the same byte again
+      first = min(first, (unsigned long long)r);
+    }
+  }
+  for (int o = 16; o; o >>= 1) {
+    bad += __shfl_xor_sync(~0u, bad, o);
+    first = min(first, __shfl_xor_sync(~0u, first, o));
+  }
+  if ((threadIdx.x & 31) == 0) {
+    if (bad) atomicAdd(stat, bad);
+    if (first != kRmNone) atomicMin(stat + 2, first);
+  }
+}
+
+// bsum[b] = flags set among rows [b * kRmTile, (b + 1) * kRmTile)
+__global__ void __launch_bounds__(kRmThreads) rm_count_kernel(const uint8_t* __restrict__ flag, uint32_t* __restrict__ bsum) {
+  __shared__ uint32_t s_warp[32];
+  const uint4 v = reinterpret_cast<const uint4*>(flag)[(size_t)blockIdx.x * kRmThreads + threadIdx.x];
+  uint32_t total;
+  block_excl_scan(flag_count(v), s_warp, &total);
+  if (threadIdx.x == 0) bsum[blockIdx.x] = total;
+}
+
+// one block: bsum -> its exclusive prefix sums (rows removed before each tile), stat[1] = their total
+__global__ void __launch_bounds__(1024) rm_scan_kernel(uint32_t* __restrict__ bsum, long long nblk,
+                                                       unsigned long long* __restrict__ stat) {
+  __shared__ uint32_t s_warp[32];
+  uint32_t carry = 0;                                // < 2^31: the index holds fewer rows
+  for (long long base = 0; base < nblk; base += blockDim.x) {
+    const long long i = base + threadIdx.x;
+    const uint32_t v = i < nblk ? bsum[i] : 0u;
+    uint32_t total;
+    const uint32_t e = block_excl_scan(v, s_warp, &total);
+    if (i < nblk) bsum[i] = carry + e;
+    carry += total;
+  }
+  if (threadIdx.x == 0) stat[1] = carry;
+}
+
+// kept[j] = the j-th live row of [first, size), for the tiles b0, b0 + 1, ... (boff: rm_scan_kernel's offsets).  A live
+// row r has boff + (flags set before r in its tile) removed rows before it, all >= first.
+__global__ void __launch_bounds__(kRmThreads) rm_fill_kernel(const uint8_t* __restrict__ flag, const uint32_t* __restrict__ boff,
+                                                             long long b0, long long first, long long size,
+                                                             int32_t* __restrict__ kept) {
+  __shared__ uint32_t s_warp[32];
+  const long long b = b0 + blockIdx.x;
+  const uint4 v = reinterpret_cast<const uint4*>(flag)[(size_t)b * kRmThreads + threadIdx.x];
+  uint32_t total;
+  uint32_t removed = boff[b] + block_excl_scan(flag_count(v), s_warp, &total);
+  const uint32_t w[4] = {v.x, v.y, v.z, v.w};
+  const long long r0 = b * kRmTile + (long long)threadIdx.x * 16;
+#pragma unroll
+  for (int i = 0; i < 16; ++i) {
+    const long long r = r0 + i;
+    const uint32_t f = (w[i >> 2] >> ((i & 3) * 8)) & 1u;
+    if (!f && r >= first && r < size) kept[r - first - removed] = (int32_t)r;
+    removed += f;
+  }
+}
+
+// one warp per piece row j < rows: source row kept[j] of every plane (vec 16-byte words per row, plane_vec words between
+// planes) -> row j of the piece's planes (piece_vec words between them), and its norm / inverse scale / tag
+__global__ void __launch_bounds__(kRmThreads) rm_gather_kernel(const int32_t* __restrict__ kept, long long rows, int planes,
+                                                               int vec, const float4* __restrict__ src, long long plane_vec,
+                                                               const float* __restrict__ norm, const float* __restrict__ scale,
+                                                               const int64_t* __restrict__ tags, float4* __restrict__ piece,
+                                                               long long piece_vec, float* __restrict__ p_norm,
+                                                               float* __restrict__ p_scale, int64_t* __restrict__ p_tags) {
+  const long long j = blockIdx.x * (long long)(kRmThreads / 32) + (threadIdx.x >> 5);
+  if (j >= rows) return;
+  const int lane = threadIdx.x & 31;
+  const long long r = kept[j];
+  for (int p = 0; p < planes; ++p) {
+    const float4* s = src + p * plane_vec + r * vec;
+    float* d = reinterpret_cast<float*>(piece + p * piece_vec + j * vec);
+    int i = lane;
+    for (; i + 96 < vec; i += 128) {                 // four 16-byte loads in flight per lane
+      const float4 a = pps::ld_stream_f4(s + i), b = pps::ld_stream_f4(s + i + 32);
+      const float4 c = pps::ld_stream_f4(s + i + 64), e = pps::ld_stream_f4(s + i + 96);
+      pps::st_stream_f4(d + 4 * i, a);
+      pps::st_stream_f4(d + 4 * (i + 32), b);
+      pps::st_stream_f4(d + 4 * (i + 64), c);
+      pps::st_stream_f4(d + 4 * (i + 96), e);
+    }
+    for (; i < vec; i += 32) pps::st_stream_f4(d + 4 * i, pps::ld_stream_f4(s + i));
+  }
+  if (lane == 0) {
+    p_norm[j] = norm[r];
+    if (scale) p_scale[j] = scale[r];
+    if (tags) p_tags[j] = tags[r];
+  }
+}
+
 }  // namespace
 
 extern "C" int pps_index_create(int device, int dim, int dtype, int precision, pps_index** out) {
@@ -159,7 +307,8 @@ extern "C" int pps_index_destroy(pps_index* x) {
   if (x->g_planes) cudaFree(x->g_planes);
   if (x->g_norm) cudaFree(x->g_norm);
   if (x->g_tags) cudaFree(x->g_tags);
-  GrowBuf* bufs[] = {&x->qs, &x->qn, &x->dist, &x->tk_bound, &x->tk_cnt, &x->tk_cand, &x->flag, &x->n_excl};
+  GrowBuf* bufs[] = {&x->qs,     &x->qn,      &x->dist,    &x->tk_bound, &x->tk_cnt,  &x->tk_cand, &x->flag,
+                     &x->n_excl, &x->rm_flag, &x->rm_bsum, &x->rm_stat,  &x->rm_kept, &x->rm_piece};
   for (GrowBuf* b : bufs) b->release();
   x->flag_h.release();
   delete x;
@@ -293,4 +442,83 @@ extern "C" int pps_index_search_excluding(pps_index* x, const void* d_q, long lo
   if (nq > 0 && !d_q_tags) return PPS_ERR_INVALID_ARG;
   if (x->size > 0 && !x->tagged) return PPS_ERR_INVALID_ARG;     // nothing to compare the query tags with
   return search(x, d_q, nq, ldq, d_q_tags, k, index_offset, flags, stream, d_keys);
+}
+
+extern "C" int pps_index_remove(pps_index* x, const int64_t* d_rows, long long n, int flags, void* stream,
+                                long long* n_removed) {
+  if (n_removed) *n_removed = 0;
+  if (!x || n < 0 || (flags & ~PPS_INDEX_PIECE(0xffff))) return PPS_ERR_INVALID_ARG;
+  if (n == 0) return PPS_OK;
+  if (!d_rows || x->size == 0) return PPS_ERR_INVALID_ARG;      // (an empty index has no row to remove)
+  DeviceGuard dg(x->device);
+  if (dg.err != cudaSuccess) return pps::cuda_fail(dg.err, "cudaSetDevice");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const long long size = x->size;
+  const long long nblk = (size + kRmTile - 1) / kRmTile;
+  PPS_TRY(x->rm_flag.ensure((size_t)nblk * kRmTile));
+  PPS_TRY(x->rm_bsum.ensure((size_t)nblk * 4));
+  PPS_TRY(x->rm_stat.ensure(3 * 8));
+  PPS_TRY(x->flag_h.ensure(3 * 8));
+  uint8_t* flag = x->rm_flag.as<uint8_t>();
+  uint32_t* bsum = x->rm_bsum.as<uint32_t>();
+  unsigned long long* stat = x->rm_stat.as<unsigned long long>();
+
+  // 1. mark, count, scan; one read-back
+  PPS_CUDA_TRY(cudaMemsetAsync(flag, 0, (size_t)nblk * kRmTile, st));
+  PPS_CUDA_TRY(cudaMemsetAsync(stat, 0, 2 * 8, st));
+  PPS_CUDA_TRY(cudaMemsetAsync(stat + 2, 0xff, 8, st));
+  const long long mark_blocks = std::min<long long>((n + kRmThreads - 1) / kRmThreads, (long long)pps::sm_count() * 8);
+  rm_mark_kernel<<<(unsigned)mark_blocks, kRmThreads, 0, st>>>(d_rows, n, size, flag, stat);
+  PPS_LAUNCH_CHECK("rm_mark_kernel");
+  rm_count_kernel<<<(unsigned)nblk, kRmThreads, 0, st>>>(flag, bsum);
+  PPS_LAUNCH_CHECK("rm_count_kernel");
+  rm_scan_kernel<<<1, 1024, 0, st>>>(bsum, nblk, stat);
+  PPS_LAUNCH_CHECK("rm_scan_kernel");
+  PPS_CUDA_TRY(cudaMemcpyAsync(x->flag_h.p, stat, 3 * 8, cudaMemcpyDeviceToHost, st));
+  PPS_CUDA_TRY(cudaStreamSynchronize(st));
+  const unsigned long long* h = x->flag_h.as<unsigned long long>();
+  if (h[0] != 0) return PPS_ERR_INVALID_ARG;                     // nothing has moved
+  const long long removed = (long long)h[1], first = (long long)h[2];
+  const long long moving = size - first - removed;              // the live rows after the first removed one
+
+  if (moving > 0) {
+    // 2. kept list
+    PPS_TRY(x->rm_kept.ensure((size_t)moving * 4));
+    int32_t* kept = x->rm_kept.as<int32_t>();
+    const long long b0 = first / kRmTile;
+    rm_fill_kernel<<<(unsigned)(nblk - b0), kRmThreads, 0, st>>>(flag, bsum, b0, first, size, kept);
+    PPS_LAUNCH_CHECK("rm_fill_kernel");
+
+    // 3. move in pieces: gather into the piece buffer [planes][piece][kpad] | tags | norms | inverse scales, copy down
+    const size_t per_row = x->plane_bytes(1) * x->planes + (x->tagged ? 8 : 0) + (x->scaled() ? 8 : 4);
+    const long long hook = (flags >> 8) & 0xffff;
+    const long long piece = std::min(moving, hook > 0 ? hook : std::max<long long>(1, (long long)(kRmPieceBytes / per_row)));
+    PPS_TRY(x->rm_piece.ensure((size_t)piece * per_row));
+    unsigned char* pb = x->rm_piece.as<unsigned char>();
+    int64_t* p_tags = reinterpret_cast<int64_t*>(pb + x->planes * x->plane_bytes(piece));
+    float* p_norm = reinterpret_cast<float*>(pb + x->planes * x->plane_bytes(piece) + (x->tagged ? (size_t)piece * 8 : 0));
+    float* p_scale = p_norm + piece;
+    const int vec = x->kpad * 2 / 16;
+    for (long long j0 = 0; j0 < moving; j0 += piece) {
+      const long long len = std::min(piece, moving - j0);
+      const long long dst = first + j0;
+      rm_gather_kernel<<<(unsigned)((len + kRmThreads / 32 - 1) / (kRmThreads / 32)), kRmThreads, 0, st>>>(
+          kept + j0, len, x->planes, vec, static_cast<const float4*>(x->g_planes), x->capacity * vec, x->g_norm,
+          x->scaled() ? x->g_norm + x->capacity : nullptr, x->tagged ? x->g_tags : nullptr, reinterpret_cast<float4*>(pb),
+          piece * vec, p_norm, p_scale, p_tags);
+      PPS_LAUNCH_CHECK("rm_gather_kernel");
+      for (int p = 0; p < x->planes; ++p)
+        PPS_CUDA_TRY(cudaMemcpyAsync(static_cast<unsigned char*>(x->g_planes) + p * x->plane_bytes(x->capacity) +
+                                         x->plane_bytes(dst),
+                                     pb + p * x->plane_bytes(piece), x->plane_bytes(len), cudaMemcpyDeviceToDevice, st));
+      PPS_CUDA_TRY(cudaMemcpyAsync(x->g_norm + dst, p_norm, (size_t)len * 4, cudaMemcpyDeviceToDevice, st));
+      if (x->scaled())
+        PPS_CUDA_TRY(cudaMemcpyAsync(x->g_norm + x->capacity + dst, p_scale, (size_t)len * 4, cudaMemcpyDeviceToDevice, st));
+      if (x->tagged)
+        PPS_CUDA_TRY(cudaMemcpyAsync(x->g_tags + dst, p_tags, (size_t)len * 8, cudaMemcpyDeviceToDevice, st));
+    }
+  }
+  x->size = size - removed;
+  if (n_removed) *n_removed = removed;
+  return PPS_OK;
 }

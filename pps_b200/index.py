@@ -42,6 +42,14 @@ class GalleryIndex:
     ``tags[r] == exclude_tags[i]`` and pads with -1 / inf when fewer than k rows remain; it needs a tagged index (an
     empty one answers with padding).  Without ``exclude_tags`` the tags are ignored.  Sharded: every rank passes the
     same exclude tags and its own rows' tags.
+
+    ``remove(rows)`` deletes local rows (integer numpy or torch, [n], any order, duplicates allowed) as ``np.delete``
+    does: every later row moves down by the number of removed rows before it, ``len`` shrinks by the number of distinct
+    rows removed (the return value), and every later search equals that of a fresh index given the remaining rows in
+    their order (with their tags), bit for bit.  Apply the same deletion to the rows' metadata.  A row outside
+    ``[0, len)`` raises and leaves the index unchanged.  The memory is kept for later adds; an index emptied by
+    ``remove`` decides again at its next non-empty add whether it is tagged.  Sharded: ``remove`` is local, not
+    collective; a rank removes its own rows, and the next ``search`` gathers the new shard sizes.
     """
 
     def __init__(self, dim, dtype=None, precision="f16x3", device=None, group=None):
@@ -91,19 +99,19 @@ class GalleryIndex:
         return x, is_np
 
     def _tags(self, t, n, name):
-        """[n] int64 CUDA tensor on the index's device from integer numpy or torch tags"""
+        """[n] int64 CUDA tensor on the index's device from integer numpy or torch values (n None: any length)"""
         import torch
         if isinstance(t, np.ndarray):
             if not np.issubdtype(t.dtype, np.integer):
-                raise RuntimeError("%s: expected integer tags, got %s" % (name, t.dtype))
+                raise RuntimeError("%s: expected integers, got %s" % (name, t.dtype))
             t = torch.from_numpy(np.ascontiguousarray(t, dtype=np.int64))
         elif isinstance(t, torch.Tensor):
             if t.dtype.is_floating_point or t.dtype.is_complex or t.dtype == torch.bool:
-                raise RuntimeError("%s: expected integer tags, got %s" % (name, t.dtype))
+                raise RuntimeError("%s: expected integers, got %s" % (name, t.dtype))
         else:
             raise RuntimeError("%s: expected numpy.ndarray or torch.Tensor, got %s" % (name, type(t)))
-        if t.dim() != 1 or int(t.shape[0]) != n:
-            raise RuntimeError("%s: expected shape [%d], got %s" % (name, n, tuple(t.shape)))
+        if t.dim() != 1 or (n is not None and int(t.shape[0]) != n):
+            raise RuntimeError("%s: expected shape [%s], got %s" % (name, "n" if n is None else n, tuple(t.shape)))
         return t.to(device=self.device, dtype=torch.int64).contiguous()
 
     def add(self, feats, tags=None):
@@ -120,6 +128,20 @@ class GalleryIndex:
                 _lib.check(self._lib.pps_index_add_tagged(self._h, _lib.ptr(x), n, ld, _lib.ptr(t), _lib.stream_ptr()),
                            "pps_index_add_tagged")
         return row0, n
+
+    def remove(self, rows):
+        """Delete local rows (np.delete's renumbering); returns the number of distinct rows removed."""
+        return self._remove(rows)
+
+    def _remove(self, rows, flags=0):
+        """remove() with flags: 0 or the PPS_INDEX_PIECE(n) test hook"""
+        import torch
+        t = self._tags(rows, None, "rows")
+        n_removed = C.c_longlong(0)
+        with torch.cuda.device(self.device):
+            _lib.check(self._lib.pps_index_remove(self._h, _lib.ptr(t), int(t.shape[0]), int(flags), _lib.stream_ptr(),
+                                                  C.byref(n_removed)), "pps_index_remove")
+        return int(n_removed.value)
 
     def _search_keys(self, q, k, index_offset=0, flags=0, exclude_tags=None):
         """[nq, k] top-k keys (distance bits << 32 | index_offset + row) of this index alone; flags: PPS_INDEX_* hooks."""

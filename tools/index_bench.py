@@ -25,8 +25,20 @@ A line records untagged_ms / excluding_ms (medians of the alternated searches) a
 share of rows a query leaves out) and, for junk, rank_eval_ms and agree against rank_eval(..., topk=k) with the same
 labels.  The camera modes have no rank_eval equivalent at these sizes (every id equal: nq x ng pair lists).
 
+--remove measures GalleryIndex.remove instead, one line per (gallery, pattern): a fresh index of the whole gallery
+loses one pattern of rows, then the same pattern again on what is left (the first call also allocates the removal's
+scratch).  Patterns: row0 (everything after row 0 moves), last1000 (nothing moves), random1 / random10 (1 % / 10 % of the
+rows at random, drawn again for the second call), front (the first tenth of the rows: 1 M of 10 M, then 900 000 of
+the 9 M left).  A line records:
+  remove_ms / remove_first_ms  host time of the second / first call, ending in a device synchronise
+  moved_rows, moved_bytes      rows (and their planes, norms, scales) that the second call moved down
+  copy_gbps, copy_share        4 x moved_bytes (a gather into the piece buffer, then a copy into place: each reads and
+                               writes the bytes) over remove_ms, and that rate over the 6 525 GB/s copy rate of DESIGN §7
+  search_ms / fresh_search_ms  medians of searches (per batch size) of the compacted index and of a fresh index of the
+                               same rows, alternated; agree: their outputs are identical (indices and distance bits)
+
 usage: python tools/index_bench.py [--reps 10] [--warmup 2] [--out FILE] [--cases fp16_1M,fp16_10M,fp32_520k]
-                                   [--tags none,cam6,half,junk] [--batches 1,16,64,256,3368]
+                                   [--tags none,cam6,half,junk] [--batches 1,16,64,256,3368] [--remove]
 """
 from __future__ import annotations
 
@@ -45,6 +57,8 @@ if ROOT not in sys.path:
 
 DIM, K = 2048, 100
 HBM_BYTES_PER_S = 7.7e12          # HGX B200 data sheet, one GPU
+COPY_BYTES_PER_S = 6.525e12       # measured device-to-device copy rate (MEASURED_PEAKS.json, DESIGN §7)
+REMOVE_PATTERNS = ["row0", "last1000", "random1", "random10", "front"]
 CASES = {"fp16_1M": (1_000_000, "fp16"), "fp16_10M": (10_000_000, "fp16"), "fp32_520k": (519_732, "fp32")}
 BATCHES = [1, 16, 64, 256, 3368]
 TAG_MODES = ["none", "cam6", "half", "junk"]
@@ -160,6 +174,78 @@ def run_tagged_case(name, modes, batches, reps, warmup, emit):
     torch.cuda.empty_cache()
 
 
+def remove_rows(pattern, ng, rs):
+    """local rows of a removal pattern on an index of ng rows"""
+    if pattern == "row0":
+        return np.array([0])
+    if pattern == "last1000":
+        return np.arange(ng - 1000, ng)
+    if pattern == "random1":
+        return rs.choice(ng, ng // 100, replace=False)
+    if pattern == "random10":
+        return rs.choice(ng, ng // 10, replace=False)
+    return np.arange(ng // 10)
+
+
+def run_remove_case(name, batches, reps, warmup, emit):
+    import torch
+    import pps_b200
+    from pps_b200 import synthetic
+    ng, dtype_name = CASES[name]
+    dev = torch.device("cuda")
+    tdt = torch.float16 if dtype_name == "fp16" else torch.float32
+    qid, _, gid, _ = synthetic.make_distractor_ids(max(batches), ng)
+    q_all = synthetic.make_features_device(qid, DIM, 750, 4.0, 7, dev, tdt)
+    planes = 1 if dtype_name == "fp16" else 2
+    row_bytes = DIM * 2 * planes + (4 if dtype_name == "fp16" else 8)      # planes (kpad = 2048) + norm (+ inverse scale)
+    gpu, watts = card(torch.cuda.current_device())
+    for pattern in REMOVE_PATTERNS:
+        rs = np.random.RandomState(REMOVE_PATTERNS.index(pattern))
+        # the seeded gallery again for every pattern: at most two indexes and one copy of the rows are held at a time
+        # (about 123 GB at 10 M fp16 rows)
+        g = synthetic.make_features_device(gid, DIM, 750, 4.0, 1000, dev, tdt)
+        idx = pps_b200.GalleryIndex(DIM, dtype=tdt, precision="f16x3")
+        idx.add(g)
+        live = np.arange(ng)
+        ms, moved = [], 0
+        for _ in range(2):
+            rows = remove_rows(pattern, len(live), rs)
+            rows_t = torch.from_numpy(rows).to(dev)
+            moved = len(live) - int(rows.min()) - len(rows)
+            torch.cuda.synchronize()
+            t0 = time.perf_counter()
+            n = idx.remove(rows_t)
+            torch.cuda.synchronize()
+            ms.append((time.perf_counter() - t0) * 1e3)
+            assert n == len(rows)
+            live = np.delete(live, rows)
+        g = g.index_select(0, torch.from_numpy(live).to(dev))
+        torch.cuda.empty_cache()
+        fresh = pps_b200.GalleryIndex(DIM, dtype=tdt, precision="f16x3")
+        fresh.add(g)                      # one add: the capacity is the row count, as the compacted index's
+        del g
+        torch.cuda.synchronize()
+        rec = {"case": name, "dtype": dtype_name, "precision": "f16x1" if dtype_name == "fp16" else "f16x3", "ng": ng,
+               "dim": DIM, "pattern": pattern, "removed_per_call": int(len(rows)), "size_after": len(idx),
+               "remove_ms": round(ms[1], 3), "remove_first_ms": round(ms[0], 3), "moved_rows": moved,
+               "moved_bytes": moved * row_bytes}
+        rec["copy_gbps"] = round(4 * moved * row_bytes / (ms[1] * 1e-3) / 1e9, 1)
+        rec["copy_share"] = round(rec["copy_gbps"] * 1e9 / COPY_BYTES_PER_S, 3)
+        for nq in batches:
+            q = q_all[:nq].contiguous()
+            s_ms, f_ms, _ = timed_alternating(lambda: idx.search(q, K), lambda: fresh.search(q, K), reps, warmup)
+            (ad, ai), (bd, bi) = idx.search(q, K), fresh.search(q, K)
+            rec["search_ms_nq%d" % nq] = round(s_ms, 4)
+            rec["fresh_search_ms_nq%d" % nq] = round(f_ms, 4)
+            rec["agree_nq%d" % nq] = bool(torch.equal(ai, bi) and torch.equal(ad.view(torch.int32), bd.view(torch.int32)))
+        rec.update({"k": K, "reps": reps, "gpu": gpu, "power_limit_w": watts})
+        emit(rec)
+        del idx, fresh
+        torch.cuda.empty_cache()
+    del q_all
+    torch.cuda.empty_cache()
+
+
 def run_case(name, reps, warmup, emit, batches=BATCHES):
     import torch
     import pps_b200
@@ -206,6 +292,7 @@ def main():
     ap.add_argument("--cases", default=",".join(CASES))
     ap.add_argument("--tags", default="none", help="comma-separated tag modes: " + ", ".join(TAG_MODES))
     ap.add_argument("--batches", default=",".join(str(b) for b in BATCHES))
+    ap.add_argument("--remove", action="store_true", help="measure GalleryIndex.remove (default batches 1,64)")
     args = ap.parse_args()
     import torch
     if not torch.cuda.is_available():
@@ -219,6 +306,8 @@ def main():
         if m not in TAG_MODES:
             raise SystemExit("unknown tag mode %r (expected %s)" % (m, ", ".join(TAG_MODES)))
     batches = [int(b) for b in args.batches.split(",") if b]
+    if args.remove and args.batches == ap.get_default("batches"):
+        batches = [1, 64]
 
     def emit(rec):
         line = json.dumps(rec)
@@ -227,6 +316,10 @@ def main():
             with open(args.out, "a") as f:
                 f.write(line + "\n")
 
+    if args.remove:
+        for c in names:
+            run_remove_case(c, batches, args.reps, args.warmup, emit)
+        return
     tagged = [m for m in modes if m != "none"]
     for c in names:
         if "none" in modes:
