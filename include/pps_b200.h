@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define PPS_ABI_VERSION 8
+#define PPS_ABI_VERSION 9
 
 /* ---- error codes (the Python mirror turns every non-zero code into RuntimeError,
  * like CAFFE_ENFORCE does: detectron/tests/test_zero_even_op.py:50-53) ---- */
@@ -589,6 +589,35 @@ int pps_evaluate_host(const float* q_feats, long long nq,
  *                      on `stream`.  flags: 0, or the test hook PPS_INDEX_PIECE(n) (at most n rows per piece).  Sharded:
  *                      removal is local (a rank removes its own rows); the next search's all-gather of the shard sizes
  *                      moves the global offsets.
+ * pps_search_range_tc  the range form of pps_search_topk_tc (same kernel up to the admission and the address): every
+ *                      distance whose bits are < lim[q] is appended as (bits << 32 | col0 + row) to
+ *                      out[out_off[q] + slot] when slot < out_cap[q]; cnt[q] counts every hit, also past the capacity.
+ *                      g_tags / q_tags: both null, or both set (the pairs whose tags are equal are no hits).  The limit
+ *                      of a radius r is bits(r) + 1 for r >= 0 (-0 as 0; +inf: 0x7f800001) and 0 for a negative or NaN r:
+ *                      then bits < lim <=> d <= r, distances being >= 0 and never NaN.
+ * pps_index_range_search   every row within a radius of each query: row r is a result of query q when d(q, r) <=
+ *                      d_radius[q] (device float32 [nq]; IEEE comparison: a negative or NaN radius selects nothing, +inf
+ *                      every row), d being pps_index_search's distance, bit for bit.  d_q_tags (device [nq], may be null):
+ *                      also leave out the rows whose tag equals the query's, as pps_index_search_excluding (a non-empty
+ *                      untagged index: PPS_ERR_INVALID_ARG).  Output in FAISS's range_search layout: d_lims (caller memory,
+ *                      device int64 [nq + 1]) and *total (host) = d_lims[nq]; query q's results are keys
+ *                      [d_lims[q], d_lims[q + 1]) in (distance, index) order, the order of top-k keys, with gallery index
+ *                      index_offset + row.  The keys stay in index-owned scratch: pps_index_range_keys copies them out.
+ *                      One pass of pps_search_range_tc over every row writes uniform slices of C keys per query (C: 4 096
+ *                      at first, then the power of two at or above the largest count of an earlier call, at most 1 GiB of
+ *                      slices); a scan of the counts and one 16-byte read-back {total, largest count} follow, the call's
+ *                      only synchronisation when no slice ran over.  Otherwise a second pass writes the keys straight into
+ *                      the result layout.  pps_sort_key_segments' stages then compact and sort.  A result that does not
+ *                      fit in memory: PPS_ERR_CUDA, the index unchanged and usable.  flags: 0, or the test hook
+ *                      PPS_INDEX_TKCAP(n) (C = n).  An empty index or nq = 0: d_lims all zero.
+ * pps_index_range_keys copies the last range search's *total keys to d_keys (device); valid until the next call on the
+ *                      index.  pps_topk_unpack(keys, total, 1, ...) splits them into distances and int32 indices.
+ * pps_sort_key_segments    sorts every segment [lims[s], lims[s + 1]) of keys ascending, in place (lims: device int64
+ *                      [nseg + 1], ascending; scratch: device, lims[nseg] - lims[0] keys, may be null when that is at most
+ *                      4 096).  Reads lims[0] and lims[nseg] back (16 bytes, a synchronisation).  Keys are sorted in tiles
+ *                      of 4 096 in shared memory, then by ceil(log2(total / 4096)) merge passes; segments may hold from 0
+ *                      keys to all of them.  Equal keys are allowed; keys that are unique in their segment (range search:
+ *                      the row index is in the low bits) give one result whatever order they came in.
  * Calls on one index are ordered by the caller (one stream, or events between streams); every call sets the index's
  * device for its duration.  A sharded gallery: one index per rank, index_offset = the rows of the ranks before, an
  * all-gather of the [nq][k] keys and the k smallest per query (every rank's list is sorted, keys are unique).
@@ -622,6 +651,16 @@ int       pps_index_search_excluding(pps_index* idx, const void* d_q, long long 
                                      uint64_t* d_keys);
 int       pps_index_remove(pps_index* idx, const int64_t* d_rows, long long n, int flags, void* stream,
                            long long* n_removed);
+int pps_search_range_tc(const void* g_planes, const float* g_sqnorm, long long ng, int g_planes_n, long long g_plane_rows,
+                        const void* q_planes, const float* q_sqnorm, long long nq, int q_planes_n, long long q_plane_rows,
+                        int dim, int precision, int flags, long long col0, const uint32_t* lim, uint32_t* cnt,
+                        const long long* out_off, const uint32_t* out_cap, uint64_t* out, const int64_t* g_tags,
+                        const int64_t* q_tags, void* stream);
+int       pps_index_range_search(pps_index* idx, const void* d_q, long long nq, long long ldq, const float* d_radius,
+                                 const int64_t* d_q_tags /*nullable*/, long long index_offset, int flags, void* stream,
+                                 int64_t* d_lims, long long* total);
+int       pps_index_range_keys(pps_index* idx, uint64_t* d_keys, void* stream);
+int       pps_sort_key_segments(uint64_t* keys, const int64_t* lims, long long nseg, uint64_t* scratch, void* stream);
 
 /* ------------------------------------------------------------------------------------
  * Next row (SURVEY §8f.4) — the reference's training-side triplet mining ops.

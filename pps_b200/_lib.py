@@ -13,7 +13,7 @@ import threading
 from . import build as _build
 
 # ---- constants (keep in sync with include/pps_b200.h) ----
-ABI_VERSION = 8
+ABI_VERSION = 9
 PPS_OK = 0
 PPS_ERR_INVALID_ARG = -1
 PPS_ERR_SHAPE = -2
@@ -30,7 +30,8 @@ PASS_NO_FUSED_COUNT = 4
 
 
 def index_tkcap(n: int) -> int:
-    """PPS_INDEX_TKCAP(n): pps_index_search test hook, candidate entries per query and chunk."""
+    """PPS_INDEX_TKCAP(n): pps_index_search test hook, candidate entries per query and chunk (pps_index_range_search: keys
+    per query in the first pass's slices)."""
     return (n & 0xffff) << 8
 
 
@@ -162,6 +163,11 @@ SIGNATURES = {
     "pps_index_add_tagged": (_i, [_vp, _vp, _ll, _ll, _vp, _vp]),
     "pps_index_search_excluding": (_i, [_vp, _vp, _ll, _ll, _vp, _i, _ll, _i, _vp, _vp]),
     "pps_index_remove": (_i, [_vp, _vp, _ll, _i, _vp, C.POINTER(_ll)]),
+    "pps_search_range_tc": (_i, [_vp, _vp, _ll, _i, _ll, _vp, _vp, _ll, _i, _ll, _i, _i, _i, _ll, _vp, _vp, _vp, _vp, _vp,
+                                 _vp, _vp, _vp]),
+    "pps_index_range_search": (_i, [_vp, _vp, _ll, _ll, _vp, _vp, _ll, _i, _vp, _vp, C.POINTER(_ll)]),
+    "pps_index_range_keys": (_i, [_vp, _vp, _vp]),
+    "pps_sort_key_segments": (_i, [_vp, _vp, _ll, _vp, _vp]),
     "pps_pairwise_distance_fwd": (_i, [_vp, _i, _i, _vp, _vp]),
     "pps_pairwise_distance_bwd": (_i, [_vp, _vp, _i, _i, _vp, _vp]),
     "pps_batch_hard_fwd": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _vp]),

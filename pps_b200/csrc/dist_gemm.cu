@@ -421,7 +421,7 @@ __device__ __forceinline__ void dist_tc2_body(const CUtensorMap& tmA, const CUte
           bn_s[256 + etid] = gj < g.m2 ? __ldg(g.b_scale + gj) : 0.f;
           if (BN > 128) bn_s[256 + etid + 128] = gj + 128 < g.m2 ? __ldg(g.b_scale + gj + 128) : 0.f;
         }
-        if (epi_search(EPI)) {                 // the admission bound of every query column, double-buffered like |b|^2
+        if (epi_search(EPI)) {                 // the admission bound (EPI_RANGE: limit) of every query column, double-buffered
           uint32_t* bd = reinterpret_cast<uint32_t*>(stage_out) + as * 256;
           bd[etid] = gj < g.m2 ? __ldg(rf.tk_bound + gj) : 0u;
           if (BN > 128) bd[etid + 128] = gj + 128 < g.m2 ? __ldg(rf.tk_bound + gj + 128) : 0u;
@@ -469,23 +469,24 @@ __device__ __forceinline__ void dist_tc2_body(const CUtensorMap& tmA, const CUte
               float d2 = __fadd_rn(__fmaf_rn(sc[e], dot, qq[e]), an);
               d2 = fmaxf(d2, 0.f);
               v[4 * j + e] = __float_as_uint(want_sq ? d2 : (sqrt_rn ? __fsqrt_rn(d2) : sqrt_approx(d2)));
-              hit |= (v[4 * j + e] <= bb[e]) & (4 * j + e < valid_cols);   // distances are >= 0: bits order like values
+              // distances are >= 0: bits order like values.  EPI_RANGE: bb is the limit bits(radius) + 1 (0: none)
+              hit |= (epi_range(EPI) ? v[4 * j + e] < bb[e] : v[4 * j + e] <= bb[e]) & (4 * j + e < valid_cols);
             }
           }
           // admission, aggregated per (warp, query): one atomic reserves the slots of every lane that passes
           if (__any_sync(0xffffffffu, hit && row_ok)) {
             const uint32_t lanes_below = (1u << lane) - 1u;
             const unsigned long long gkey = (unsigned long long)(uint32_t)(rf.col0 + gi);
-            // EPI_SEARCH_EXCL: the row's tag is loaded on the row's first hit of the tile (the n tiles of one m tile
-            // share it)
-            if (EPI == EPI_SEARCH_EXCL && hit && row_ok && tag_tile != w.m_tile) {
+            // EPI_SEARCH_EXCL, EPI_RANGE_EXCL: the row's tag is loaded on the row's first hit of the tile (the n tiles of
+            // one m tile share it)
+            if (epi_excl(EPI) && hit && row_ok && tag_tile != w.m_tile) {
               row_tag = __ldg(rf.g_tags + gi);
               tag_tile = w.m_tile;
             }
 #pragma unroll
             for (int e = 0; e < 32; ++e) {                     // (unrolled: v[] must stay in registers)
-              bool pass = row_ok && e < valid_cols && v[e] <= bd[e];
-              if (EPI == EPI_SEARCH_EXCL && pass)              // one address per warp: an L1 broadcast
+              bool pass = row_ok && e < valid_cols && (epi_range(EPI) ? v[e] < bd[e] : v[e] <= bd[e]);
+              if (epi_excl(EPI) && pass)                       // one address per warp: an L1 broadcast
                 pass = row_tag != __ldg(rf.q_tags + ((long long)n0 + c + e));
               const uint32_t m = __ballot_sync(0xffffffffu, pass);
               if (m) {
@@ -495,8 +496,12 @@ __device__ __forceinline__ void dist_tc2_body(const CUtensorMap& tmA, const CUte
                 if (lane == leader) base = atomicAdd(rf.tk_cnt + col, (uint32_t)__popc(m));
                 base = __shfl_sync(0xffffffffu, base, leader);
                 const uint32_t slot = base + (uint32_t)__popc(m & lanes_below);
-                if (pass && slot < (uint32_t)rf.tk_cap)
+                if (epi_range(EPI)) {                          // (the query's offset and capacity: broadcasts too)
+                  if (pass && slot < __ldg(rf.out_cap + col))
+                    rf.tk_cand[__ldg(rf.out_off + col) + slot] = ((unsigned long long)v[e] << 32) | gkey;
+                } else if (pass && slot < (uint32_t)rf.tk_cap) {
                   rf.tk_cand[col * rf.tk_cap + slot] = ((unsigned long long)v[e] << 32) | gkey;
+                }
               }
             }
           }
@@ -1020,29 +1025,38 @@ static int launch_search(const CUtensorMap& tmA, const CUtensorMap& tmB, const G
     configured_dev = dev;
   }
   dist_tc2_kernel<BN, EPI><<<(unsigned)(2 * pairs), kGemmThreads, kGemm2Smem, st>>>(tmA, tmB, tmA /*no output map*/, ga, rf);
-  PPS_LAUNCH_CHECK(EPI == EPI_SEARCH ? "dist_tc2_kernel<search>" : "dist_tc2_kernel<search_excl>");
+  PPS_LAUNCH_CHECK(EPI == EPI_SEARCH        ? "dist_tc2_kernel<search>"
+                   : EPI == EPI_SEARCH_EXCL ? "dist_tc2_kernel<search_excl>"
+                   : EPI == EPI_RANGE       ? "dist_tc2_kernel<range>"
+                                            : "dist_tc2_kernel<range_excl>");
   return PPS_OK;
 }
 
 template <int BN>
 static int launch_search(const CUtensorMap& tmA, const CUtensorMap& tmB, const Gemm2Args& ga, const RankFuse& rf, int dev,
                          long long pairs, cudaStream_t st) {
+  if (rf.out_off)
+    return rf.q_tags ? launch_search<BN, EPI_RANGE_EXCL>(tmA, tmB, ga, rf, dev, pairs, st)
+                     : launch_search<BN, EPI_RANGE>(tmA, tmB, ga, rf, dev, pairs, st);
   return rf.q_tags ? launch_search<BN, EPI_SEARCH_EXCL>(tmA, tmB, ga, rf, dev, pairs, st)
                    : launch_search<BN, EPI_SEARCH>(tmA, tmB, ga, rf, dev, pairs, st);
 }
 
-// g_tags / q_tags: both null (no exclusion) or both set (pps_search_topk_excl_tc)
+// g_tags / q_tags: both null (no exclusion) or both set (pps_search_topk_excl_tc, pps_search_range_tc with tags).
+// out_off / out_cap: null (top-k candidates, tk_cand[q][tk_cap]) or both set (range search, tk_cap unused)
 static int search_topk_impl(const void* g_planes, const float* g_sqnorm, long long ng, int g_planes_n, long long g_plane_rows,
                             const void* q_planes, const float* q_sqnorm, long long nq, int q_planes_n, long long q_plane_rows,
                             int dim, int precision, int flags, long long col0, const uint32_t* tk_bound, uint32_t* tk_cnt,
-                            uint64_t* tk_cand, int tk_cap, const int64_t* g_tags, const int64_t* q_tags, void* stream) {
-  if (ng < 0 || nq < 0 || dim <= 0 || col0 < 0 || tk_cap < 1) return PPS_ERR_INVALID_ARG;
+                            uint64_t* tk_cand, int tk_cap, const int64_t* g_tags, const int64_t* q_tags, void* stream,
+                            const long long* out_off = nullptr, const uint32_t* out_cap = nullptr) {
+  if (ng < 0 || nq < 0 || dim <= 0 || col0 < 0 || (!out_off && tk_cap < 1)) return PPS_ERR_INVALID_ARG;
   if (flags & ~(PPS_DIST_SQUARED | PPS_DIST_SQRT_RN)) return PPS_ERR_INVALID_ARG;   // keys order by the bits of a distance
   if (g_plane_rows == 0) g_plane_rows = ng;
   if (q_plane_rows == 0) q_plane_rows = nq;
   if (g_plane_rows < ng || q_plane_rows < nq || col0 + ng > 0xffffffffLL) return PPS_ERR_INVALID_ARG;
   if (ng == 0 || nq == 0) return PPS_OK;
   if (!g_planes || !g_sqnorm || !q_planes || !q_sqnorm || !tk_bound || !tk_cnt || !tk_cand) return PPS_ERR_INVALID_ARG;
+  if ((out_off == nullptr) != (out_cap == nullptr)) return PPS_ERR_INVALID_ARG;
   if ((reinterpret_cast<uintptr_t>(g_planes) & 15u) || (reinterpret_cast<uintptr_t>(q_planes) & 15u)) return PPS_ERR_ALIGN;
   if (ng > 0x7fffff00LL || nq > 0x7fffff00LL) return PPS_ERR_UNSUPPORTED;   // TMA coordinates are int32
   GemmArgs terms;
@@ -1087,6 +1101,7 @@ static int search_topk_impl(const void* g_planes, const float* g_sqnorm, long lo
   rf.col0 = col0;
   rf.tk_bound = tk_bound; rf.tk_cnt = tk_cnt; rf.tk_cand = reinterpret_cast<unsigned long long*>(tk_cand); rf.tk_cap = tk_cap;
   rf.g_tags = reinterpret_cast<const long long*>(g_tags); rf.q_tags = reinterpret_cast<const long long*>(q_tags);
+  rf.out_off = out_off; rf.out_cap = out_cap;
   int dev = 0;
   PPS_CUDA_TRY(cudaGetDevice(&dev));
   const long long tiles = (long long)g.m_tiles * g.n_tiles;
@@ -1118,6 +1133,20 @@ extern "C" int pps_search_topk_excl_tc(const void* g_planes, const float* g_sqno
   if (ng > 0 && nq > 0 && (!g_tags || !q_tags)) return PPS_ERR_INVALID_ARG;
   return search_topk_impl(g_planes, g_sqnorm, ng, g_planes_n, g_plane_rows, q_planes, q_sqnorm, nq, q_planes_n, q_plane_rows,
                           dim, precision, flags, col0, tk_bound, tk_cnt, tk_cand, tk_cap, g_tags, q_tags, stream);
+}
+
+// Range search: every element whose distance bits are below lim[q] (pps_index_range_search's limit of a radius) is
+// appended to out[out_off[q] + slot] while slot < out_cap[q]; cnt[q] counts every hit, also past the capacity.  The
+// same kernel as pps_search_topk_tc up to the admission and the address (instances EPI_RANGE / EPI_RANGE_EXCL).
+extern "C" int pps_search_range_tc(const void* g_planes, const float* g_sqnorm, long long ng, int g_planes_n,
+                                   long long g_plane_rows, const void* q_planes, const float* q_sqnorm, long long nq,
+                                   int q_planes_n, long long q_plane_rows, int dim, int precision, int flags, long long col0,
+                                   const uint32_t* lim, uint32_t* cnt, const long long* out_off, const uint32_t* out_cap,
+                                   uint64_t* out, const int64_t* g_tags, const int64_t* q_tags, void* stream) {
+  if ((g_tags == nullptr) != (q_tags == nullptr)) return PPS_ERR_INVALID_ARG;
+  if (ng > 0 && nq > 0 && (!out_off || !out_cap)) return PPS_ERR_INVALID_ARG;
+  return search_topk_impl(g_planes, g_sqnorm, ng, g_planes_n, g_plane_rows, q_planes, q_sqnorm, nq, q_planes_n, q_plane_rows,
+                          dim, precision, flags, col0, lim, cnt, out, 0, g_tags, q_tags, stream, out_off, out_cap);
 }
 
 extern "C" int pps_dist_fp32(const float* a, long long lda, const float* a_sqnorm, long long m1, const float* b,

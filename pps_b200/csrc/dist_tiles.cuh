@@ -62,6 +62,10 @@ struct RankFuse {
   // EPI_SEARCH_EXCL: row r of the block is no candidate of query q when g_tags[r] == q_tags[q]
   const long long* g_tags;  // [rows of the block]
   const long long* q_tags;  // [queries]
+  // EPI_RANGE(_EXCL): tk_bound holds the per-query limits, tk_cnt counts every hit and tk_cand is the output; query q's
+  // hits go to tk_cand[out_off[q] + slot] for slot < out_cap[q]
+  const long long* out_off; // [queries]
+  const uint32_t* out_cap;  // [queries]
 };
 
 constexpr int EPI_DIST = 0;          // |a|^2 + |b|^2 - 2ab, clamp, sqrt (or squared / raw dot by flags) -> matrix
@@ -70,11 +74,15 @@ constexpr int EPI_RANK = 2;          // distance as EPI_DIST, consumed by the co
 constexpr int EPI_DIST_TOPK = 3;     // EPI_DIST + one compare per element against the row's top-k admission bound
 constexpr int EPI_SEARCH = 4;        // A = gallery, B = queries: distance -> top-k admission per COLUMN; no matrix
 constexpr int EPI_SEARCH_EXCL = 5;   // EPI_SEARCH without the (row, query) pairs whose tags are equal
-__host__ __device__ constexpr bool epi_search(int epi) { return epi == EPI_SEARCH || epi == EPI_SEARCH_EXCL; }
+constexpr int EPI_RANGE = 6;         // EPI_SEARCH's tile walk and distances: every element below its query's limit, appended
+constexpr int EPI_RANGE_EXCL = 7;    // EPI_RANGE without the (row, query) pairs whose tags are equal
+__host__ __device__ constexpr bool epi_range(int epi) { return epi == EPI_RANGE || epi == EPI_RANGE_EXCL; }
+__host__ __device__ constexpr bool epi_excl(int epi) { return epi == EPI_SEARCH_EXCL || epi == EPI_RANGE_EXCL; }
+__host__ __device__ constexpr bool epi_search(int epi) { return epi == EPI_SEARCH || epi_excl(epi) || epi_range(epi); }
 
 // Tile order.  EPI_DIST / EPI_AFFINE_RELU: tile t = pair, pair + npairs, ... with the m index fastest, so that the
-// CTA pairs running concurrently share B tiles in L2.  EPI_SEARCH(_EXCL): the same tiles with the n index fastest, so that a
-// gallery (m) tile is read from HBM once and its other query tiles find it in L2.  EPI_RANK: a CTA pair keeps ONE m tile per run (its rows'
+// CTA pairs running concurrently share B tiles in L2.  EPI_SEARCH(_EXCL) and EPI_RANGE(_EXCL): the same tiles with the
+// n index fastest, so that a gallery (m) tile is read from HBM once and its other query tiles find it in L2.  EPI_RANK: a CTA pair keeps ONE m tile per run (its rows'
 // thresholds and counters stay in shared memory) and walks a contiguous range of n tiles.
 //   npairs >= m_tiles: k = npairs / m_tiles pairs per m tile walk n tiles [0, Na) in k aligned parts - the pairs that own
 //     the other m tiles walk the same n range at the same pace, which keeps the L2 sharing of B - and the X = npairs % m_tiles

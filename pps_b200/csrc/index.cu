@@ -27,6 +27,11 @@
 //      so a piece's destinations overlap only its own sources (already in the buffer) or earlier pieces' (already read).
 // The moved rows are the bytes a fresh add of the remaining rows would have written (the split is per row), so every
 // later search equals a fresh index's bit for bit.
+//
+// Range search (pps_index_range_search): radius -> per-query limit, one pps_search_range_tc over every row into uniform
+// slices, a scan of the counts into lims and one 16-byte read-back {total, largest count}; a second pass straight into
+// the lims layout only when a slice ran over.  The segment sort (pps_sort_key_segments) compacts the slices and sorts
+// each query's keys: tiles of 4 096 keys in shared memory, then merge passes of aligned runs, all sized by the total.
 #include "ctx.cuh"
 
 namespace {
@@ -63,6 +68,9 @@ struct pps_index {
   bool tagged = false;          // decided by the first non-empty add
   GrowBuf qs, qn, dist, tk_bound, tk_cnt, tk_cand, flag, n_excl;
   GrowBuf rm_flag, rm_bsum, rm_stat, rm_kept, rm_piece;    // scratch of pps_index_remove
+  GrowBuf rg_lim, rg_cnt, rg_off, rg_cap, rg_slices, rg_stat, rg_keys, rg_tmp;   // scratch of pps_index_range_search
+  long long rg_total = 0;       // keys of the last range search (in rg_keys)
+  long long rg_slice = 4096;    // first-pass slice per query: a power of two >= the largest count seen so far
   PinBuf flag_h;
   bool scaled() const { return precision == PPS_PREC_F16X3; }
   size_t plane_bytes(long long rows) const { return (size_t)rows * kpad * 2; }
@@ -140,26 +148,27 @@ constexpr size_t kRmPieceBytes = 256ull << 20;      // the piece buffer of the m
 constexpr unsigned long long kRmNone = ~0ull;
 
 // exclusive prefix of v over the block (blockDim.x a multiple of 32, <= 1024) and the block's total
-__device__ __forceinline__ uint32_t block_excl_scan(uint32_t v, uint32_t* s_warp, uint32_t* total) {
+template <class T>
+__device__ __forceinline__ T block_excl_scan(T v, T* s_warp, T* total) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
-  uint32_t x = v;
+  T x = v;
   for (int o = 1; o < 32; o <<= 1) {
-    const uint32_t y = __shfl_up_sync(~0u, x, o);
+    const T y = __shfl_up_sync(~0u, x, o);
     if (lane >= o) x += y;
   }
   if (lane == 31) s_warp[warp] = x;
   __syncthreads();
   if (warp == 0) {
-    uint32_t w = lane < nw ? s_warp[lane] : 0u;
+    T w = lane < nw ? s_warp[lane] : T(0);
     for (int o = 1; o < 32; o <<= 1) {
-      const uint32_t y = __shfl_up_sync(~0u, w, o);
+      const T y = __shfl_up_sync(~0u, w, o);
       if (lane >= o) w += y;
     }
     s_warp[lane] = w;
   }
   __syncthreads();
   *total = s_warp[nw - 1];
-  const uint32_t r = (warp ? s_warp[warp - 1] : 0u) + x - v;
+  const T r = (warp ? s_warp[warp - 1] : T(0)) + x - v;
   __syncthreads();                                   // s_warp is reused by the caller's next scan
   return r;
 }
@@ -269,6 +278,247 @@ __global__ void __launch_bounds__(kRmThreads) rm_gather_kernel(const int32_t* __
   }
 }
 
+
+// ---- range search (pps_index_range_search) and the segment sort (pps_sort_key_segments) ----
+constexpr int kSortThreads = 256;
+constexpr int kSortTile = 4096;                     // S: keys one CTA sorts in shared memory (16 per thread)
+constexpr int kMergeTile = 2048;                    // output keys per CTA of a merge pass (< S: at most two pair blocks)
+constexpr size_t kSortSmem = 2 * kSortTile * sizeof(unsigned long long);
+constexpr long long kSliceBytes = 1LL << 30;        // cap of the first pass's slices, nq * C * 8 bytes
+
+// radius -> admission limit of the range kernel: distance bits < lim  <=>  d <= r (distances are >= 0 and never NaN).
+// -0 counts as 0, +inf gives 0x7f800001 (every row), a negative or NaN radius 0 (none).  Counters zeroed, slice q at q * C.
+__global__ void range_prep_kernel(const float* __restrict__ radius, long long nq, long long slice, uint32_t* __restrict__ lim,
+                                  uint32_t* __restrict__ cnt, long long* __restrict__ off, uint32_t* __restrict__ cap) {
+  const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+  if (i >= nq) return;
+  const float r = radius[i];
+  lim[i] = r >= 0.f ? (r == 0.f ? 0u : __float_as_uint(r)) + 1u : 0u;
+  cnt[i] = 0u;
+  off[i] = i * slice;
+  cap[i] = (uint32_t)slice;
+}
+
+// one block: lims = exclusive prefix sums of cnt (int64, [n + 1]); stat = {total, largest count}
+__global__ void __launch_bounds__(1024) range_scan_kernel(const uint32_t* __restrict__ cnt, long long n, long long* __restrict__ lims,
+                                                          unsigned long long* __restrict__ stat) {
+  __shared__ unsigned long long s_warp[32];
+  __shared__ uint32_t s_max;
+  if (threadIdx.x == 0) s_max = 0u;
+  unsigned long long carry = 0;
+  uint32_t m = 0u;
+  for (long long base = 0; base < n; base += blockDim.x) {
+    const long long i = base + threadIdx.x;
+    const uint32_t v = i < n ? cnt[i] : 0u;
+    m = max(m, v);
+    unsigned long long total;
+    const unsigned long long e = block_excl_scan<unsigned long long>(v, s_warp, &total);
+    if (i < n) lims[i] = (long long)(carry + e);
+    carry += total;
+  }
+  __syncthreads();                                   // (n == 0: s_max's initialisation)
+  atomicMax(&s_max, m);
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    lims[n] = (long long)carry;
+    stat[0] = carry;
+    stat[1] = s_max;
+  }
+}
+
+// The segment sort works on CSR positions o in [0, total) of keys[base + o] (base = lims[0]).  Runs are aligned to
+// multiples of their width w counted from position 0 and clipped to their segment; the tile stage leaves every aligned
+// S-block of a segment sorted, and the merge pass of width w merges the two w-runs of every aligned 2w-block.  After
+// ceil(log2(total / S)) passes every segment lies in one sorted run.
+
+// segment of position o: the last s with lims[s] - base <= o  (o < lims[nseg] - base)
+__device__ __forceinline__ long long seg_of(const long long* __restrict__ lims, long long nseg, long long base, long long o) {
+  long long lo = 0, hi = nseg;
+  while (hi - lo > 1) {
+    const long long mid = (lo + hi) >> 1;
+    if (__ldg(lims + mid) - base <= o) lo = mid;
+    else hi = mid;
+  }
+  return lo;
+}
+
+// #{i < n : a[i] < x} (LE: a[i] <= x) of an ascending a.  A merge places a key of run A after the smaller keys of run B
+// and a key of B after the keys of A that are not greater: equal keys keep A before B.
+template <bool LE>
+__device__ __forceinline__ int count_below(const unsigned long long* a, int n, unsigned long long x) {
+  int lo = 0;
+  while (n > 0) {
+    const int h = n >> 1;
+    if (LE ? a[lo + h] <= x : a[lo + h] < x) {
+      lo += h + 1;
+      n -= h + 1;
+    } else {
+      n = h;
+    }
+  }
+  return lo;
+}
+
+// merge path of one warp: how many of the first d outputs of merge(a[0, na), b[0, nb)) come from a (A first on ties).
+// 32 probes per step, so a split in runs of 2^20 keys takes 4 dependent loads instead of 20.
+__device__ long long merge_split_warp(const unsigned long long* __restrict__ a, long long na,
+                                      const unsigned long long* __restrict__ b, long long nb, long long d) {
+  long long lo = d - nb > 0 ? d - nb : 0, hi = d < na ? d : na;
+  const int lane = threadIdx.x & 31;
+  while (lo < hi) {                                  // a[i] <= b[d - 1 - i] holds for i < answer, fails from there on
+    const long long step = (hi - lo + 31) / 32, i = lo + lane * step;
+    const bool p = i < hi && a[i] <= b[d - 1 - i];
+    const long long c = __popc(__ballot_sync(~0u, p));
+    if (c == 0) {
+      hi = lo;
+    } else {
+      const long long nlo = lo + (c - 1) * step + 1;
+      hi = min(hi, lo + c * step);
+      lo = nlo;
+    }
+  }
+  return lo;
+}
+
+// tile stage: CTA b sorts positions [b S, b S + S) ∩ [0, total) piece by piece of segment, in shared memory, by merging
+// aligned runs of 1, 2, 4, ... keys (every piece at once: no pass per segment).  Position o's key comes from
+// src[s * stride + o - (lims[s] - base)] (stride > 0: the first pass's per-query slices) or src[o]; the result goes to
+// dst[o] (may be src: the tile is read before it is written).  src / dst point at position 0.
+__global__ void __launch_bounds__(kSortThreads) seg_tile_sort_kernel(const unsigned long long* src, long long stride,
+                                                                     unsigned long long* dst, const long long* __restrict__ lims,
+                                                                     long long nseg, long long base, long long total) {
+  extern __shared__ unsigned long long s_keys[];     // [2][S]
+  constexpr int kPer = kSortTile / kSortThreads;
+  const long long t0 = (long long)blockIdx.x * kSortTile;
+  const int n = (int)min((long long)kSortTile, total - t0);
+  int seg_lo[kPer], seg_hi[kPer];                    // the segment's piece of the tile, per position (positions stay put)
+  unsigned long long* cur = s_keys;
+  unsigned long long* nxt = s_keys + kSortTile;
+#pragma unroll
+  for (int j = 0; j < kPer; ++j) {
+    const int i = threadIdx.x + j * kSortThreads;
+    seg_lo[j] = seg_hi[j] = i;
+    if (i < n) {
+      const long long o = t0 + i, s = seg_of(lims, nseg, base, o);
+      const long long l = __ldg(lims + s) - base, r = __ldg(lims + s + 1) - base;
+      seg_lo[j] = (int)(max(l, t0) - t0);
+      seg_hi[j] = (int)(min(r, t0 + n) - t0);
+      cur[i] = stride > 0 ? src[s * stride + (o - l)] : src[o];
+    }
+  }
+  __syncthreads();
+  for (int w = 1; w < n; w <<= 1) {
+#pragma unroll
+    for (int j = 0; j < kPer; ++j) {
+      const int i = threadIdx.x + j * kSortThreads;
+      if (i < n) {
+        const unsigned long long x = cur[i];
+        const int ps = i & ~(2 * w - 1), m = ps + w;
+        const int a0 = max(ps, seg_lo[j]), a1 = min(m, seg_hi[j]);          // run A of i's pair block, clipped
+        const int b0 = max(m, seg_lo[j]), b1 = min(ps + 2 * w, seg_hi[j]);  // run B
+        const int pos = i < m ? i + count_below<false>(cur + b0, max(b1 - b0, 0), x)
+                              : a0 + (i - b0) + count_below<true>(cur + a0, max(a1 - a0, 0), x);
+        nxt[pos] = x;
+      }
+    }
+    __syncthreads();
+    unsigned long long* t = cur;
+    cur = nxt;
+    nxt = t;
+  }
+#pragma unroll
+  for (int j = 0; j < kPer; ++j) {
+    const int i = threadIdx.x + j * kSortThreads;
+    if (i < n) dst[t0 + i] = cur[i];
+  }
+}
+
+// merge pass of width w >= S: CTA b writes output positions [b T, b T + T) ∩ [0, total) of dst (src, dst: position 0).
+// A pair block [ps, ps + 2w) needs a merge only where a segment crosses its middle m = ps + w; the tile touches at most two pair blocks (T < 2w),
+// so it holds at most two merged pieces.  Each piece: merge-path splits of its ends (one warp each), the keys of both runs
+// that land in it -> shared memory, every key's rank in the other run there.  Every other position is copied.
+__global__ void __launch_bounds__(kSortThreads) seg_merge_kernel(const unsigned long long* __restrict__ src,
+                                                                 unsigned long long* __restrict__ dst,
+                                                                 const long long* __restrict__ lims, long long nseg,
+                                                                 long long base, long long total, long long w) {
+  __shared__ unsigned long long s_in[kMergeTile];
+  __shared__ long long s_pc[2][6];                   // piece: out begin, out end, P0 (pair start in the segment), m, ia, ib
+  __shared__ int s_ok[2];
+  const long long o0 = (long long)blockIdx.x * kMergeTile, o1 = min(o0 + kMergeTile, total);
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const unsigned long long* in = src;
+  if (warp < 2) {
+    const long long ps = ((warp == 0 ? o0 : o1 - 1) / (2 * w)) * (2 * w), m = ps + w;
+    bool ok = m < total && !(warp == 1 && ps == (o0 / (2 * w)) * (2 * w));
+    if (ok) {
+      const long long s = seg_of(lims, nseg, base, m);
+      const long long l = __ldg(lims + s) - base, r = __ldg(lims + s + 1) - base;
+      const long long p0 = max(ps, l), p1 = min(ps + 2 * w, r);
+      const long long a = max(o0, p0), b = min(o1, p1);
+      ok = l < m && a < b;                           // the segment crosses m and its pair block meets the tile
+      if (ok) {
+        const long long ia = merge_split_warp(in + p0, m - p0, in + m, p1 - m, a - p0);
+        const long long ib = merge_split_warp(in + p0, m - p0, in + m, p1 - m, b - p0);
+        if (lane == 0) {
+          s_pc[warp][0] = a; s_pc[warp][1] = b; s_pc[warp][2] = p0; s_pc[warp][3] = m;
+          s_pc[warp][4] = ia; s_pc[warp][5] = ib;
+        }
+      }
+    }
+    if (lane == 0) s_ok[warp] = ok;
+  }
+  __syncthreads();
+  for (long long o = o0 + threadIdx.x; o < o1; o += kSortThreads) {
+    const bool merged = (s_ok[0] && o >= s_pc[0][0] && o < s_pc[0][1]) || (s_ok[1] && o >= s_pc[1][0] && o < s_pc[1][1]);
+    if (!merged) dst[o] = in[o];
+  }
+  for (int k = 0; k < 2; ++k) {
+    if (!s_ok[k]) continue;                          // (uniform)
+    const long long a = s_pc[k][0], b = s_pc[k][1], p0 = s_pc[k][2], m = s_pc[k][3], ia = s_pc[k][4], ib = s_pc[k][5];
+    const int na = (int)(ib - ia), nb = (int)((b - a) - na);
+    const long long jb = (a - p0) - ia;              // first key of run B in the piece
+    for (int u = threadIdx.x; u < na + nb; u += kSortThreads) s_in[u] = u < na ? in[p0 + ia + u] : in[m + jb + (u - na)];
+    __syncthreads();
+    for (int u = threadIdx.x; u < na + nb; u += kSortThreads) {
+      const unsigned long long x = s_in[u];
+      const int pos = u < na ? u + count_below<false>(s_in + na, nb, x) : (u - na) + count_below<true>(s_in, na, x);
+      dst[a + pos] = x;
+    }
+    __syncthreads();
+  }
+}
+
+// sorts every segment [lims[s], lims[s + 1]) of keys ascending (base = lims[0], total = lims[nseg] - base; scratch holds
+// total keys when total > S); slices / stride > 0: the keys come from the first pass's slices and the tile stage
+// compacts them into keys.  Ends in keys.
+int sort_segments(unsigned long long* keys, const long long* lims, long long nseg, long long base, long long total,
+                  unsigned long long* scratch, const unsigned long long* slices, long long stride, cudaStream_t st) {
+  if (total <= 0) return PPS_OK;
+  int passes = 0;
+  for (long long w = kSortTile; w < total; w <<= 1) ++passes;
+  if (passes > 0 && !scratch) return PPS_ERR_INVALID_ARG;
+  static thread_local int configured_dev = -1;
+  int dev = 0;
+  PPS_CUDA_TRY(cudaGetDevice(&dev));
+  if (configured_dev != dev) {
+    PPS_CUDA_TRY(cudaFuncSetAttribute(seg_tile_sort_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSortSmem));
+    configured_dev = dev;
+  }
+  // the tile stage writes where an even number of merge passes after it ends in keys
+  unsigned long long* const out = keys + base;
+  unsigned long long* cur = (passes & 1) ? scratch : out;
+  seg_tile_sort_kernel<<<(unsigned)((total + kSortTile - 1) / kSortTile), kSortThreads, kSortSmem, st>>>(
+      slices ? slices : out, slices ? stride : 0, cur, lims, nseg, base, total);
+  PPS_LAUNCH_CHECK("seg_tile_sort_kernel");
+  for (long long w = kSortTile; w < total; w <<= 1) {
+    unsigned long long* nxt = cur == out ? scratch : out;
+    seg_merge_kernel<<<(unsigned)((total + kMergeTile - 1) / kMergeTile), kSortThreads, 0, st>>>(cur, nxt, lims, nseg, base,
+                                                                                                  total, w);
+    PPS_LAUNCH_CHECK("seg_merge_kernel");
+    cur = nxt;
+  }
+  return PPS_OK;
+}
 }  // namespace
 
 extern "C" int pps_index_create(int device, int dim, int dtype, int precision, pps_index** out) {
@@ -307,8 +557,9 @@ extern "C" int pps_index_destroy(pps_index* x) {
   if (x->g_planes) cudaFree(x->g_planes);
   if (x->g_norm) cudaFree(x->g_norm);
   if (x->g_tags) cudaFree(x->g_tags);
-  GrowBuf* bufs[] = {&x->qs,     &x->qn,      &x->dist,    &x->tk_bound, &x->tk_cnt,  &x->tk_cand, &x->flag,
-                     &x->n_excl, &x->rm_flag, &x->rm_bsum, &x->rm_stat,  &x->rm_kept, &x->rm_piece};
+  GrowBuf* bufs[] = {&x->qs,      &x->qn,     &x->dist,    &x->tk_bound, &x->tk_cnt,    &x->tk_cand, &x->flag,
+                     &x->n_excl,  &x->rm_flag, &x->rm_bsum, &x->rm_stat,  &x->rm_kept,   &x->rm_piece, &x->rg_lim,
+                     &x->rg_cnt,  &x->rg_off, &x->rg_cap,  &x->rg_slices, &x->rg_stat, &x->rg_keys,  &x->rg_tmp};
   for (GrowBuf* b : bufs) b->release();
   x->flag_h.release();
   delete x;
@@ -521,4 +772,121 @@ extern "C" int pps_index_remove(pps_index* x, const int64_t* d_rows, long long n
   x->size = size - removed;
   if (n_removed) *n_removed = removed;
   return PPS_OK;
+}
+
+namespace {
+
+// cudaMalloc's failure is also the runtime's last error: clear it, so that the index's next call does not report it again
+int ensure_or_clear(GrowBuf& b, size_t bytes) {
+  const int rc = b.ensure(bytes);
+  if (rc != PPS_OK) cudaGetLastError();
+  return rc;
+}
+
+int range_search(pps_index* x, const void* d_q, long long nq, long long ldq, const float* d_radius, const int64_t* q_tags,
+                 long long index_offset, int flags, void* stream, int64_t* d_lims, long long* total) {
+  if (!total) return PPS_ERR_INVALID_ARG;
+  *total = 0;
+  if (nq < 0 || index_offset < 0 || (flags & ~PPS_INDEX_TKCAP(0xffff))) return PPS_ERR_INVALID_ARG;
+  if (!d_lims || (nq > 0 && (ldq < x->dim || !d_q || !d_radius))) return PPS_ERR_INVALID_ARG;
+  if (index_offset + x->size > kMaxIndex || nq > kMaxIndex) return PPS_ERR_UNSUPPORTED;
+  DeviceGuard dg(x->device);
+  if (dg.err != cudaSuccess) return pps::cuda_fail(dg.err, "cudaSetDevice");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  x->rg_total = 0;
+  const long long size = x->size;
+  if (nq == 0 || size == 0) {
+    PPS_CUDA_TRY(cudaMemsetAsync(d_lims, 0, (size_t)(nq + 1) * sizeof(int64_t), st));
+    return PPS_OK;
+  }
+  long long* lims = reinterpret_cast<long long*>(d_lims);
+  const long long hook = (flags >> 8) & 0xffff;
+  const long long slice = hook > 0 ? hook : std::min(x->rg_slice, std::max(1LL, kSliceBytes / 8 / nq));
+  PPS_TRY(ensure_or_clear(x->qs, (size_t)pps_split_bytes(nq, x->dim, x->planes)));
+  PPS_TRY(ensure_or_clear(x->qn, (size_t)nq * 2 * sizeof(float)));
+  PPS_TRY(ensure_or_clear(x->rg_lim, (size_t)nq * 4));
+  PPS_TRY(ensure_or_clear(x->rg_cnt, (size_t)nq * 2 * 4));     // first-pass counts | second-pass counters
+  PPS_TRY(ensure_or_clear(x->rg_off, (size_t)nq * 8));
+  PPS_TRY(ensure_or_clear(x->rg_cap, (size_t)nq * 4));
+  PPS_TRY(ensure_or_clear(x->rg_slices, (size_t)nq * slice * 8));
+  PPS_TRY(ensure_or_clear(x->rg_stat, 2 * 8));
+  PPS_TRY(x->flag_h.ensure(2 * 8));
+  uint32_t* lim = x->rg_lim.as<uint32_t>();
+  uint32_t* cnt = x->rg_cnt.as<uint32_t>();
+  unsigned long long* stat = x->rg_stat.as<unsigned long long>();
+  const int64_t* g_tags = q_tags ? x->g_tags : nullptr;
+
+  // 1. split, limits; 2. first pass into uniform slices; 3. counts -> lims, one 16-byte read-back
+  PPS_TRY(pps_split_rows(d_q, x->dtype, nq, x->dim, ldq, x->split_planes, x->qs.p, x->qn.as<float>(), st));
+  range_prep_kernel<<<(unsigned)((nq + 255) / 256), 256, 0, st>>>(d_radius, nq, slice, lim, cnt, x->rg_off.as<long long>(),
+                                                                  x->rg_cap.as<uint32_t>());
+  PPS_LAUNCH_CHECK("range_prep_kernel");
+  PPS_TRY(pps_search_range_tc(x->planes_at(0), x->g_norm, size, x->planes, x->capacity, x->qs.p, x->qn.as<float>(), nq,
+                              x->planes, 0, x->dim, x->precision, 0, index_offset, lim, cnt, x->rg_off.as<long long>(),
+                              x->rg_cap.as<uint32_t>(), x->rg_slices.as<uint64_t>(), g_tags, q_tags, st));
+  range_scan_kernel<<<1, 1024, 0, st>>>(cnt, nq, lims, stat);
+  PPS_LAUNCH_CHECK("range_scan_kernel");
+  PPS_CUDA_TRY(cudaMemcpyAsync(x->flag_h.p, stat, 2 * 8, cudaMemcpyDeviceToHost, st));
+  PPS_CUDA_TRY(cudaStreamSynchronize(st));
+  const long long tot = (long long)x->flag_h.as<unsigned long long>()[0];
+  const long long largest = (long long)x->flag_h.as<unsigned long long>()[1];
+  while (x->rg_slice < largest) x->rg_slice <<= 1;
+  if (tot == 0) return PPS_OK;
+
+  // 4. the sorted keys in index-owned scratch (grow-only); a result that does not fit fails here, before anything changes
+  if (tot > (1LL << 56)) return pps::cuda_fail(cudaErrorMemoryAllocation, "range search result");
+  PPS_TRY(ensure_or_clear(x->rg_keys, (size_t)tot * 8));
+  if (tot > kSortTile) PPS_TRY(ensure_or_clear(x->rg_tmp, (size_t)tot * 8));
+  unsigned long long* keys = x->rg_keys.as<unsigned long long>();
+  unsigned long long* tmp = tot > kSortTile ? x->rg_tmp.as<unsigned long long>() : nullptr;
+  if (largest > slice) {
+    // 5. a slice ran over: the same pass again, straight into the CSR layout (capacities = the exact counts)
+    uint32_t* cnt2 = cnt + nq;
+    PPS_CUDA_TRY(cudaMemsetAsync(cnt2, 0, (size_t)nq * 4, st));
+    PPS_TRY(pps_search_range_tc(x->planes_at(0), x->g_norm, size, x->planes, x->capacity, x->qs.p, x->qn.as<float>(), nq,
+                                x->planes, 0, x->dim, x->precision, 0, index_offset, lim, cnt2, lims, cnt,
+                                reinterpret_cast<uint64_t*>(keys), g_tags, q_tags, st));
+    PPS_TRY(sort_segments(keys, lims, nq, 0, tot, tmp, nullptr, 0, st));
+  } else {
+    PPS_TRY(sort_segments(keys, lims, nq, 0, tot, tmp, x->rg_slices.as<unsigned long long>(), slice, st));
+  }
+  x->rg_total = tot;
+  *total = tot;
+  return PPS_OK;
+}
+
+}  // namespace
+
+extern "C" int pps_index_range_search(pps_index* x, const void* d_q, long long nq, long long ldq, const float* d_radius,
+                                      const int64_t* d_q_tags, long long index_offset, int flags, void* stream,
+                                      int64_t* d_lims, long long* total) {
+  if (total) *total = 0;
+  if (!x) return PPS_ERR_INVALID_ARG;
+  if (d_q_tags && x->size > 0 && !x->tagged) return PPS_ERR_INVALID_ARG;     // nothing to compare the query tags with
+  return range_search(x, d_q, nq, ldq, d_radius, d_q_tags, index_offset, flags, stream, d_lims, total);
+}
+
+extern "C" int pps_index_range_keys(pps_index* x, uint64_t* d_keys, void* stream) {
+  if (!x) return PPS_ERR_INVALID_ARG;
+  if (x->rg_total == 0) return PPS_OK;
+  if (!d_keys) return PPS_ERR_INVALID_ARG;
+  DeviceGuard dg(x->device);
+  if (dg.err != cudaSuccess) return pps::cuda_fail(dg.err, "cudaSetDevice");
+  PPS_CUDA_TRY(cudaMemcpyAsync(d_keys, x->rg_keys.p, (size_t)x->rg_total * 8, cudaMemcpyDeviceToDevice,
+                               static_cast<cudaStream_t>(stream)));
+  return PPS_OK;
+}
+
+extern "C" int pps_sort_key_segments(uint64_t* keys, const int64_t* lims, long long nseg, uint64_t* scratch, void* stream) {
+  if (nseg < 0) return PPS_ERR_INVALID_ARG;
+  if (nseg == 0) return PPS_OK;
+  if (!keys || !lims) return PPS_ERR_INVALID_ARG;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  long long ends[2] = {0, 0};                        // lims[0], lims[nseg]: the grid depends on their difference only
+  PPS_CUDA_TRY(cudaMemcpyAsync(ends, lims, 8, cudaMemcpyDeviceToHost, st));
+  PPS_CUDA_TRY(cudaMemcpyAsync(ends + 1, lims + nseg, 8, cudaMemcpyDeviceToHost, st));
+  PPS_CUDA_TRY(cudaStreamSynchronize(st));
+  if (ends[0] < 0 || ends[1] < ends[0]) return PPS_ERR_INVALID_ARG;
+  return sort_segments(reinterpret_cast<unsigned long long*>(keys), reinterpret_cast<const long long*>(lims), nseg, ends[0],
+                       ends[1] - ends[0], reinterpret_cast<unsigned long long*>(scratch), nullptr, 0, st);
 }

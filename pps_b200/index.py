@@ -50,6 +50,15 @@ class GalleryIndex:
     ``[0, len)`` raises and leaves the index unchanged.  The memory is kept for later adds; an index emptied by
     ``remove`` decides again at its next non-empty add whether it is tagged.  Sharded: ``remove`` is local, not
     collective; a rank removes its own rows, and the next ``search`` gathers the new shard sizes.
+
+    ``lims, dist, index = range_search(q, radius, exclude_tags=None)`` returns every row within ``radius`` of each query
+    (FAISS's ``range_search`` layout): row r is a result of query i when ``d(i, r) <= radius[i]``, d being ``search``'s
+    distance bit for bit.  ``radius`` is a number or [nq] floats or integers (numpy or torch), converted to float32; the
+    comparison is IEEE (a negative or NaN radius selects nothing, ``inf`` every row).  ``lims`` is [nq + 1] int64 and
+    query i's results are ``dist[lims[i]:lims[i + 1]]`` (float32) and ``index[lims[i]:lims[i + 1]]`` (int64) in
+    (distance, index) order, so with ``radius[i]`` the k-th distance of ``search(q, k)`` the first k equal ``search``'s
+    row and the rest are ties at ``radius[i]``.  ``exclude_tags`` as in ``search``.  Sharded: collective, every rank gets
+    the result of one index holding the concatenated shards.
     """
 
     def __init__(self, dim, dtype=None, precision="f16x3", device=None, group=None):
@@ -176,18 +185,124 @@ class GalleryIndex:
             return dist.cpu().numpy(), index.cpu().numpy()
         return dist, index
 
+    def _radius(self, radius, nq):
+        """[nq] float32 CUDA tensor on the index's device from a number or [nq] floats / integers (numpy or torch)"""
+        import torch
+        if isinstance(radius, (bool, np.bool_)):
+            raise RuntimeError("radius: expected a number or [nq] floats, got %r" % (radius,))
+        if isinstance(radius, (int, float, np.integer, np.floating)):
+            return torch.full((nq,), float(radius), dtype=torch.float32, device=self.device)
+        if isinstance(radius, np.ndarray):
+            if not (np.issubdtype(radius.dtype, np.integer) or np.issubdtype(radius.dtype, np.floating)):
+                raise RuntimeError("radius: expected floats or integers, got %s" % radius.dtype)
+            radius = torch.from_numpy(np.ascontiguousarray(radius))
+        elif isinstance(radius, torch.Tensor):
+            if radius.dtype.is_complex or radius.dtype == torch.bool:
+                raise RuntimeError("radius: expected floats or integers, got %s" % radius.dtype)
+        else:
+            raise RuntimeError("radius: expected a number, numpy.ndarray or torch.Tensor, got %s" % type(radius))
+        if radius.dim() != 1 or int(radius.shape[0]) != nq:
+            raise RuntimeError("radius: expected a number or shape [%d], got %s" % (nq, tuple(radius.shape)))
+        return radius.to(device=self.device, dtype=torch.float32).contiguous()
+
+    def _range_keys(self, q, radius, index_offset=0, flags=0, exclude_tags=None):
+        """(lims [nq + 1] int64, keys [total] of this index alone, sorted per query, whether q was numpy); flags: 0 or the
+        PPS_INDEX_TKCAP(n) hook (keys per query in the first pass's slices)."""
+        import torch
+        x, is_np = self._rows(q, "q")
+        nq = int(x.shape[0])
+        ldq = int(x.stride(0)) if nq else self.dim
+        r = self._radius(radius, nq)
+        t = None if exclude_tags is None else self._tags(exclude_tags, nq, "exclude_tags")
+        lims = torch.empty(nq + 1, dtype=torch.int64, device=self.device)
+        total = C.c_longlong(0)
+        with torch.cuda.device(self.device):
+            _lib.check(self._lib.pps_index_range_search(self._h, _lib.ptr(x), nq, ldq, _lib.ptr(r), _lib.ptr(t),
+                                                        int(index_offset), int(flags), _lib.stream_ptr(), _lib.ptr(lims),
+                                                        C.byref(total)), "pps_index_range_search")
+            keys = torch.empty(int(total.value), dtype=torch.int64, device=self.device)
+            _lib.check(self._lib.pps_index_range_keys(self._h, _lib.ptr(keys), _lib.stream_ptr()), "pps_index_range_keys")
+        return lims, keys, is_np
+
+    def _unpack_range(self, lims, keys, is_np):
+        import torch
+        n = int(keys.shape[0])
+        dist = torch.empty(n, dtype=torch.float32, device=self.device)
+        index = torch.empty(n, dtype=torch.int32, device=self.device)
+        with torch.cuda.device(self.device):
+            _lib.check(self._lib.pps_topk_unpack(_lib.ptr(keys), n, 1, _lib.ptr(dist), _lib.ptr(index), _lib.stream_ptr()),
+                       "pps_topk_unpack")
+        index = index.long()
+        if is_np:
+            return lims.cpu().numpy(), dist.cpu().numpy(), index.cpu().numpy()
+        return lims, dist, index
+
+    def _offset(self):
+        """index_offset of this rank's rows: one all-gather of the shard sizes (0 without a group)"""
+        import torch
+        if self.group is None:
+            return 0
+        import torch.distributed as dist_mod
+        mine = torch.tensor([len(self)], dtype=torch.int64, device=self.device)
+        sizes = [torch.empty_like(mine) for _ in range(dist_mod.get_world_size(self.group))]
+        dist_mod.all_gather(sizes, mine, group=self.group)
+        return int(sum(int(s.item()) for s in sizes[:dist_mod.get_rank(self.group)]))
+
+    def range_search(self, q, radius, exclude_tags=None):
+        """(lims [nq + 1] int64, dist [total] float32, index [total] int64): every gallery row within radius of each query
+        row (with exclude_tags: of the rows whose tag is not the query's), per query in (distance, index) order."""
+        lims, keys, is_np = self._range_keys(q, radius, self._offset(), exclude_tags=exclude_tags)
+        if self.group is not None:
+            lims, keys = gather_range_keys(lims, keys, self.group)
+        return self._unpack_range(lims, keys, is_np)
+
     def search(self, q, k, exclude_tags=None):
         """(dist [nq, k] float32, index [nq, k] int64) of the k nearest gallery rows of every query row (with
         exclude_tags: of the rows whose tag is not the query's)."""
-        import torch
-        offset = 0
-        if self.group is not None:
-            import torch.distributed as dist_mod
-            mine = torch.tensor([len(self)], dtype=torch.int64, device=self.device)
-            sizes = [torch.empty_like(mine) for _ in range(dist_mod.get_world_size(self.group))]
-            dist_mod.all_gather(sizes, mine, group=self.group)
-            offset = int(sum(int(s.item()) for s in sizes[:dist_mod.get_rank(self.group)]))
-        keys, is_np = self._search_keys(q, k, offset, exclude_tags=exclude_tags)
+        keys, is_np = self._search_keys(q, k, self._offset(), exclude_tags=exclude_tags)
         if self.group is not None:
             keys = merge_topk_keys(keys, int(k), self.group)
         return self._unpack(keys, is_np)
+
+
+def gather_range_keys(lims, keys, group):
+    """All-gather every rank's range-search result (lims [nq + 1], keys [total]) and merge them (merge_range_lists)."""
+    import torch
+    import torch.distributed as dist_mod
+    world = dist_mod.get_world_size(group)
+    all_lims = [torch.empty_like(lims) for _ in range(world)]
+    dist_mod.all_gather(all_lims, lims, group=group)
+    totals = [int(x[-1].item()) for x in all_lims]
+    pad = torch.zeros(max(totals), dtype=torch.int64, device=keys.device)
+    pad[:keys.shape[0]] = keys
+    all_keys = [torch.empty_like(pad) for _ in range(world)]
+    dist_mod.all_gather(all_keys, pad, group=group)
+    return merge_range_lists(all_lims, [k[:n] for k, n in zip(all_keys, totals)])
+
+
+def merge_range_lists(lims_list, keys_list):
+    """One range-search result from several (lims [nq + 1] int64, keys [total]) of disjoint row sets (shards, in rank
+    order): every query's keys of every list, query-major, then each query's keys sorted (pps_sort_key_segments)."""
+    import torch
+    nq = int(lims_list[0].shape[0]) - 1
+    dev = lims_list[0].device
+    counts = torch.stack([x[1:] - x[:-1] for x in lims_list])                        # [lists, nq]
+    lims = torch.zeros(nq + 1, dtype=torch.int64, device=dev)
+    lims[1:] = torch.cumsum(counts.sum(0), 0)
+    before = torch.cumsum(counts, 0) - counts                                         # keys of earlier lists, per query
+    total = int(lims[-1].item())
+    keys = torch.empty(total, dtype=torch.int64, device=dev)
+    for j, (lx, kx) in enumerate(zip(lims_list, keys_list)):
+        n = int(kx.shape[0])
+        if n == 0:
+            continue
+        q = torch.repeat_interleave(torch.arange(nq, device=dev), counts[j])        # query of every key of list j
+        dest = lims[:-1][q] + before[j][q] + (torch.arange(n, device=dev) - lx[:-1][q])
+        keys[dest] = kx
+    if total:
+        lib = _lib.load()
+        scratch = torch.empty_like(keys)
+        with torch.cuda.device(dev):
+            _lib.check(lib.pps_sort_key_segments(_lib.ptr(keys), _lib.ptr(lims), nq, _lib.ptr(scratch), _lib.stream_ptr()),
+                       "pps_sort_key_segments")
+    return lims, keys

@@ -37,8 +37,20 @@ the 9 M left).  A line records:
   search_ms / fresh_search_ms  medians of searches (per batch size) of the compacted index and of a fresh index of the
                                same rows, alternated; agree: their outputs are identical (indices and distance bits)
 
+--range measures GalleryIndex.range_search instead, one line per (gallery, batch, target): every query gets the radius
+that admits about `target` rows (its target-th distance, from a top-128 search of the same index for 10 and 100 hits,
+from compute_dist's rows of the batch otherwise), targets 10, 1 000 and 100 000, plus inf (every row) at 1 and 16
+queries.  Default galleries fp16_10M and fp32_520k, batches 1, 16, 64, 256.  A line records:
+  range_ms / topk_ms     medians of range_search and of search(q, 100) on the same index, alternated
+  hits_mean, hits_max    results per query
+  total_keys             keys of the whole result (8 bytes each)
+  split_ms               one more call with CUDA events around its parts: the first pass (search kernel), the second
+                         pass (when a slice ran over) and the sort, from torch.profiler's kernel times
+  ok                     the output against the top-k invariant: the first k results of each query equal search's row
+                         (k = min(100, hits)), every result is within the radius, lims add up
+
 usage: python tools/index_bench.py [--reps 10] [--warmup 2] [--out FILE] [--cases fp16_1M,fp16_10M,fp32_520k]
-                                   [--tags none,cam6,half,junk] [--batches 1,16,64,256,3368] [--remove]
+                                   [--tags none,cam6,half,junk] [--batches 1,16,64,256,3368] [--remove] [--range]
 """
 from __future__ import annotations
 
@@ -246,6 +258,105 @@ def run_remove_case(name, batches, reps, warmup, emit):
     torch.cuda.empty_cache()
 
 
+RANGE_TARGETS = [10, 1000, 100000, "inf"]
+
+
+def range_radius(idx, q, own_rows, target):
+    """[nq] float32 radii admitting about `target` rows per query"""
+    import torch
+    if target == "inf":
+        return torch.full((q.shape[0],), float("inf"), dtype=torch.float32, device=q.device)
+    if target <= 128:
+        d, _ = idx.search(q, target)
+        return d[:, target - 1].contiguous()
+    return torch.kthvalue(own_rows(), target, dim=1).values.contiguous()
+
+
+def check_range(idx, q, radius, out):
+    """the top-k invariant (k = min(100, hits)) and the radius, on the GPU"""
+    import torch
+    lims, dist, index = out
+    counts = (lims[1:] - lims[:-1]).cpu()
+    if int(lims[0]) != 0 or int(lims[-1]) != dist.shape[0] or (counts < 0).any():
+        return False
+    if not bool((dist <= torch.repeat_interleave(radius, counts.to(radius.device))).all()):
+        return False
+    k = int(min(100, int(counts.min())))
+    if k == 0:
+        return True
+    sd, si = idx.search(q, k)
+    first = lims[:-1, None] + torch.arange(k, device=lims.device)[None, :]
+    return bool(torch.equal(index[first], si) and torch.equal(dist[first].view(torch.int32), sd.view(torch.int32)))
+
+
+def range_split_ms(fn):
+    """device time of one call's kernels by part: first pass, second pass (search kernels after the first), sort"""
+    import torch
+    from torch.profiler import ProfilerActivity, profile
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        fn()
+        torch.cuda.synchronize()
+    search, sort = [], 0.0
+    for ev in prof.events():
+        if ev.device_type != torch.autograd.DeviceType.CUDA:
+            continue
+        us = ev.device_time_total if hasattr(ev, "device_time_total") else ev.cuda_time_total
+        if "dist_tc2_kernel" in ev.name:
+            search.append((ev.time_range.start, us))
+        elif "seg_tile_sort" in ev.name or "seg_merge" in ev.name:
+            sort += us
+    search.sort()
+    return {"first_pass_ms": round(search[0][1] / 1e3, 4) if search else None,
+            "second_pass_ms": round(sum(u for _, u in search[1:]) / 1e3, 4),
+            "sort_ms": round(sort / 1e3, 4)}
+
+
+def run_range_case(name, batches, reps, warmup, emit):
+    import torch
+    import pps_b200
+    from pps_b200 import synthetic
+    ng, dtype_name = CASES[name]
+    dev = torch.device("cuda")
+    tdt = torch.float16 if dtype_name == "fp16" else torch.float32
+    qid, _, gid, _ = synthetic.make_distractor_ids(max(batches), ng)
+    q_all = synthetic.make_features_device(qid, DIM, 750, 4.0, 7, dev, tdt)
+    g = synthetic.make_features_device(gid, DIM, 750, 4.0, 1000, dev, tdt)
+    idx = pps_b200.GalleryIndex(DIM, dtype=tdt, precision="f16x3")
+    idx.add(g)
+    gpu, watts = card(torch.cuda.current_device())
+    for nq in batches:
+        q = q_all[:nq].contiguous()
+        rows = {}
+
+        def own_rows():                    # compute_dist's rows of the batch, in pieces of the gallery (memory)
+            if "d" not in rows:
+                step = max(1, (1 << 30) // (4 * nq))
+                rows["d"] = torch.cat([pps_b200.compute_dist(q, g[i:i + step]).float() for i in range(0, ng, step)], 1)
+            return rows["d"]
+        for target in RANGE_TARGETS:
+            if target == "inf" and nq > 16:
+                continue
+            if target != "inf" and target >= ng:
+                continue
+            radius = range_radius(idx, q, own_rows, target)
+            s_ms, r_ms, out = timed_alternating(lambda: idx.search(q, K), lambda: idx.range_search(q, radius), reps, warmup)
+            lims = out[0]
+            counts = (lims[1:] - lims[:-1]).float()
+            rec = {"case": name, "dtype": dtype_name, "precision": "f16x1" if dtype_name == "fp16" else "f16x3", "ng": ng,
+                   "dim": DIM, "nq": nq, "target_hits": target, "range_ms": round(r_ms, 4), "topk_ms": round(s_ms, 4),
+                   "ratio": round(r_ms / s_ms, 3), "hits_mean": round(float(counts.mean()), 1),
+                   "hits_max": int(counts.max()), "total_keys": int(lims[-1])}
+            rec.update(range_split_ms(lambda: idx.range_search(q, radius)))
+            rec["ok"] = check_range(idx, q, radius, out)
+            rec.update({"k_topk": K, "reps": reps, "gpu": gpu, "power_limit_w": watts})
+            emit(rec)
+            del out
+        rows.clear()
+        torch.cuda.empty_cache()
+    del idx, g, q_all
+    torch.cuda.empty_cache()
+
+
 def run_case(name, reps, warmup, emit, batches=BATCHES):
     import torch
     import pps_b200
@@ -293,6 +404,8 @@ def main():
     ap.add_argument("--tags", default="none", help="comma-separated tag modes: " + ", ".join(TAG_MODES))
     ap.add_argument("--batches", default=",".join(str(b) for b in BATCHES))
     ap.add_argument("--remove", action="store_true", help="measure GalleryIndex.remove (default batches 1,64)")
+    ap.add_argument("--range", action="store_true",
+                    help="measure GalleryIndex.range_search (default galleries fp16_10M,fp32_520k, batches 1,16,64,256)")
     args = ap.parse_args()
     import torch
     if not torch.cuda.is_available():
@@ -308,6 +421,10 @@ def main():
     batches = [int(b) for b in args.batches.split(",") if b]
     if args.remove and args.batches == ap.get_default("batches"):
         batches = [1, 64]
+    if args.range and args.batches == ap.get_default("batches"):
+        batches = [1, 16, 64, 256]
+    if args.range and args.cases == ap.get_default("cases"):
+        names = ["fp16_10M", "fp32_520k"]
 
     def emit(rec):
         line = json.dumps(rec)
@@ -319,6 +436,10 @@ def main():
     if args.remove:
         for c in names:
             run_remove_case(c, batches, args.reps, args.warmup, emit)
+        return
+    if args.range:
+        for c in names:
+            run_range_case(c, batches, args.reps, args.warmup, emit)
         return
     tagged = [m for m in modes if m != "none"]
     for c in names:
