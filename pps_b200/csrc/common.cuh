@@ -124,6 +124,12 @@ __device__ __forceinline__ uint32_t ld_volatile_u32(const uint32_t* p) {
 __device__ __forceinline__ void st_volatile_u32(uint32_t* p, uint32_t v) {
   asm volatile("st.volatile.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
 }
+// max(x, 0) that keeps NaN, as the reference's d2[d2 < 0] = 0 does (fmaxf(NaN, 0) is 0); one FMNMX like fmaxf
+__device__ __forceinline__ float clamp0_keep_nan(float x) {
+  float y;
+  asm("max.NaN.f32 %0, %1, 0f00000000;" : "=f"(y) : "f"(x));
+  return y;
+}
 __device__ __forceinline__ float sqrt_approx(float x) {
   float y;
   asm("sqrt.approx.f32 %0, %1;" : "=f"(y) : "f"(x));

@@ -467,7 +467,7 @@ __device__ __forceinline__ void dist_tc2_body(const CUtensorMap& tmA, const CUte
             for (int e = 0; e < 4; ++e) {
               const float dot = __uint_as_float(r[4 * j + e]);
               float d2 = __fadd_rn(__fmaf_rn(sc[e], dot, qq[e]), an);
-              d2 = fmaxf(d2, 0.f);
+              d2 = clamp0_keep_nan(d2);
               v[4 * j + e] = __float_as_uint(want_sq ? d2 : (sqrt_rn ? __fsqrt_rn(d2) : sqrt_approx(d2)));
               // distances are >= 0: bits order like values.  EPI_RANGE: bb is the limit bits(radius) + 1 (0: none)
               hit |= (epi_range(EPI) ? v[4 * j + e] < bb[e] : v[4 * j + e] <= bb[e]) & (4 * j + e < valid_cols);
@@ -519,22 +519,23 @@ __device__ __forceinline__ void dist_tc2_body(const CUtensorMap& tmA, const CUte
             for (int e = 0; e < 4; ++e) {
               const float dot = __uint_as_float(r[4 * j + e]);
               float d2 = __fadd_rn(__fmaf_rn(-2.f, dot, an), bb[e]);      // the EPI_DIST arithmetic, bit for bit
-              d2 = fmaxf(d2, 0.f);
+              d2 = clamp0_keep_nan(d2);
               d[4 * j + e] = want_sq ? d2 : sqrt_approx(d2);
             }
           }
           // lower bound of every element among this row's thresholds: 32 independent searches per step, the first two
           // levels against pivots held in registers.  The position is kept as the BYTE offset of (threshold lo, this row)
           // in the [threshold][row] tables, so that a probe is one LDS at (uniform base + offset) and the counter of the
-          // result sits at the same offset of the counter table.
+          // result sits at the same offset of the counter table.  "Above t" is the unordered !(d <= t), so that a NaN
+          // distance falls past every threshold (as in the reference's argsort) for the price of a plain compare.
           uint32_t off[32];
           const int half1 = p_cap >> 1, half2 = (p_cap - half1) >> 1;
           const uint32_t row_off = (uint32_t)row * 4u, h1o = (uint32_t)half1 * 512u, h2o = (uint32_t)half2 * 512u;
 #pragma unroll
           for (int e = 0; e < 32; ++e) {
-            const bool up = piv1 < d[e];
+            const bool up = !(d[e] <= piv1);
             off[e] = row_off + (up ? h1o : 0u);
-            off[e] += ((up ? piv2b : piv2a) < d[e]) ? h2o : 0u;
+            off[e] += !(d[e] <= (up ? piv2b : piv2a)) ? h2o : 0u;
           }
           const uint32_t thr_base = smem_u32(thr_s);
           int len = p_cap - half1 - half2;
@@ -542,13 +543,13 @@ __device__ __forceinline__ void dist_tc2_body(const CUtensorMap& tmA, const CUte
             const int half = len >> 1;
             const uint32_t probe = thr_base + (uint32_t)(half - 1) * 512u, step = (uint32_t)half * 512u;
 #pragma unroll
-            for (int e = 0; e < 32; ++e) off[e] += (lds_f32(probe + off[e]) < d[e]) ? step : 0u;
+            for (int e = 0; e < 32; ++e) off[e] += !(d[e] <= lds_f32(probe + off[e])) ? step : 0u;
             len -= half;
           }
           bool tie = false;
 #pragma unroll
           for (int e = 0; e < 32; ++e) {
-            off[e] += (lds_f32(thr_base + off[e]) < d[e]) ? 512u : 0u;
+            off[e] += !(d[e] <= lds_f32(thr_base + off[e])) ? 512u : 0u;
             tie |= (d[e] == dstar);
           }
           // one fire-and-forget shared-memory add per element (no read-back, so no dependent chain).  An element beyond every
@@ -624,7 +625,7 @@ __device__ __forceinline__ void dist_tc2_body(const CUtensorMap& tmA, const CUte
                 // same association as the reference: (-2*ab + |a|^2) + |b|^2   (-2*ab is exact, so the FMA rounds once;
                 // with scaled operands sc = -2 / (s_a s_b) and sc * dot is the same exact product)
                 float d2 = __fadd_rn(__fmaf_rn(sc[e], dot, an), bb[e]);
-                d2 = fmaxf(d2, 0.f);
+                d2 = clamp0_keep_nan(d2);
                 v[e] = want_sq ? d2 : (sqrt_rn ? __fsqrt_rn(d2) : sqrt_approx(d2));
               }
             }

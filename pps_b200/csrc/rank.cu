@@ -256,7 +256,7 @@ __global__ void __launch_bounds__(kCntThreads, TOPK ? 6 : 16) rank_count_kernel(
         const uint32_t info = binfo[b];
         const int first = (int)(info >> 16), cnt = (int)(info & 0xffffu);
         int j = 0;
-        while (j < cnt && thr[first + j] < d) ++j;
+        while (j < cnt && !(d <= thr[first + j])) ++j;           // (unordered: a NaN distance is past every threshold)
         if (j < cnt) atomicAdd(&exact[first + j], 1u);
         if (d == dstar) tie_corr += ((col0 + col) < gstar ? 1u : 0u) - 1u;
       }

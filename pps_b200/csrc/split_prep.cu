@@ -127,8 +127,10 @@ __global__ void __launch_bounds__(32 * kSplitWarps) split_rows_kernel(const void
 // fp32 rows -> TWO fp16 residual planes of the row scaled by a power of two (PPS_SPLIT_F16_SCALED): with
 // s = 2^e chosen per row so that max|x| * s lies in [2^14, 2^15), p0 = fp16(x s), p1 = fp16(x s - p0).  fp16 carries
 // 11 significant bits, so p0 + p1 holds 22 bits of every element (bf16 planes: 16) at the same two-plane cost, and
-// the scaling keeps p1 out of the fp16 subnormals.  The distance epilogue multiplies the accumulator by the two
-// inverse scales - exact, they are powers of two.  out_sqnorm[row] = |x|^2, out_sqnorm[rows + row] = 1 / s.
+// the scaling keeps p1 out of the fp16 subnormals.  The distance epilogue multiplies the accumulator by the product of
+// the two inverse scales, formed as one float.  e <= 63 keeps that product a normal float (>= 2^-126), so it is exact:
+// rows with max|x| < 2^-48 are scaled less than fully (max|x| s < 2^14), which costs only their smallest elements
+// bits.  out_sqnorm[row] = |x|^2, out_sqnorm[rows + row] = 1 / s.
 // Two streaming passes over the row (max + norm, then split); the second one hits L1 / L2.  Keeping the row in registers
 // between the passes (kF16Cache4 = 16: 98 registers, 16 warps per SM) measured SLOWER: 2.9 TB/s against 4.6-5.1 TB/s
 // (profiles/r02_notes.md).
@@ -191,7 +193,7 @@ __global__ void __launch_bounds__(32 * kSplitWarps) split_rows_f16s_kernel(const
     int ex;
     frexpf(mx, &ex);                        // mx = m * 2^ex, m in [0.5, 1)
     e = 15 - ex;
-    e = e > 100 ? 100 : (e < -100 ? -100 : e);
+    e = e > 63 ? 63 : (e < -100 ? -100 : e);   // 63: 1 / (s_a s_b) >= 2^-126 (see above)
   }
   const float s = ldexpf(1.f, e), inv = ldexpf(1.f, -e);
   const long long plane_stride = rows * (long long)kpad;
