@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define PPS_ABI_VERSION 9
+#define PPS_ABI_VERSION 10
 
 /* ---- error codes (the Python mirror turns every non-zero code into RuntimeError,
  * like CAFFE_ENFORCE does: detectron/tests/test_zero_even_op.py:50-53) ---- */
@@ -618,6 +618,32 @@ int pps_evaluate_host(const float* q_feats, long long nq,
  *                      of 4 096 in shared memory, then by ceil(log2(total / 4096)) merge passes; segments may hold from 0
  *                      keys to all of them.  Equal keys are allowed; keys that are unique in their segment (range search:
  *                      the row index is in the low bits) give one result whatever order they came in.
+ * Grouped search: every row may carry one int64 group (a tracklet, an identity), and a grouped search returns the nearest
+ * row of each of the k nearest groups.  Order the rows a search (plain or excluding) admits by their key; keep the first
+ * row of each group; return the first k.  Every row its own group: the search's keys, bit for bit.
+ * pps_index_add_grouped   pps_index_add with d_groups[n] (device int64, required) and d_tags[n] (device, may be null).
+ *                      The first non-empty add decides whether the index is grouped (and whether tagged); a later add
+ *                      of the other kind is PPS_ERR_INVALID_ARG.
+ * pps_index_search_groups   d_keys[nq][k] = the keys of each query's k nearest groups' nearest rows, d_groups[nq][k] their
+ *                      groups; past the last group ~0 / -1.  d_q_tags (may be null): leave out rows as
+ *                      pps_index_search_excluding.  A non-empty ungrouped index: PPS_ERR_INVALID_ARG.  Schedule: materialised
+ *                      blocks swept by pps_topk_group_update until every query holds k groups (a 4-byte read-back per
+ *                      block), one counting pass of pps_search_range_tc over those rows (L = the most rows of a query at
+ *                      or below its bound, a 4-byte read-back), then chunks of pps_search_topk(_excl)_tc +
+ *                      pps_topk_group_merge sized cap * rows done / (2.2 max(k, L)), cap = 8 192 candidates per query;
+ *                      the overflow read-back; on overflow materialised blocks only.  flags: as pps_index_search
+ *                      (PPS_INDEX_TKCAP(n) up to 8 192).
+ * pps_index_group_stats    the schedule of the index's last grouped search: rows swept as materialised blocks before
+ *                      the chunks, chunks, and whether the materialised fallback ran (host pointers, each may be null).
+ * pps_topk_group_update    grouped counterpart of pps_topk_update: dist [nq][ldd] columns c < ncols (gallery index col0 + c,
+ *                      group g_groups[c]) into the grouped state topk_key / topk_group [nq][k] (initialised to ~0 / -1).
+ *                      g_tags / q_tags: both null, or both set (columns with g_tags[c] == q_tags[q] are left out).
+ * pps_topk_group_merge     grouped counterpart of pps_topk_merge: candidates tk_cand[q][tk_cap] of pps_search_topk_tc
+ *                      (tk_cnt[q] of them) with groups g_groups[index - index_offset] into the state; new tk_bound
+ *                      (the k-th key's distance bits, all ones while fewer than k groups are held), tk_cnt = 0,
+ *                      *overflow = 1 if a buffer ran over.
+ * pps_topk_group_merge_lists   the grouped state of `lists` states keys / groups [lists][nq][k] (disjoint row sets, e.g.
+ *                      the shards of a gallery; a group may span lists) -> out_key / out_group [nq][k].
  * Calls on one index are ordered by the caller (one stream, or events between streams); every call sets the index's
  * device for its duration.  A sharded gallery: one index per rank, index_offset = the rows of the ranks before, an
  * all-gather of the [nq][k] keys and the k smallest per query (every rank's list is sorted, keys are unique).
@@ -661,6 +687,20 @@ int       pps_index_range_search(pps_index* idx, const void* d_q, long long nq, 
                                  int64_t* d_lims, long long* total);
 int       pps_index_range_keys(pps_index* idx, uint64_t* d_keys, void* stream);
 int       pps_sort_key_segments(uint64_t* keys, const int64_t* lims, long long nseg, uint64_t* scratch, void* stream);
+int       pps_index_add_grouped(pps_index* idx, const void* d_rows, long long n, long long ld, const int64_t* d_tags,
+                                const int64_t* d_groups, void* stream);
+int       pps_index_search_groups(pps_index* idx, const void* d_q, long long nq, long long ldq,
+                                  const int64_t* d_q_tags /*nullable*/, int k, long long index_offset, int flags, void* stream,
+                                  uint64_t* d_keys, int64_t* d_groups);
+int       pps_index_group_stats(const pps_index* idx, long long* prefix_rows, long long* chunks, int* fallback);
+int pps_topk_group_update(const float* dist, long long ldd, long long nq, long long ncols, long long col0,
+                          const int64_t* g_groups, const int64_t* g_tags, const int64_t* q_tags, uint64_t* topk_key,
+                          int64_t* topk_group, int k, void* stream);
+int pps_topk_group_merge(uint64_t* topk_key, int64_t* topk_group, long long nq, int k, const uint64_t* tk_cand, int tk_cap,
+                         uint32_t* tk_cnt, uint32_t* tk_bound, const int64_t* g_groups, long long index_offset,
+                         int32_t* overflow, void* stream);
+int pps_topk_group_merge_lists(const uint64_t* keys, const int64_t* groups, int lists, long long nq, int k,
+                               uint64_t* out_key, int64_t* out_group, void* stream);
 
 /* ------------------------------------------------------------------------------------
  * Next row (SURVEY §8f.4) — the reference's training-side triplet mining ops.

@@ -13,7 +13,7 @@ import threading
 from . import build as _build
 
 # ---- constants (keep in sync with include/pps_b200.h) ----
-ABI_VERSION = 9
+ABI_VERSION = 10
 PPS_OK = 0
 PPS_ERR_INVALID_ARG = -1
 PPS_ERR_SHAPE = -2
@@ -168,6 +168,12 @@ SIGNATURES = {
     "pps_index_range_search": (_i, [_vp, _vp, _ll, _ll, _vp, _vp, _ll, _i, _vp, _vp, C.POINTER(_ll)]),
     "pps_index_range_keys": (_i, [_vp, _vp, _vp]),
     "pps_sort_key_segments": (_i, [_vp, _vp, _ll, _vp, _vp]),
+    "pps_index_add_grouped": (_i, [_vp, _vp, _ll, _ll, _vp, _vp, _vp]),
+    "pps_index_search_groups": (_i, [_vp, _vp, _ll, _ll, _vp, _i, _ll, _i, _vp, _vp, _vp]),
+    "pps_index_group_stats": (_i, [_vp, C.POINTER(_ll), C.POINTER(_ll), C.POINTER(_i)]),
+    "pps_topk_group_update": (_i, [_vp, _ll, _ll, _ll, _ll, _vp, _vp, _vp, _vp, _vp, _i, _vp]),
+    "pps_topk_group_merge": (_i, [_vp, _vp, _ll, _i, _vp, _i, _vp, _vp, _vp, _ll, _vp, _vp]),
+    "pps_topk_group_merge_lists": (_i, [_vp, _vp, _i, _ll, _i, _vp, _vp, _vp]),
     "pps_pairwise_distance_fwd": (_i, [_vp, _i, _i, _vp, _vp]),
     "pps_pairwise_distance_bwd": (_i, [_vp, _vp, _i, _i, _vp, _vp]),
     "pps_batch_hard_fwd": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _vp]),

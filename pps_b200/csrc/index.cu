@@ -41,6 +41,7 @@ using pps::PinBuf;
 
 constexpr long long kPrefixRows = 32768;
 constexpr int kTkCap = 2048;
+constexpr int kGroupTkCap = 8192;     // grouped search: candidates per query and chunk (DESIGN §4.16)
 constexpr long long kMinCapacity = 1024;
 constexpr long long kMaxIndex = 0x7fffffffLL;   // keys carry the gallery index in 32 bits, unpacked as int32
 
@@ -65,12 +66,16 @@ struct pps_index {
   void* g_planes = nullptr;     // [planes][capacity][kpad] 16-bit elements
   float* g_norm = nullptr;      // [capacity] norms (+ [capacity] inverse scales for PPS_PREC_F16X3)
   int64_t* g_tags = nullptr;    // [capacity] row tags (tagged indexes)
+  int64_t* g_groups = nullptr;  // [capacity] row groups (grouped indexes)
   bool tagged = false;          // decided by the first non-empty add
+  bool grouped = false;         // decided by the first non-empty add
   GrowBuf qs, qn, dist, tk_bound, tk_cnt, tk_cand, flag, n_excl;
   GrowBuf rm_flag, rm_bsum, rm_stat, rm_kept, rm_piece;    // scratch of pps_index_remove
   GrowBuf rg_lim, rg_cnt, rg_off, rg_cap, rg_slices, rg_stat, rg_keys, rg_tmp;   // scratch of pps_index_range_search
   long long rg_total = 0;       // keys of the last range search (in rg_keys)
   long long rg_slice = 4096;    // first-pass slice per query: a power of two >= the largest count seen so far
+  long long last_prefix = 0, last_chunks = 0;   // schedule of the last grouped search (pps_index_group_stats)
+  int last_fallback = 0;
   PinBuf flag_h;
   bool scaled() const { return precision == PPS_PREC_F16X3; }
   size_t plane_bytes(long long rows) const { return (size_t)rows * kpad * 2; }
@@ -79,20 +84,23 @@ struct pps_index {
 
 namespace {
 
-// capacity -> new_cap: planes, both halves of the norm array and the tags move to their new offsets
+// capacity -> new_cap: planes, both halves of the norm array, the tags and the groups move to their new offsets
 int grow(pps_index* x, long long need, cudaStream_t st) {
   long long cap = std::max(x->capacity * 2, std::max(need, kMinCapacity));
   if (cap > kMaxIndex) cap = kMaxIndex;
   void* planes = nullptr;
   float* norm = nullptr;
   int64_t* tags = nullptr;
+  int64_t* groups = nullptr;
   const size_t norm_n = (size_t)cap * (x->scaled() ? 2 : 1);
   cudaError_t e = cudaMalloc(&planes, (size_t)x->planes * x->plane_bytes(cap));
   if (e == cudaSuccess) e = cudaMalloc(&norm, norm_n * sizeof(float));
   if (e == cudaSuccess && x->tagged) e = cudaMalloc(&tags, (size_t)cap * sizeof(int64_t));
+  if (e == cudaSuccess && x->grouped) e = cudaMalloc(&groups, (size_t)cap * sizeof(int64_t));
   if (e != cudaSuccess) {
     if (planes) cudaFree(planes);
     if (norm) cudaFree(norm);
+    if (tags) cudaFree(tags);
     return pps::cuda_fail(e, "cudaMalloc(index)");
   }
   if (x->size > 0) {
@@ -106,14 +114,18 @@ int grow(pps_index* x, long long need, cudaStream_t st) {
                                    cudaMemcpyDeviceToDevice, st));
     if (tags)
       PPS_CUDA_TRY(cudaMemcpyAsync(tags, x->g_tags, (size_t)x->size * sizeof(int64_t), cudaMemcpyDeviceToDevice, st));
+    if (groups)
+      PPS_CUDA_TRY(cudaMemcpyAsync(groups, x->g_groups, (size_t)x->size * sizeof(int64_t), cudaMemcpyDeviceToDevice, st));
     PPS_CUDA_TRY(cudaStreamSynchronize(st));     // the old buffers are read until here
   }
   if (x->g_planes) cudaFree(x->g_planes);
   if (x->g_norm) cudaFree(x->g_norm);
   if (x->g_tags) cudaFree(x->g_tags);
+  if (x->g_groups) cudaFree(x->g_groups);
   x->g_planes = planes;
   x->g_norm = norm;
   x->g_tags = tags;
+  x->g_groups = groups;
   x->capacity = cap;
   return PPS_OK;
 }
@@ -278,6 +290,12 @@ __global__ void __launch_bounds__(kRmThreads) rm_gather_kernel(const int32_t* __
   }
 }
 
+// the groups of piece rows j < rows (kept apart from rm_gather_kernel, which moves everything else)
+__global__ void __launch_bounds__(kRmThreads) rm_gather_i64_kernel(const int32_t* __restrict__ kept, long long rows,
+                                                                   const int64_t* __restrict__ src, int64_t* __restrict__ dst) {
+  const long long j = blockIdx.x * (long long)kRmThreads + threadIdx.x;
+  if (j < rows) dst[j] = src[kept[j]];
+}
 
 // ---- range search (pps_index_range_search) and the segment sort (pps_sort_key_segments) ----
 constexpr int kSortThreads = 256;
@@ -557,6 +575,7 @@ extern "C" int pps_index_destroy(pps_index* x) {
   if (x->g_planes) cudaFree(x->g_planes);
   if (x->g_norm) cudaFree(x->g_norm);
   if (x->g_tags) cudaFree(x->g_tags);
+  if (x->g_groups) cudaFree(x->g_groups);
   GrowBuf* bufs[] = {&x->qs,      &x->qn,     &x->dist,    &x->tk_bound, &x->tk_cnt,    &x->tk_cand, &x->flag,
                      &x->n_excl,  &x->rm_flag, &x->rm_bsum, &x->rm_stat,  &x->rm_kept,   &x->rm_piece, &x->rg_lim,
                      &x->rg_cnt,  &x->rg_off, &x->rg_cap,  &x->rg_slices, &x->rg_stat, &x->rg_keys,  &x->rg_tmp};
@@ -570,23 +589,31 @@ extern "C" long long pps_index_size(const pps_index* x) { return x ? x->size : P
 
 namespace {
 
-int add_rows(pps_index* x, const void* d_rows, long long n, long long ld, const int64_t* d_tags, void* stream) {
+int add_rows(pps_index* x, const void* d_rows, long long n, long long ld, const int64_t* d_tags, const int64_t* d_groups,
+             void* stream) {
   if (!x || n < 0 || ld < x->dim) return PPS_ERR_INVALID_ARG;
   if (n == 0) return PPS_OK;
   if (!d_rows) return PPS_ERR_INVALID_ARG;
   if (x->size > 0 && x->tagged != (d_tags != nullptr)) return PPS_ERR_INVALID_ARG;   // all rows tagged, or none
+  if (x->size > 0 && x->grouped != (d_groups != nullptr)) return PPS_ERR_INVALID_ARG; // all rows grouped, or none
   if (x->size + n > kMaxIndex) return PPS_ERR_UNSUPPORTED;
   DeviceGuard dg(x->device);
   if (dg.err != cudaSuccess) return pps::cuda_fail(dg.err, "cudaSetDevice");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (x->size == 0) x->tagged = d_tags != nullptr;
-  if (x->size + n > x->capacity || (x->tagged && !x->g_tags)) PPS_TRY(grow(x, x->size + n, st));
+  if (x->size == 0) {
+    x->tagged = d_tags != nullptr;
+    x->grouped = d_groups != nullptr;
+  }
+  if (x->size + n > x->capacity || (x->tagged && !x->g_tags) || (x->grouped && !x->g_groups))
+    PPS_TRY(grow(x, x->size + n, st));
   // pps_split_rows_slab reads row r of the source at base + r * ld: the new rows sit at rows [size, size + n) of it
   const size_t esz = x->dtype == PPS_DTYPE_F16 ? 2 : 4;
   const unsigned char* base = static_cast<const unsigned char*>(d_rows) - (size_t)x->size * (size_t)ld * esz;
   PPS_TRY(pps_split_rows_slab(base, x->dtype, x->size, n, x->capacity, x->dim, ld, x->split_planes, x->g_planes, x->g_norm, st));
   if (d_tags)
     PPS_CUDA_TRY(cudaMemcpyAsync(x->g_tags + x->size, d_tags, (size_t)n * sizeof(int64_t), cudaMemcpyDeviceToDevice, st));
+  if (d_groups)
+    PPS_CUDA_TRY(cudaMemcpyAsync(x->g_groups + x->size, d_groups, (size_t)n * sizeof(int64_t), cudaMemcpyDeviceToDevice, st));
   x->size += n;
   return PPS_OK;
 }
@@ -669,16 +696,164 @@ int search(pps_index* x, const void* d_q, long long nq, long long ldq, const int
   return PPS_OK;
 }
 
+// grouped materialised block: rows [r0, r0 + rows) swept into the grouped state
+int group_block_update(pps_index* x, long long nq, long long r0, long long rows, long long ldd, long long index_offset, int k,
+                       uint64_t* keys, int64_t* groups, const int64_t* q_tags, cudaStream_t st) {
+  PPS_TRY(pps_dist_tc(x->qs.p, x->qn.as<float>(), nq, x->planes, 0, x->planes_at(r0), x->g_norm + r0, rows, x->planes,
+                      x->capacity, x->dim, x->precision, 0, x->dist.as<float>(), ldd, st));
+  return pps_topk_group_update(x->dist.as<float>(), ldd, nq, rows, index_offset + r0, x->g_groups + r0,
+                               q_tags ? x->g_tags + r0 : nullptr, q_tags, keys, groups, k, st);
+}
+
+// *out = the number of queries whose state holds fewer than k groups (its k-th key is ~0)
+__global__ void short_count_kernel(const unsigned long long* __restrict__ keys, long long nq, int k, uint32_t* __restrict__ out) {
+  __shared__ uint32_t s_n;
+  if (threadIdx.x == 0) s_n = 0u;
+  __syncthreads();
+  uint32_t n = 0u;
+  for (long long q = threadIdx.x; q < nq; q += blockDim.x) n += keys[q * k + k - 1] == ~0ull;
+  atomicAdd(&s_n, n);
+  __syncthreads();
+  if (threadIdx.x == 0) *out = s_n;
+}
+
+// range-kernel limits that count the rows at or below each query's bound (bits <= bound <=> bits < bound + 1), with no
+// room for keys: counters zeroed, capacities 0
+__global__ void count_lim_kernel(const uint32_t* __restrict__ bound, long long nq, uint32_t* __restrict__ lim,
+                                 uint32_t* __restrict__ cnt, long long* __restrict__ off, uint32_t* __restrict__ cap) {
+  const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+  if (i >= nq) return;
+  lim[i] = bound[i] == 0xffffffffu ? 0xffffffffu : bound[i] + 1u;
+  cnt[i] = 0u;
+  off[i] = 0;
+  cap[i] = 0u;
+}
+
+// Grouped search (pps_index_search_groups).  The admission kernels are search's: a row above the bound of a state that
+// holds k groups is either worse than its own group's row in the state or beaten by k other groups (DESIGN §4.16).
+//   1. prefix: materialised blocks of F rows swept by the grouped sweep until every query holds k groups (a 4-byte
+//      read-back per block: the queries still short) or the gallery ends
+//   2. L = the largest number of prefix rows at or below their query's bound (one counting pass of the range kernel over
+//      the prefix, one 4-byte read-back); chunks of R = cap F_done / (2.2 max(k, L)) rows, each admitted by the search
+//      kernel and merged by the grouped merge
+//   3. the overflow read-back; on overflow every block materialised and swept (right for any row order)
+int search_groups(pps_index* x, const void* d_q, long long nq, long long ldq, const int64_t* q_tags, int k,
+                  long long index_offset, int flags, void* stream, uint64_t* d_keys, int64_t* d_groups) {
+  if (nq < 0 || k < 1 || k > PPS_TOPK_MAX || index_offset < 0) return PPS_ERR_INVALID_ARG;
+  if (flags & ~(PPS_INDEX_TKCAP(0xffff) | PPS_INDEX_PREFIX(0x7f))) return PPS_ERR_INVALID_ARG;
+  if (nq > 0 && (ldq < x->dim || !d_q || !d_keys || !d_groups)) return PPS_ERR_INVALID_ARG;
+  if (index_offset + x->size > kMaxIndex || nq > kMaxIndex) return PPS_ERR_UNSUPPORTED;
+  if (nq == 0) return PPS_OK;
+  DeviceGuard dg(x->device);
+  if (dg.err != cudaSuccess) return pps::cuda_fail(dg.err, "cudaSetDevice");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  PPS_TRY(pps_topk_init(d_keys, nq, k, st));
+  PPS_CUDA_TRY(cudaMemsetAsync(d_groups, 0xff, (size_t)nq * k * sizeof(int64_t), st));   // -1
+  const long long size = x->size;
+  x->last_prefix = size;
+  x->last_chunks = 0;
+  x->last_fallback = 0;
+  if (size == 0) return PPS_OK;
+  int tk_cap = (flags >> 8) & 0xffff;
+  if (tk_cap <= 0 || tk_cap > kGroupTkCap) tk_cap = kGroupTkCap;
+  const long long prefix_hook = (long long)((flags >> 24) & 0x7f) * 256;
+  const long long first = std::min(size, prefix_hook > 0 ? prefix_hook : kPrefixRows);
+  const long long ldd = (first + 3) / 4 * 4;
+
+  PPS_TRY(x->qs.ensure((size_t)pps_split_bytes(nq, x->dim, x->planes)));
+  PPS_TRY(x->qn.ensure((size_t)nq * 2 * sizeof(float)));
+  PPS_TRY(x->dist.ensure((size_t)nq * ldd * sizeof(float)));
+  PPS_TRY(x->flag.ensure(8));           // [0] overflow flag, [1] queries short of k groups / largest count L
+  PPS_TRY(x->flag_h.ensure(4));
+  int32_t* flag = x->flag.as<int32_t>();
+  uint32_t* stat = reinterpret_cast<uint32_t*>(flag + 1);
+  PPS_TRY(pps_split_rows(d_q, x->dtype, nq, x->dim, ldq, x->split_planes, x->qs.p, x->qn.as<float>(), st));
+
+  // 1. prefix
+  long long done = 0;
+  while (done < size) {
+    const long long rows = std::min(first, size - done);
+    PPS_TRY(group_block_update(x, nq, done, rows, ldd, index_offset, k, d_keys, d_groups, q_tags, st));
+    done += rows;
+    if (done == size) break;
+    short_count_kernel<<<1, 256, 0, st>>>(reinterpret_cast<const unsigned long long*>(d_keys), nq, k, stat);
+    PPS_LAUNCH_CHECK("short_count_kernel");
+    PPS_CUDA_TRY(cudaMemcpyAsync(x->flag_h.p, stat, 4, cudaMemcpyDeviceToHost, st));
+    PPS_CUDA_TRY(cudaStreamSynchronize(st));
+    if (*x->flag_h.as<uint32_t>() == 0) break;
+  }
+  if (done == size) return PPS_OK;
+
+  // 2. L, then the chunks
+  PPS_TRY(x->tk_bound.ensure((size_t)nq * 4));
+  PPS_TRY(x->tk_cnt.ensure((size_t)nq * 4));
+  PPS_TRY(x->tk_cand.ensure((size_t)nq * tk_cap * 8));
+  PPS_TRY(x->rg_lim.ensure((size_t)nq * 4));
+  PPS_TRY(x->rg_cnt.ensure((size_t)nq * 2 * 4));
+  PPS_TRY(x->rg_off.ensure((size_t)nq * 8));
+  PPS_TRY(x->rg_cap.ensure((size_t)nq * 4));
+  uint32_t* bound = x->tk_bound.as<uint32_t>();
+  uint32_t* cnt = x->tk_cnt.as<uint32_t>();
+  uint32_t* n_le = x->rg_cnt.as<uint32_t>();
+  PPS_TRY(pps_topk_bound(d_keys, nq, k, bound, cnt, st));
+  count_lim_kernel<<<(unsigned)((nq + 255) / 256), 256, 0, st>>>(bound, nq, x->rg_lim.as<uint32_t>(), n_le,
+                                                                 x->rg_off.as<long long>(), x->rg_cap.as<uint32_t>());
+  PPS_LAUNCH_CHECK("count_lim_kernel");
+  PPS_TRY(pps_search_range_tc(x->planes_at(0), x->g_norm, done, x->planes, x->capacity, x->qs.p, x->qn.as<float>(), nq,
+                              x->planes, 0, x->dim, x->precision, 0, index_offset, x->rg_lim.as<uint32_t>(), n_le,
+                              x->rg_off.as<long long>(), x->rg_cap.as<uint32_t>(), x->tk_cand.as<uint64_t>(),
+                              q_tags ? x->g_tags : nullptr, q_tags, st));
+  max_u32_kernel<<<1, 256, 0, st>>>(n_le, nq, stat);
+  PPS_LAUNCH_CHECK("max_u32_kernel");
+  PPS_CUDA_TRY(cudaMemcpyAsync(x->flag_h.p, stat, 4, cudaMemcpyDeviceToHost, st));
+  PPS_CUDA_TRY(cudaMemsetAsync(flag, 0, 4, st));
+  PPS_CUDA_TRY(cudaStreamSynchronize(st));
+  const double per_row = (double)std::max<uint32_t>((uint32_t)k, *x->flag_h.as<uint32_t>());
+  x->last_prefix = done;
+  for (; done < size;) {
+    long long rows = (long long)((double)tk_cap * (double)done / (2.2 * per_row)) / 256 * 256;
+    rows = std::min(size - done, std::max<long long>(rows, 256));
+    if (q_tags)
+      PPS_TRY(pps_search_topk_excl_tc(x->planes_at(done), x->g_norm + done, rows, x->planes, x->capacity, x->qs.p,
+                                      x->qn.as<float>(), nq, x->planes, 0, x->dim, x->precision, 0, index_offset + done, bound,
+                                      cnt, x->tk_cand.as<uint64_t>(), tk_cap, st, x->g_tags + done, q_tags));
+    else
+      PPS_TRY(pps_search_topk_tc(x->planes_at(done), x->g_norm + done, rows, x->planes, x->capacity, x->qs.p,
+                                 x->qn.as<float>(), nq, x->planes, 0, x->dim, x->precision, 0, index_offset + done, bound, cnt,
+                                 x->tk_cand.as<uint64_t>(), tk_cap, st));
+    PPS_TRY(pps_topk_group_merge(d_keys, d_groups, nq, k, x->tk_cand.as<uint64_t>(), tk_cap, cnt, bound, x->g_groups,
+                                 index_offset, flag, st));
+    done += rows;
+    ++x->last_chunks;
+  }
+  PPS_CUDA_TRY(cudaMemcpyAsync(x->flag_h.p, flag, 4, cudaMemcpyDeviceToHost, st));
+  PPS_CUDA_TRY(cudaStreamSynchronize(st));
+  if (*x->flag_h.as<int32_t>() == 0) return PPS_OK;
+  // 3. a candidate buffer ran over: every block materialised and swept
+  x->last_fallback = 1;
+  PPS_TRY(pps_topk_init(d_keys, nq, k, st));
+  PPS_CUDA_TRY(cudaMemsetAsync(d_groups, 0xff, (size_t)nq * k * sizeof(int64_t), st));
+  for (long long r0 = 0; r0 < size; r0 += first)
+    PPS_TRY(group_block_update(x, nq, r0, std::min(first, size - r0), ldd, index_offset, k, d_keys, d_groups, q_tags, st));
+  return PPS_OK;
+}
+
 }  // namespace
 
 extern "C" int pps_index_add(pps_index* x, const void* d_rows, long long n, long long ld, void* stream) {
-  return add_rows(x, d_rows, n, ld, nullptr, stream);
+  return add_rows(x, d_rows, n, ld, nullptr, nullptr, stream);
 }
 
 extern "C" int pps_index_add_tagged(pps_index* x, const void* d_rows, long long n, long long ld, const int64_t* d_tags,
                                     void* stream) {
   if (n > 0 && !d_tags) return PPS_ERR_INVALID_ARG;
-  return add_rows(x, d_rows, n, ld, d_tags, stream);
+  return add_rows(x, d_rows, n, ld, d_tags, nullptr, stream);
+}
+
+extern "C" int pps_index_add_grouped(pps_index* x, const void* d_rows, long long n, long long ld, const int64_t* d_tags,
+                                     const int64_t* d_groups, void* stream) {
+  if (n > 0 && !d_groups) return PPS_ERR_INVALID_ARG;
+  return add_rows(x, d_rows, n, ld, d_tags, d_groups, stream);
 }
 
 extern "C" int pps_index_search(pps_index* x, const void* d_q, long long nq, long long ldq, int k, long long index_offset,
@@ -693,6 +868,23 @@ extern "C" int pps_index_search_excluding(pps_index* x, const void* d_q, long lo
   if (nq > 0 && !d_q_tags) return PPS_ERR_INVALID_ARG;
   if (x->size > 0 && !x->tagged) return PPS_ERR_INVALID_ARG;     // nothing to compare the query tags with
   return search(x, d_q, nq, ldq, d_q_tags, k, index_offset, flags, stream, d_keys);
+}
+
+extern "C" int pps_index_search_groups(pps_index* x, const void* d_q, long long nq, long long ldq, const int64_t* d_q_tags,
+                                       int k, long long index_offset, int flags, void* stream, uint64_t* d_keys,
+                                       int64_t* d_groups) {
+  if (!x) return PPS_ERR_INVALID_ARG;
+  if (x->size > 0 && !x->grouped) return PPS_ERR_INVALID_ARG;    // no groups to collapse
+  if (d_q_tags && x->size > 0 && !x->tagged) return PPS_ERR_INVALID_ARG;
+  return search_groups(x, d_q, nq, ldq, d_q_tags, k, index_offset, flags, stream, d_keys, d_groups);
+}
+
+extern "C" int pps_index_group_stats(const pps_index* x, long long* prefix_rows, long long* chunks, int* fallback) {
+  if (!x) return PPS_ERR_INVALID_ARG;
+  if (prefix_rows) *prefix_rows = x->last_prefix;
+  if (chunks) *chunks = x->last_chunks;
+  if (fallback) *fallback = x->last_fallback;
+  return PPS_OK;
 }
 
 extern "C" int pps_index_remove(pps_index* x, const int64_t* d_rows, long long n, int flags, void* stream,
@@ -740,14 +932,16 @@ extern "C" int pps_index_remove(pps_index* x, const int64_t* d_rows, long long n
     rm_fill_kernel<<<(unsigned)(nblk - b0), kRmThreads, 0, st>>>(flag, bsum, b0, first, size, kept);
     PPS_LAUNCH_CHECK("rm_fill_kernel");
 
-    // 3. move in pieces: gather into the piece buffer [planes][piece][kpad] | tags | norms | inverse scales, copy down
-    const size_t per_row = x->plane_bytes(1) * x->planes + (x->tagged ? 8 : 0) + (x->scaled() ? 8 : 4);
+    // 3. move in pieces: gather into the piece buffer [planes][piece][kpad] | tags | groups | norms | inverse scales,
+    //    copy down
+    const size_t per_row = x->plane_bytes(1) * x->planes + (x->tagged ? 8 : 0) + (x->scaled() ? 8 : 4) + (x->grouped ? 8 : 0);
     const long long hook = (flags >> 8) & 0xffff;
     const long long piece = std::min(moving, hook > 0 ? hook : std::max<long long>(1, (long long)(kRmPieceBytes / per_row)));
     PPS_TRY(x->rm_piece.ensure((size_t)piece * per_row));
     unsigned char* pb = x->rm_piece.as<unsigned char>();
     int64_t* p_tags = reinterpret_cast<int64_t*>(pb + x->planes * x->plane_bytes(piece));
-    float* p_norm = reinterpret_cast<float*>(pb + x->planes * x->plane_bytes(piece) + (x->tagged ? (size_t)piece * 8 : 0));
+    int64_t* p_groups = p_tags + (x->tagged ? piece : 0);
+    float* p_norm = reinterpret_cast<float*>(p_groups + (x->grouped ? piece : 0));
     float* p_scale = p_norm + piece;
     const int vec = x->kpad * 2 / 16;
     for (long long j0 = 0; j0 < moving; j0 += piece) {
@@ -758,6 +952,11 @@ extern "C" int pps_index_remove(pps_index* x, const int64_t* d_rows, long long n
           x->scaled() ? x->g_norm + x->capacity : nullptr, x->tagged ? x->g_tags : nullptr, reinterpret_cast<float4*>(pb),
           piece * vec, p_norm, p_scale, p_tags);
       PPS_LAUNCH_CHECK("rm_gather_kernel");
+      if (x->grouped) {
+        rm_gather_i64_kernel<<<(unsigned)((len + kRmThreads - 1) / kRmThreads), kRmThreads, 0, st>>>(kept + j0, len,
+                                                                                                  x->g_groups, p_groups);
+        PPS_LAUNCH_CHECK("rm_gather_i64_kernel");
+      }
       for (int p = 0; p < x->planes; ++p)
         PPS_CUDA_TRY(cudaMemcpyAsync(static_cast<unsigned char*>(x->g_planes) + p * x->plane_bytes(x->capacity) +
                                          x->plane_bytes(dst),
@@ -767,6 +966,8 @@ extern "C" int pps_index_remove(pps_index* x, const int64_t* d_rows, long long n
         PPS_CUDA_TRY(cudaMemcpyAsync(x->g_norm + x->capacity + dst, p_scale, (size_t)len * 4, cudaMemcpyDeviceToDevice, st));
       if (x->tagged)
         PPS_CUDA_TRY(cudaMemcpyAsync(x->g_tags + dst, p_tags, (size_t)len * 8, cudaMemcpyDeviceToDevice, st));
+      if (x->grouped)
+        PPS_CUDA_TRY(cudaMemcpyAsync(x->g_groups + dst, p_groups, (size_t)len * 8, cudaMemcpyDeviceToDevice, st));
     }
   }
   x->size = size - removed;

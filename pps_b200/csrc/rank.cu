@@ -720,6 +720,226 @@ __global__ void __launch_bounds__(kCntThreads) topk_merge_kernel(unsigned long l
 }
 
 // ------------------------------------------------------------------------------------
+// Grouped top-k (pps_index_search_groups): every gallery row carries an int64 group, and a query's state is the first
+// row of each of its k nearest groups - k keys ascending (~0 past the last group) plus the parallel [k] groups.  The
+// buffers of the grouped kernels hold kCand (key, group) pairs; group_select turns a buffer into a state: sort by key,
+// keep the first element of every group (a shared-memory hash of group -> smallest position, atomicMin), keep k.
+// ------------------------------------------------------------------------------------
+constexpr int kGrpHash = 2 * kCand;                     // open-addressing slots: load factor <= 1/2
+constexpr size_t kGrpSmem = (size_t)kCand * 16 + (size_t)kGrpHash * 4;
+
+__device__ __noinline__ void bitonic_sort_pairs_smem(unsigned long long* a, long long* g, int n /*pow2*/, int tid,
+                                                     int nthreads) {
+  for (int k = 2; k <= n; k <<= 1) {
+    for (int j = k >> 1; j > 0; j >>= 1) {
+      for (int i = tid; i < n; i += nthreads) {
+        const int ixj = i ^ j;
+        if (ixj > i) {
+          const unsigned long long x = a[i], y = a[ixj];
+          const bool up = (i & k) == 0;
+          if ((x > y) == up) {
+            a[i] = y; a[ixj] = x;
+            const long long t = g[i]; g[i] = g[ixj]; g[ixj] = t;
+          }
+        }
+      }
+      __syncthreads();
+    }
+  }
+}
+
+__device__ __forceinline__ int group_slot(long long g) {
+  return (int)(((unsigned long long)g * 0x9E3779B97F4A7C15ull) >> 52) & (kGrpHash - 1);
+}
+
+// a[kCand] / g[kCand] (unused slots: key ~0) -> the first element of each group in key order, compacted to the front,
+// at most k of them; the rest ~0.  Returns how many are kept (every thread).  Thread t owns positions
+// [t NPT, (t + 1) NPT), so the compaction is one block scan.  Keys are unique (the row is in the low bits).
+template <int NPT>
+__device__ __forceinline__ int group_select(unsigned long long* a, long long* g, int* slot, int k, int tid, int* s_warp,
+                                         int* s_total) {
+  constexpr int kThreads = kCand / NPT;
+  bitonic_sort_pairs_smem(a, g, kCand, tid, kThreads);
+  for (int i = tid; i < kGrpHash; i += kThreads) slot[i] = -1;
+  __syncthreads();
+  unsigned long long key[NPT];
+  long long grp[NPT];
+  int h[NPT];
+#pragma unroll
+  for (int j = 0; j < NPT; ++j) {
+    const int i = tid * NPT + j;
+    key[j] = a[i];
+    grp[j] = g[i];
+    h[j] = group_slot(grp[j]);
+    if (key[j] == ~0ull) continue;
+    while (true) {                                       // a slot only ever holds positions of one group
+      int cur = slot[h[j]];
+      if (cur < 0) {
+        cur = atomicCAS(slot + h[j], -1, i);
+        if (cur < 0) break;
+      }
+      if (g[cur] == grp[j]) {
+        atomicMin(slot + h[j], i);
+        break;
+      }
+      h[j] = (h[j] + 1) & (kGrpHash - 1);
+    }
+  }
+  __syncthreads();
+  int keep = 0;
+#pragma unroll
+  for (int j = 0; j < NPT; ++j) keep += key[j] != ~0ull && slot[h[j]] == tid * NPT + j;
+  // exclusive scan of keep over the threads
+  const int lane = tid & 31, warp = tid >> 5;
+  int x = keep;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const int y = __shfl_up_sync(0xffffffffu, x, o);
+    if (lane >= o) x += y;
+  }
+  if (lane == 31) s_warp[warp] = x;
+  __syncthreads();
+  int pos = x - keep;
+  for (int w = 0; w < warp; ++w) pos += s_warp[w];
+  if (tid == kThreads - 1) *s_total = pos + keep;
+#pragma unroll
+  for (int j = 0; j < NPT; ++j) {                        // every thread's elements are in registers: rewrite in place
+    a[tid * NPT + j] = ~0ull;
+    g[tid * NPT + j] = -1;
+  }
+  __syncthreads();
+#pragma unroll
+  for (int j = 0; j < NPT; ++j)
+    if (key[j] != ~0ull && slot[h[j]] == tid * NPT + j) {
+      if (pos < k) { a[pos] = key[j]; g[pos] = grp[j]; }
+      ++pos;
+    }
+  __syncthreads();
+  return min(*s_total, k);
+}
+
+// bitonic_sort_pairs_smem's stride loop over n = kCand with kThreads threads; group_select's scan needs kThreads <= 1024
+static_assert(kTopkThreads * 8 == kCand, "grouped kernels: 8 buffer entries per thread");
+
+// grouped counterpart of topk_update_kernel (materialised block, one CTA per query): column c is admitted when its key
+// beats the state's k-th key (all columns while fewer than k groups are held), with g_groups[c] read for admitted
+// columns only; TAGS: not when g_tags[c] == q_tags[q].  A full buffer is re-selected by group_select.
+template <bool TAGS>
+__global__ void __launch_bounds__(kTopkThreads, 2) topk_group_update_kernel(const float* __restrict__ dist, long long ldd,
+                                                                          long long ncols, long long col0,
+                                                                          const long long* __restrict__ g_groups,
+                                                                          const long long* __restrict__ g_tags,
+                                                                          const long long* __restrict__ q_tags,
+                                                                          unsigned long long* __restrict__ topk_key,
+                                                                          long long* __restrict__ topk_group, int k) {
+  extern __shared__ unsigned long long grp_smem[];
+  unsigned long long* cand = grp_smem;
+  long long* cgrp = reinterpret_cast<long long*>(grp_smem + kCand);
+  int* slot = reinterpret_cast<int*>(grp_smem + 2 * kCand);
+  __shared__ int s_n, s_warp[32], s_total;
+  __shared__ unsigned long long s_bound;
+  const int q = blockIdx.x, tid = threadIdx.x;
+  unsigned long long* state = topk_key + (long long)q * k;
+  long long* sgrp = topk_group + (long long)q * k;
+  for (int i = tid; i < kCand; i += kTopkThreads) {
+    cand[i] = i < k ? state[i] : ~0ull;
+    cgrp[i] = i < k ? sgrp[i] : -1;
+  }
+  if (tid == 0) { s_n = k; s_bound = state[k - 1]; }
+  __syncthreads();
+  const float* drow = dist + (long long)q * ldd;
+  const long long qtag = TAGS ? q_tags[q] : 0;
+  const long long tile = 4LL * kTopkThreads;
+  for (long long c0 = 0; c0 < ncols; c0 += tile) {
+    const unsigned long long bound = s_bound;
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+      const long long c = c0 + (long long)u * kTopkThreads + tid;
+      if (c < ncols) {
+        const float d = ld_stream_f32(drow + c);
+        const unsigned long long key = ((unsigned long long)__float_as_uint(d) << 32) | (unsigned long long)(uint32_t)(col0 + c);
+        if (key < bound && !(TAGS && __ldg(g_tags + c) == qtag)) {
+          const int s = atomicAdd(&s_n, 1);              // s_n <= kCand - tile at tile start, so s < kCand
+          cand[s] = key;
+          cgrp[s] = __ldg(g_groups + c);
+        }
+      }
+    }
+    __syncthreads();
+    const int n_now = s_n;
+    __syncthreads();
+    if (n_now > kCand - (int)tile) {
+      const int fill = group_select<kCand / kTopkThreads>(cand, cgrp, slot, k, tid, s_warp, &s_total);
+      if (tid == 0) { s_n = fill; s_bound = fill == k ? cand[k - 1] : ~0ull; }
+      __syncthreads();
+    }
+  }
+  group_select<kCand / kTopkThreads>(cand, cgrp, slot, k, tid, s_warp, &s_total);
+  for (int i = tid; i < k; i += kTopkThreads) {
+    state[i] = cand[i];
+    sgrp[i] = cgrp[i];
+  }
+}
+
+// grouped counterpart of topk_merge_kernel, also the merge of per-shard lists.  Query q's n candidates: candidate i is
+// key cand[(i / seg) * seg_stride + q * q_stride + i % seg] (~0: none), its group cand_groups[same place] or, without
+// cand_groups, g_groups[row - index_offset].  n = min(tk_cnt[q], seg) with tk_cnt (overflow raised past seg; tk_cnt
+// reset, tk_bound = the new state's k-th distance bits), n_fixed otherwise.  in_key / in_group: the state merged with
+// (null: none).  The candidates pass through the kCand buffer in pieces, so n is not bounded by it.
+__global__ void __launch_bounds__(kTopkThreads, 2) topk_group_merge_kernel(
+    const unsigned long long* in_key, const long long* in_group, unsigned long long* out_key,
+    long long* out_group, int k, const unsigned long long* __restrict__ cand, const long long* __restrict__ cand_groups,
+    const long long* __restrict__ g_groups, long long index_offset, int seg, long long seg_stride, long long q_stride,
+    long long n_fixed, uint32_t* __restrict__ tk_cnt, uint32_t* __restrict__ tk_bound, int* __restrict__ overflow) {
+  extern __shared__ unsigned long long grp_smem[];
+  unsigned long long* buf = grp_smem;
+  long long* bgrp = reinterpret_cast<long long*>(grp_smem + kCand);
+  int* slot = reinterpret_cast<int*>(grp_smem + 2 * kCand);
+  __shared__ int s_n, s_warp[32], s_total;
+  const int q = blockIdx.x, tid = threadIdx.x;
+  long long n = n_fixed;
+  if (tk_cnt) {
+    const uint32_t raw = tk_cnt[q];
+    if (raw == 0u) return;                               // nothing was admitted for this query in the chunk
+    if (raw > (uint32_t)seg && tid == 0) atomicExch(overflow, 1);
+    n = min((long long)raw, (long long)seg);
+  }
+  const int k0 = in_key ? k : 0;
+  for (int i = tid; i < kCand; i += kTopkThreads) {
+    buf[i] = i < k0 ? in_key[(long long)q * k + i] : ~0ull;
+    bgrp[i] = i < k0 ? in_group[(long long)q * k + i] : -1;
+  }
+  if (tid == 0) s_n = k0;
+  __syncthreads();
+  int fill = k0;
+  for (long long base = 0; base < n;) {
+    const long long take = min(n - base, (long long)(kCand - fill));
+    for (long long i = base + tid; i < base + take; i += kTopkThreads) {
+      const long long at = (i / seg) * seg_stride + q * q_stride + i % seg;
+      const unsigned long long key = cand[at];
+      if (key == ~0ull) continue;
+      const int s = atomicAdd(&s_n, 1);
+      buf[s] = key;
+      bgrp[s] = cand_groups ? cand_groups[at] : g_groups[(long long)(key & 0xffffffffull) - index_offset];
+    }
+    base += take;
+    __syncthreads();
+    fill = group_select<kCand / kTopkThreads>(buf, bgrp, slot, k, tid, s_warp, &s_total);
+    if (tid == 0) s_n = fill;
+    __syncthreads();
+  }
+  if (n == 0) fill = group_select<kCand / kTopkThreads>(buf, bgrp, slot, k, tid, s_warp, &s_total);
+  for (int i = tid; i < k; i += kTopkThreads) {
+    out_key[(long long)q * k + i] = buf[i];
+    out_group[(long long)q * k + i] = bgrp[i];
+  }
+  if (tk_cnt && tid == 0) {
+    tk_bound[q] = fill == k ? (uint32_t)(buf[k - 1] >> 32) : 0xffffffffu;
+    tk_cnt[q] = 0u;
+  }
+}
+
+// ------------------------------------------------------------------------------------
 // Secondary metric: AP as scikit-learn 0.18.1 defined it (the version reid_dataset_evaluator.py:398-407 asks for):
 // area under the precision-recall curve by the trapezoidal rule.  From counts, with v the distinct positive distances:
 //   AP = sum_v (tp(v) - tp(<v)) / P * ( tp(v) / n_le(v) + P_prev(v) ) / 2,
@@ -1032,6 +1252,79 @@ extern "C" int pps_topk_merge(uint64_t* topk_key, long long nq, int k, const uin
       tk_bound, filt ? pair_off : nullptr, pair_g, pair_pos, filt ? 1 : 0, overflow,
       max_pairs_per_query > 0 ? max_pairs_per_query : 1);
   PPS_LAUNCH_CHECK("topk_merge_kernel");
+  return PPS_OK;
+}
+
+// ---- grouped top-k (pps_index_search_groups) ----
+namespace {
+int group_smem_setup() {
+  static thread_local int configured_dev = -1;
+  int dev = 0;
+  PPS_CUDA_TRY(cudaGetDevice(&dev));
+  if (configured_dev != dev) {
+    PPS_CUDA_TRY(cudaFuncSetAttribute(topk_group_update_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kGrpSmem));
+    PPS_CUDA_TRY(cudaFuncSetAttribute(topk_group_update_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kGrpSmem));
+    PPS_CUDA_TRY(cudaFuncSetAttribute(topk_group_merge_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kGrpSmem));
+    configured_dev = dev;
+  }
+  return PPS_OK;
+}
+}  // namespace
+
+extern "C" int pps_topk_group_update(const float* dist, long long ldd, long long nq, long long ncols, long long col0,
+                                     const int64_t* g_groups, const int64_t* g_tags, const int64_t* q_tags, uint64_t* topk_key,
+                                     int64_t* topk_group, int k, void* stream) {
+  if (nq < 0 || ncols < 0 || ldd < ncols || k < 1 || k > PPS_TOPK_MAX) return PPS_ERR_INVALID_ARG;
+  if (nq == 0) return PPS_OK;
+  if (!topk_key || !topk_group || (!g_tags != !q_tags) || (ncols > 0 && (!dist || !g_groups))) return PPS_ERR_INVALID_ARG;
+  if (nq > 0x7fffffffLL || col0 < 0 || col0 + ncols > 0xffffffffLL) return PPS_ERR_UNSUPPORTED;
+  if (const int rc = group_smem_setup()) return rc;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  auto* keys = reinterpret_cast<unsigned long long*>(topk_key);
+  auto* grps = reinterpret_cast<long long*>(topk_group);
+  const auto* gg = reinterpret_cast<const long long*>(g_groups);
+  if (q_tags) {
+    topk_group_update_kernel<true><<<(unsigned)nq, kTopkThreads, kGrpSmem, st>>>(
+        dist, ldd, ncols, col0, gg, reinterpret_cast<const long long*>(g_tags), reinterpret_cast<const long long*>(q_tags),
+        keys, grps, k);
+    PPS_LAUNCH_CHECK("topk_group_update_kernel<excl>");
+  } else {
+    topk_group_update_kernel<false><<<(unsigned)nq, kTopkThreads, kGrpSmem, st>>>(dist, ldd, ncols, col0, gg, nullptr, nullptr,
+                                                                                  keys, grps, k);
+    PPS_LAUNCH_CHECK("topk_group_update_kernel");
+  }
+  return PPS_OK;
+}
+
+extern "C" int pps_topk_group_merge(uint64_t* topk_key, int64_t* topk_group, long long nq, int k, const uint64_t* tk_cand,
+                                    int tk_cap, uint32_t* tk_cnt, uint32_t* tk_bound, const int64_t* g_groups,
+                                    long long index_offset, int32_t* overflow, void* stream) {
+  if (nq < 0 || k < 1 || k > PPS_TOPK_MAX || tk_cap < 1 || index_offset < 0) return PPS_ERR_INVALID_ARG;
+  if (nq == 0) return PPS_OK;
+  if (!topk_key || !topk_group || !tk_cand || !tk_cnt || !tk_bound || !g_groups || !overflow) return PPS_ERR_INVALID_ARG;
+  if (nq > 0x7fffffffLL) return PPS_ERR_UNSUPPORTED;
+  if (const int rc = group_smem_setup()) return rc;
+  auto* keys = reinterpret_cast<unsigned long long*>(topk_key);
+  auto* grps = reinterpret_cast<long long*>(topk_group);
+  topk_group_merge_kernel<<<(unsigned)nq, kTopkThreads, kGrpSmem, static_cast<cudaStream_t>(stream)>>>(
+      keys, grps, keys, grps, k, reinterpret_cast<const unsigned long long*>(tk_cand), nullptr,
+      reinterpret_cast<const long long*>(g_groups), index_offset, tk_cap, 0, tk_cap, 0, tk_cnt, tk_bound, overflow);
+  PPS_LAUNCH_CHECK("topk_group_merge_kernel");
+  return PPS_OK;
+}
+
+extern "C" int pps_topk_group_merge_lists(const uint64_t* keys, const int64_t* groups, int lists, long long nq, int k,
+                                          uint64_t* out_key, int64_t* out_group, void* stream) {
+  if (lists < 1 || nq < 0 || k < 1 || k > PPS_TOPK_MAX) return PPS_ERR_INVALID_ARG;
+  if (nq == 0) return PPS_OK;
+  if (!keys || !groups || !out_key || !out_group) return PPS_ERR_INVALID_ARG;
+  if (nq > 0x7fffffffLL) return PPS_ERR_UNSUPPORTED;
+  if (const int rc = group_smem_setup()) return rc;
+  topk_group_merge_kernel<<<(unsigned)nq, kTopkThreads, kGrpSmem, static_cast<cudaStream_t>(stream)>>>(
+      nullptr, nullptr, reinterpret_cast<unsigned long long*>(out_key), reinterpret_cast<long long*>(out_group), k,
+      reinterpret_cast<const unsigned long long*>(keys), reinterpret_cast<const long long*>(groups), nullptr, 0, k, nq * k, k,
+      (long long)lists * k, nullptr, nullptr, nullptr);
+  PPS_LAUNCH_CHECK("topk_group_merge_kernel<lists>");
   return PPS_OK;
 }
 

@@ -12,6 +12,10 @@ encodings cover person retrieval:
 - cross-camera search: ``tags = gallery cameras``, ``exclude_tags = query cameras``;
 - the evaluation protocol's junk rule (same id and same camera): ``tag = (id << 32) | camera`` for ids in int32 and
   cameras in [0, 2^32), on both sides.  The result then equals ``rank_eval(..., topk=k)`` bit for bit.
+
+Rows may also carry one int64 group each (``add(feats, groups=...)``: a tracklet or an identity), and
+``search_groups(q, k)`` returns the nearest row of each of the k nearest groups, so that the frames of one tracklet
+take one place of the result instead of all of them.
 """
 from __future__ import annotations
 
@@ -59,6 +63,16 @@ class GalleryIndex:
     (distance, index) order, so with ``radius[i]`` the k-th distance of ``search(q, k)`` the first k equal ``search``'s
     row and the rest are ties at ``radius[i]``.  ``exclude_tags`` as in ``search``.  Sharded: collective, every rank gets
     the result of one index holding the concatenated shards.
+
+    ``add(feats, tags=None, groups=None)`` with ``groups`` ([n] integers, e.g. tracklet or identity ids) makes the index
+    grouped; as with tags, the first non-empty add decides, a later add of the other kind raises, and an index emptied by
+    ``remove`` decides again.  ``dist, index, group = search_groups(q, k, exclude_tags=None)`` returns, per query, the
+    rows ``search(q, k, exclude_tags)`` would order, by the same (distance, index) keys, with every row after the first
+    of its group dropped, the first k of them: [nq, k] float32 distances, int64 rows (each group's nearest row) and int64
+    groups, padded with inf / -1 / -1 past the last group (find padding by ``index == -1``).  When every row is its own
+    group, ``dist`` and ``index`` equal ``search``'s bit for bit.  k is in [1, 128]; it needs a grouped index (an empty
+    one answers with padding).  Groups move with their rows in ``remove``.  Sharded: collective, and a group may have rows
+    on several ranks; every rank gets the result of one index holding the concatenated shards.
     """
 
     def __init__(self, dim, dtype=None, precision="f16x3", device=None, group=None):
@@ -123,14 +137,19 @@ class GalleryIndex:
             raise RuntimeError("%s: expected shape [%s], got %s" % (name, "n" if n is None else n, tuple(t.shape)))
         return t.to(device=self.device, dtype=torch.int64).contiguous()
 
-    def add(self, feats, tags=None):
-        """Append rows (with their tags); returns (row0, rows), their range among this index's (local) rows."""
+    def add(self, feats, tags=None, groups=None):
+        """Append rows (with their tags and groups); returns (row0, rows), their range among this index's (local) rows."""
         import torch
         x, _ = self._rows(feats, "feats")
         row0, n = len(self), int(x.shape[0])
         ld = int(x.stride(0)) if n else self.dim
         with torch.cuda.device(self.device):
-            if tags is None:
+            if groups is not None:
+                gr = self._tags(groups, n, "groups")
+                t = None if tags is None else self._tags(tags, n, "tags")
+                _lib.check(self._lib.pps_index_add_grouped(self._h, _lib.ptr(x), n, ld, _lib.ptr(t), _lib.ptr(gr),
+                                                           _lib.stream_ptr()), "pps_index_add_grouped")
+            elif tags is None:
                 _lib.check(self._lib.pps_index_add(self._h, _lib.ptr(x), n, ld, _lib.stream_ptr()), "pps_index_add")
             else:
                 t = self._tags(tags, n, "tags")
@@ -256,6 +275,42 @@ class GalleryIndex:
             lims, keys = gather_range_keys(lims, keys, self.group)
         return self._unpack_range(lims, keys, is_np)
 
+    def _search_group_keys(self, q, k, index_offset=0, flags=0, exclude_tags=None):
+        """([nq, k] keys, [nq, k] groups, whether q was numpy) of this index alone; flags: PPS_INDEX_* hooks."""
+        import torch
+        x, is_np = self._rows(q, "q")
+        if not isinstance(k, (int, np.integer)) or not 1 <= int(k) <= _lib.TOPK_MAX:
+            raise RuntimeError("k must be an integer in [1, %d], got %r" % (_lib.TOPK_MAX, k))
+        nq, k = int(x.shape[0]), int(k)
+        ldq = int(x.stride(0)) if nq else self.dim
+        t = None if exclude_tags is None else self._tags(exclude_tags, nq, "exclude_tags")
+        keys = torch.empty((nq, k), dtype=torch.int64, device=self.device)
+        groups = torch.empty((nq, k), dtype=torch.int64, device=self.device)
+        with torch.cuda.device(self.device):
+            _lib.check(self._lib.pps_index_search_groups(self._h, _lib.ptr(x), nq, ldq, _lib.ptr(t), k, int(index_offset),
+                                                         int(flags), _lib.stream_ptr(), _lib.ptr(keys), _lib.ptr(groups)),
+                       "pps_index_search_groups")
+        return keys, groups, is_np
+
+    def _group_stats(self):
+        """(rows swept as materialised blocks before the chunks, chunks, whether the fallback ran) of the last
+        search_groups on this index"""
+        prefix, chunks, fallback = C.c_longlong(0), C.c_longlong(0), C.c_int(0)
+        _lib.check(self._lib.pps_index_group_stats(self._h, C.byref(prefix), C.byref(chunks), C.byref(fallback)),
+                   "pps_index_group_stats")
+        return int(prefix.value), int(chunks.value), bool(fallback.value)
+
+    def search_groups(self, q, k, exclude_tags=None):
+        """(dist [nq, k] float32, index [nq, k] int64, group [nq, k] int64): the nearest row of each of the k nearest
+        groups of every query row (with exclude_tags: among the rows whose tag is not the query's)."""
+        keys, groups, is_np = self._search_group_keys(q, k, self._offset(), exclude_tags=exclude_tags)
+        if self.group is not None:
+            keys, groups = merge_group_keys(keys, groups, int(k), self.group)
+        dist, index = self._unpack(keys, False)
+        if is_np:
+            return dist.cpu().numpy(), index.cpu().numpy(), groups.cpu().numpy()
+        return dist, index, groups
+
     def search(self, q, k, exclude_tags=None):
         """(dist [nq, k] float32, index [nq, k] int64) of the k nearest gallery rows of every query row (with
         exclude_tags: of the rows whose tag is not the query's)."""
@@ -263,6 +318,33 @@ class GalleryIndex:
         if self.group is not None:
             keys = merge_topk_keys(keys, int(k), self.group)
         return self._unpack(keys, is_np)
+
+
+def merge_group_keys(keys, groups, k, group):
+    """All-gather every rank's [nq, k] grouped keys and groups and merge them (merge_group_lists)."""
+    import torch.distributed as dist_mod
+    world = dist_mod.get_world_size(group)
+    all_keys = [keys.new_empty(keys.shape) for _ in range(world)]
+    all_groups = [groups.new_empty(groups.shape) for _ in range(world)]
+    dist_mod.all_gather(all_keys, keys, group=group)
+    dist_mod.all_gather(all_groups, groups, group=group)
+    return merge_group_lists(all_keys, all_groups, k)
+
+
+def merge_group_lists(keys_list, groups_list, k):
+    """One grouped result from several ([nq, k] keys, [nq, k] groups) of disjoint row sets (shards; a group may span
+    them): per query, every list's keys in key order, the first of each group, the first k (pps_topk_group_merge_lists)."""
+    import torch
+    keys = torch.stack(list(keys_list)).contiguous()
+    groups = torch.stack(list(groups_list)).contiguous()
+    lists, nq = int(keys.shape[0]), int(keys.shape[1])
+    out_k = torch.empty((nq, k), dtype=torch.int64, device=keys.device)
+    out_g = torch.empty((nq, k), dtype=torch.int64, device=keys.device)
+    lib = _lib.load()
+    with torch.cuda.device(keys.device):
+        _lib.check(lib.pps_topk_group_merge_lists(_lib.ptr(keys), _lib.ptr(groups), lists, nq, k, _lib.ptr(out_k),
+                                                  _lib.ptr(out_g), _lib.stream_ptr()), "pps_topk_group_merge_lists")
+    return out_k, out_g
 
 
 def gather_range_keys(lims, keys, group):

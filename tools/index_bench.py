@@ -49,8 +49,19 @@ queries.  Default galleries fp16_10M and fp32_520k, batches 1, 16, 64, 256.  A l
   ok                     the output against the top-k invariant: the first k results of each query equal search's row
                          (k = min(100, hits)), every result is within the radius, lims add up
 
+--groups measures GalleryIndex.search_groups instead, one line per (gallery, layout, batch), k = 100.  The rows form
+tracklets of 1, 16, 256 or 2 048 rows (group = row // length), stored contiguously or with the groups shuffled over the
+rows.  Default galleries fp16_10M and fp32_520k, batches 1, 16, 64, 256.  A line records:
+  groups_ms / search_ms  medians of search_groups(q, 100) and of search(q, 100) on the same index, alternated
+  prefix_rows, chunks, fallback   the grouped schedule of the last call: rows swept as materialised blocks, chunks after
+                         them, and whether the materialised fallback ran
+  launches               kernels the library launched for one grouped call
+  ok                     query 0's result against NumPy on compute_dist's own distances of the whole gallery (first row
+                         of each group in key order), bit for bit
+
 usage: python tools/index_bench.py [--reps 10] [--warmup 2] [--out FILE] [--cases fp16_1M,fp16_10M,fp32_520k]
                                    [--tags none,cam6,half,junk] [--batches 1,16,64,256,3368] [--remove] [--range]
+                                   [--groups]
 """
 from __future__ import annotations
 
@@ -357,6 +368,59 @@ def run_range_case(name, batches, reps, warmup, emit):
     torch.cuda.empty_cache()
 
 
+GROUP_LENGTHS = [1, 16, 256, 2048]
+
+
+def np_first_per_group(dist_row, groups, k):
+    """(dist, index) of the first row of each group in (distance bits, row) order, the first k"""
+    order = np.lexsort((np.arange(len(dist_row)), dist_row.view(np.uint32)))
+    _, first = np.unique(groups[order], return_index=True)
+    pick = order[np.sort(first)][:k]
+    return dist_row[pick], pick
+
+
+def run_groups_case(name, batches, reps, warmup, emit):
+    import torch
+    import pps_b200
+    from pps_b200 import _lib, synthetic
+    ng, dtype_name = CASES[name]
+    dev = torch.device("cuda")
+    tdt = torch.float16 if dtype_name == "fp16" else torch.float32
+    qid, _, gid, _ = synthetic.make_distractor_ids(max(batches), ng)
+    q_all = synthetic.make_features_device(qid, DIM, 750, 4.0, 7, dev, tdt)
+    g = synthetic.make_features_device(gid, DIM, 750, 4.0, 1000, dev, tdt)
+    own0 = pps_b200.compute_dist(q_all[:1], g)[0].cpu().numpy()          # query 0 against every row
+    gpu, watts = card(torch.cuda.current_device())
+    rs = np.random.RandomState(11)
+    for length in GROUP_LENGTHS:
+        for layout in ("contiguous", "shuffled"):
+            groups = (np.arange(ng) // length).astype(np.int64)
+            if layout == "shuffled":
+                groups = groups[rs.permutation(ng)]
+            want_d, want_i = np_first_per_group(own0, groups, K)
+            idx = pps_b200.GalleryIndex(DIM, dtype=tdt, precision="f16x3")
+            idx.add(g, None, torch.from_numpy(groups).to(dev))
+            for nq in batches:
+                q = q_all[:nq].contiguous()
+                s_ms, g_ms, (gd, gi, _) = timed_alternating(lambda: idx.search(q, K), lambda: idx.search_groups(q, K),
+                                                            reps, warmup)
+                n0 = _lib.launch_count()
+                idx.search_groups(q, K)
+                launches = _lib.launch_count() - n0
+                prefix, chunks, fallback = idx._group_stats()
+                ok = bool(np.array_equal(gi[0].cpu().numpy(), want_i)
+                          and np.array_equal(gd[0].cpu().numpy().view(np.uint32), want_d.view(np.uint32)))
+                emit({"case": name, "dtype": dtype_name, "precision": "f16x1" if dtype_name == "fp16" else "f16x3",
+                      "ng": ng, "dim": DIM, "nq": nq, "k": K, "group_rows": length, "layout": layout,
+                      "groups_ms": round(g_ms, 4), "search_ms": round(s_ms, 4), "ratio": round(g_ms / s_ms, 3),
+                      "prefix_rows": prefix, "chunks": chunks, "fallback": fallback, "launches": launches, "ok": ok,
+                      "reps": reps, "gpu": gpu, "power_limit_w": watts})
+            del idx
+            torch.cuda.empty_cache()
+    del g, q_all
+    torch.cuda.empty_cache()
+
+
 def run_case(name, reps, warmup, emit, batches=BATCHES):
     import torch
     import pps_b200
@@ -406,6 +470,8 @@ def main():
     ap.add_argument("--remove", action="store_true", help="measure GalleryIndex.remove (default batches 1,64)")
     ap.add_argument("--range", action="store_true",
                     help="measure GalleryIndex.range_search (default galleries fp16_10M,fp32_520k, batches 1,16,64,256)")
+    ap.add_argument("--groups", action="store_true",
+                    help="measure GalleryIndex.search_groups (default galleries fp16_10M,fp32_520k, batches 1,16,64,256)")
     args = ap.parse_args()
     import torch
     if not torch.cuda.is_available():
@@ -421,9 +487,9 @@ def main():
     batches = [int(b) for b in args.batches.split(",") if b]
     if args.remove and args.batches == ap.get_default("batches"):
         batches = [1, 64]
-    if args.range and args.batches == ap.get_default("batches"):
+    if (args.range or args.groups) and args.batches == ap.get_default("batches"):
         batches = [1, 16, 64, 256]
-    if args.range and args.cases == ap.get_default("cases"):
+    if (args.range or args.groups) and args.cases == ap.get_default("cases"):
         names = ["fp16_10M", "fp32_520k"]
 
     def emit(rec):
@@ -440,6 +506,10 @@ def main():
     if args.range:
         for c in names:
             run_range_case(c, batches, args.reps, args.warmup, emit)
+        return
+    if args.groups:
+        for c in names:
+            run_groups_case(c, batches, args.reps, args.warmup, emit)
         return
     tagged = [m for m in modes if m != "none"]
     for c in names:
